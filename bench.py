@@ -13,7 +13,8 @@ A "step" = one pass of the hot path over one batch of synthetic input.  `value` 
 region).  `roofline` = dominant kernel, timed live with CUDA events on the launching stream (library profile
 scopes).  `cpu_baseline` = the oracle (C restatement of halo2_proofs' rayon algorithms) on this box's host cores
 over a bounded sample.  `--impl reference` times that CPU restatement alone (the Rust reference cannot be built
-or run here: no cargo, crates not vendored -- DESIGN.md).
+or run here: no cargo, crates not vendored -- DESIGN.md).  `--dump-outputs DIR` writes what the last device-resident
+step computed (proof bytes, MSM point, NTT output or commitments) for output-for-output comparison of two builds.
 """
 import argparse, json, os, subprocess, sys, threading, time
 
@@ -60,7 +61,12 @@ def parse():
     ap.add_argument("--cpu-sample-log", type=int, default=18)
     ap.add_argument("--no-extras", dest="extras", action="store_false",
                     help="default (shot) run only: skip the compact Board / MSM / NTT sub-benchmarks reported under `extras`")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last device-resident step computed as DIR/<name>.npy "
+                         "(bytes as float32, at most 64 MB in all); inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.inflight <= 0:          # measured on 1xB200 / 16 cores: 4 lanes 3 153, 6 lanes 3 254, 8 lanes 3 286 Shot proofs/s
         try:
             cores = len(os.sched_getaffinity(0))
@@ -168,6 +174,23 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(outputs, out_dir):
+    """outputs: {name: array whose first axis indexes items}.  Every item is written as its bytes in float32 (exact); if
+    that exceeds DUMP_LIMIT in all, every output keeps the same seeded random sample of a share of its items."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = {k: np.ascontiguousarray(v).view(np.uint8).reshape(len(v), -1) for k, v in outputs.items()}
+    total = sum(4 * r.size for r in rows.values())
+    budget = DUMP_LIMIT - 4096 * len(rows)                       # room for the .npy headers
+    for name, r in rows.items():
+        if total > budget:
+            keep = max(1, len(r) * budget // total)
+            r = r[np.sort(np.random.default_rng(0).choice(len(r), keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), r.astype(np.float32))
 
 
 def rand_field(rng, n):
@@ -303,6 +326,17 @@ class MsmWorkload:
             return self.n_total / self.world
         return self.n
 
+    def outputs(self):
+        """the MSM result of the last device step as an affine point (Jacobian coordinates are not unique)"""
+        if self.world > 1:
+            return {"msm": self.result_affine()[None]}
+        c = self.ctx
+        d_a = c.alloc(64)
+        c._check(c.lib.bz_batch_normalize_dev(c.h, self.curve, self.d_out.ptr, d_a.ptr, 1))
+        out = d_a.download((1, 8))
+        d_a.free()
+        return {"msm": out}
+
     def dominant(self):
         # MSM algorithmic bytes: 32 B scalar + 64 B base per point (SURVEY §8d: 96*N); dominant kernel = bucket accumulation
         return "msm_bucket", 96.0 * self.n
@@ -358,6 +392,9 @@ class NttWorkload:
         c = self.ctx
         c._check(c.lib.bz_best_fft(c.h, 0, ctypes.c_void_p(self.h_a.data_ptr()), self.omega.ctypes.data_as(ctypes.c_void_p), self.log))
         return 64.0 * self.n / 1e9
+
+    def outputs(self):
+        return {"ntt": self.d_b.download((self.n, 4))}
 
     def dominant(self):
         npass = 1 if self.log <= 12 else (2 if self.log <= 20 else 3)
@@ -443,6 +480,9 @@ class CommitWorkload:
         units = self._commit()
         self.h_result = self.result.cpu()
         return units
+
+    def outputs(self):
+        return {"commitments": self.result.cpu().numpy()}
 
     def dominant(self):
         tag = "fixed_msm" if self.k <= 19 else "msm_bucket"
@@ -661,6 +701,11 @@ class ProofWorkload:
             f.result()
         return self.B * self.T * steps
 
+    def outputs(self):
+        """proof bytes of the last call of every lane; row t * B + i is proof i of lane t, whose witness and RNG stream
+        depend on that row alone"""
+        return {"proofs": np.concatenate([lane["proofs"] for lane in self.lanes])}
+
     def single_latency(self, reps=7):
         """latency of ONE proof (batch 1, one lane, device-resident inputs): median wall ms of `reps` calls"""
         import ctypes
@@ -801,8 +846,9 @@ def run_reference(args, rank):
         "gpu_launches": 0}))
 
 
-def measure(args, wl, ctx, stream, rank, world, local_rank, want_cpu=True, steps=None, warmup=None):
-    """One workload, three timed passes (device-resident, per-kernel profile, end-to-end with host buffers) -> dict."""
+def measure(args, wl, ctx, stream, rank, world, local_rank, want_cpu=True, steps=None, warmup=None, dump_dir=None):
+    """One workload, three timed passes (device-resident, per-kernel profile, end-to-end with host buffers) -> dict.
+    dump_dir: rank 0 writes the outputs of the device-resident pass's last step there (dump_outputs)."""
     import torch
     import torch.distributed as dist
     steps = steps or args.steps
@@ -834,6 +880,8 @@ def measure(args, wl, ctx, stream, rank, world, local_rank, want_cpu=True, steps
     ms = float(ms.item())
     clocks = sampler.stop() if rank == 0 else None
     launches = sum(c.kernel_launches() for c in ctxs) - launches0
+    if dump_dir and rank == 0:          # before the passes below overwrite the outputs
+        dump_outputs(wl.outputs(), dump_dir)
     # ---- per-kernel pass: the same steps on ONE lane with the library's CUDA-event scopes on, so every kernel is
     # timed alone on the GPU (with several lanes in flight, kernels of different lanes overlap and a per-kernel
     # duration would measure the time-slicing, not the kernel).  The roofline / int_pipe objects come from here.
@@ -953,7 +1001,8 @@ def main():
     ctx = bz.Context(local_rank, stream=stream.cuda_stream)
     wl = WORKLOADS[args.workload](args)
     wl.setup(ctx, rank)
-    line = measure(args, wl, ctx, stream, rank, world, local_rank, want_cpu=(rank == 0 and not os.environ.get("BZ_NO_CPU_BASELINE")))
+    line = measure(args, wl, ctx, stream, rank, world, local_rank, want_cpu=(rank == 0 and not os.environ.get("BZ_NO_CPU_BASELINE")),
+                   dump_dir=args.dump_outputs)
     if line is not None:
         line["config"] = config_for(wl, sched)
         if getattr(wl, "setup_info", None):

@@ -38,3 +38,25 @@ def test_both_arms_share_the_config_dict():
         args.workload = name
         a, b = bench.WORKLOADS[name](args), bench.WORKLOADS[name](args)
         assert bench.config_for(a) == bench.config_for(b) and "workload" in bench.config_for(a)
+
+
+def test_dump_outputs_exact_bytes_and_a_seeded_sample_within_the_limit(tmp_path, monkeypatch):
+    """--dump-outputs: every item's bytes exactly in float32; over the size limit, the same seeded sample of whole items."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    small = np.arange(3 * 4, dtype=np.uint64).reshape(3, 4) * 0x0102030405060708
+    bench.dump_outputs({"small": small}, str(tmp_path / "a"))
+    got = np.load(tmp_path / "a" / "small.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small.view(np.uint8).reshape(3, 32))
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 1 << 16)
+    big = np.repeat(np.arange(4000, dtype="<u2")[:, None], 8, axis=1)               # item i: 16 bytes that encode i
+    other = np.arange(4000 * 2, dtype=np.uint32).reshape(4000, 2)
+    for d in ("b", "c"):
+        bench.dump_outputs({"big": big, "other": other}, str(tmp_path / d))
+    files = sorted((tmp_path / "b").iterdir())
+    assert sum(f.stat().st_size for f in files) <= 1 << 16
+    rows = np.load(tmp_path / "b" / "big.npy").astype(np.uint8).view("<u2")
+    assert 0 < len(rows) < 4000 and (rows == rows[:, :1]).all() and (np.diff(rows[:, 0]) > 0).all()
+    for f in files:
+        assert np.array_equal(np.load(f), np.load(tmp_path / "c" / f.name))
