@@ -10,21 +10,9 @@ import random
 import numpy as np
 import pytest
 from battlezips_halo2_b200 import arithmetic as ar
-from battlezips_halo2_b200.binding import _np_ptr
+from tests.util_msm import urs_points as _urs_points
 
 pytestmark = pytest.mark.gpu
-
-
-def _urs_points(ctx, co, curve, n):
-    msgs = np.zeros((n, 5), dtype=np.uint8)
-    msgs[:, 1:] = np.arange(n, dtype="<u4").view(np.uint8).reshape(n, 4)
-    out = np.zeros((n, 8), dtype=np.uint64)
-    ctx._check(ctx.lib.bz_hash_to_curve(ctx.h, curve, b"Halo2-Parameters", _np_ptr(msgs), 5, n, _np_ptr(out)))
-    C = co.CURVES[curve][0]
-    h = C.hash_to_curve("Halo2-Parameters")
-    for i in (0, 1, n // 2 + 3, n - 1):
-        assert co.points_from_mont(curve, out[i][None, :])[0] == h(b"\x00" + int(i).to_bytes(4, "little")), i
-    return out
 
 
 def _scalars(co, curve, n, kind, seed):
