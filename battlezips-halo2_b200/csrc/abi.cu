@@ -42,22 +42,12 @@ __attribute__((visibility("default"))) int bz_ctx_create(int device, void* strea
   bz_ctx* h = new (std::nothrow) bz_ctx();
   if (!h) return BZ_ERR_INVALID;
   h->c.device = device;
-  int prio_lo = 0, prio_hi = 0;          // numerically lowest = highest priority
-  cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-  const char* se = getenv("BZ_SPLIT_STREAMS");
-  const bool split = se && atoi(se) != 0;
   if (stream) h->c.stream = (cudaStream_t)stream;
   else {
-    if (cudaStreamCreateWithPriority(&h->c.stream, cudaStreamNonBlocking, split ? prio_hi : prio_lo) != cudaSuccess) { delete h; return BZ_ERR_CUDA; }
+    if (cudaStreamCreateWithFlags(&h->c.stream, cudaStreamNonBlocking) != cudaSuccess) { delete h; return BZ_ERR_CUDA; }
     h->own_stream = true;
   }
-  if (split) {
-    if (cudaStreamCreateWithPriority(&h->c.big, cudaStreamNonBlocking, prio_lo) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->c.ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->c.ev_join, cudaEventDisableTiming) != cudaSuccess) { delete h; return BZ_ERR_CUDA; }
-  }
   cudaDeviceGetAttribute(&h->c.sm_count, cudaDevAttrMultiProcessorCount, device);
-  { const char* pe = getenv("BZ_FB_PAIRS"); h->c.fb_pairs = pe && atoi(pe) != 0; }
   *out = h;
   return BZ_OK;
 }
@@ -67,7 +57,6 @@ __attribute__((visibility("default"))) void bz_ctx_destroy(bz_ctx* ctx) {
   cudaSetDevice(ctx->c.device);
   cudaStreamSynchronize(ctx->c.stream);
   for (void* p : ctx->allocs) cudaFree(p);
-  if (ctx->c.big) { cudaStreamSynchronize(ctx->c.big); cudaStreamDestroy(ctx->c.big); cudaEventDestroy(ctx->c.ev_fork); cudaEventDestroy(ctx->c.ev_join); }
   if (ctx->own_stream) cudaStreamDestroy(ctx->c.stream);
   delete ctx;
 }

@@ -77,7 +77,7 @@ enum ProfTag { PROF_NTT_PASS = 0, PROF_MSM_DIGITS, PROF_MSM_SORT, PROF_MSM_BUCKE
                PROF_FIXED_MSM, PROF_QUOTIENT, PROF_SCAN, PROF_EVAL, PROF_POLY, PROF_IPA, PROF_OTHER, PROF_NTAGS };
 struct ProfRec { cudaEvent_t a, b; int tag; };
 
-// One context = one GPU + one stream family.  Callable from one thread at a time (SURVEY §8b).
+// One context = one GPU + one stream.  Callable from one thread at a time (SURVEY §8b).
 struct Ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -93,17 +93,10 @@ struct Ctx {
   DevBuf stage[6];         // device staging of the host-buffer entry points (kept across calls: no cudaMalloc/cudaFree per call)
   uint64_t kernel_launches = 0;   // counted by every launch site (bench.py's gpu_launches)
   bool profiling = false;
-  bool fb_pairs = false;   // BZ_FB_PAIRS=1 at context creation: pair mode of the table MSM (fixedmsm.cu; measured slower, kept for A/B)
   DevBuf counters;        // [0] = mixed additions done by fixed_msm_kernel while profiling
   std::vector<ProfRec> prof;
   double prof_ms[PROF_NTAGS] = {0};
   uint64_t prof_count[PROF_NTAGS] = {0};
-
-  // Throughput kernels (table-MSM accumulation, h(X), NTT passes) go to a second, LOWEST-priority stream so that the
-  // latency-bound kernels of the other prover lanes (folds, scans, Horner evaluations: a few CTAs each) are dispatched ahead
-  // of a big kernel's pending CTAs instead of queueing behind its last wave (BigKernelScope below; null = one stream).
-  cudaStream_t big = nullptr;
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 
   // One large proof across the GPUs of a box (bz_ctx_set_sharding, SURVEY 8e): every rank runs the same create_proof; the MSMs
   // of a commitment batch are dealt out by column, or split by point range when there are fewer MSMs than ranks, and the
@@ -114,25 +107,6 @@ struct Ctx {
 
   const bzh::Field& field(int f) const { return f == 0 ? fp : fq; }
   ~Ctx();
-};
-
-// Launch the kernels issued inside the scope on ctx->big, ordered after everything already on ctx->stream and before
-// everything issued to it afterwards (two event edges; no host synchronisation).
-struct BigKernelScope {
-  Ctx* c; cudaStream_t s;
-  explicit BigKernelScope(Ctx* ctx) : c(ctx), s(ctx->stream) {
-    if (!c->big) return;
-    cudaEventRecord(c->ev_fork, c->stream);
-    cudaStreamWaitEvent(c->big, c->ev_fork, 0);
-    s = c->big;
-  }
-  ~BigKernelScope() {
-    if (!c->big) return;
-    cudaEventRecord(c->ev_join, c->big);
-    cudaStreamWaitEvent(c->stream, c->ev_join, 0);
-  }
-  BigKernelScope(const BigKernelScope&) = delete;
-  BigKernelScope& operator=(const BigKernelScope&) = delete;
 };
 
 // NVTX range (header-only nvtx3; a no-op unless a profiler is attached): prover phases and kernel classes show up by name

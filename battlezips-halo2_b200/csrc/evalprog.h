@@ -43,7 +43,7 @@ struct Token { uint32_t op, a; int32_t b; };
 // proving key on the extended coset -- and the gate polynomial queries it like a fixed column in slot base_slot + j.
 // Same value at every point, so h(X) does not change.  `degree` keeps the true degree for the evaluation tiers.
 struct DerivedColumn { std::vector<Token> tokens; uint32_t degree; };
-inline void split_fixed_subexpressions(const std::vector<Token>& tokens, const std::vector<uint32_t>& gate_off, uint32_t base_slot, bool enabled,
+inline void split_fixed_subexpressions(const std::vector<Token>& tokens, const std::vector<uint32_t>& gate_off, uint32_t base_slot,
                                        std::vector<DerivedColumn>& derived, std::vector<Token>& qtokens, std::vector<uint32_t>& qgate_off) {
   struct Node { Token t; int x = -1, y = -1; bool fixed_only = false, has_mul = false; uint32_t degree = 0; };
   std::map<std::vector<uint32_t>, uint32_t> index;
@@ -74,11 +74,11 @@ inline void split_fixed_subexpressions(const std::vector<Token>& tokens, const s
     BZ_EP_CHECK(st.size() == 1, "bad expression");
     struct Walk {
       const std::vector<Node>& nodes; std::map<std::vector<uint32_t>, uint32_t>& index; std::vector<DerivedColumn>& derived; std::vector<Token>& out;
-      uint32_t base_slot; bool enabled;
+      uint32_t base_slot;
       void flat(int v, std::vector<Token>& o) const { const Node& n = nodes[v]; if (n.x >= 0) flat(n.x, o); if (n.y >= 0) flat(n.y, o); o.push_back(n.t); }
       void emit(int v) {
         const Node& n = nodes[v];
-        if (enabled && n.fixed_only && n.has_mul && n.degree >= 2) {
+        if (n.fixed_only && n.has_mul && n.degree >= 2) {
           std::vector<Token> sub; flat(v, sub);
           std::vector<uint32_t> key;
           for (const Token& k : sub) { key.push_back(k.op); key.push_back(k.a); key.push_back((uint32_t)k.b); }
@@ -91,7 +91,7 @@ inline void split_fixed_subexpressions(const std::vector<Token>& tokens, const s
         if (n.y >= 0) emit(n.y);
         out.push_back(n.t);
       }
-    } walk{nodes, index, derived, qtokens, base_slot, enabled};
+    } walk{nodes, index, derived, qtokens, base_slot};
     walk.emit(st.back());
     qgate_off.push_back((uint32_t)qtokens.size());
   }

@@ -7,7 +7,7 @@
 // once per Params (affine, 64 B per entry; a few GB).  A commitment is then a flat sum of at most
 // ceil(256/c) * (n+1) table entries: no buckets, no sorting, no doublings, no bucket reduction, and
 // zero digits (witness columns are mostly 0/1) cost nothing.  One launch commits a whole batch of
-// polynomials: grid = (chunks, #msm).  All arithmetic is IMAD-pipe Montgomery work in XYZZ coordinates.
+// polynomials.  All arithmetic is IMAD-pipe Montgomery work in XYZZ coordinates.
 #include "common.h"
 #include "curve.cuh"
 #include "fixedmsm.h"
@@ -265,140 +265,6 @@ __global__ void __launch_bounds__(FB_THREADS, 4) fb_accumulate_kernel(const Affi
   }
 }
 
-// ---- pair mode (BZ_FB_PAIRS=1; A/B against the kernel above) ------------------------------------------------------
-// Two consecutive table points of a lane's share are first added in AFFINE coordinates -- lambda = (y_b - y_a)/(x_b - x_a):
-// 3 multiplications once 1/(x_b - x_a) is known -- and only their sum goes through the 10-multiplication mixed addition:
-// 8 multiplications per table point instead of 10.  The denominators of ALL pairs of a thread share one inversion
-// (Montgomery's trick across three kernels, because a Fermat chain is ~380 dependent multiplications on one lane and would
-// cost more issue slots than the pairs save if every warp ran its own):
-//   A  fb_pair_prefix_kernel      walks the thread's pairs LAST to FIRST, stores the running product of the denominators
-//                                 seen so far next to every pair and the thread's total at the end
-//   B  batch_invert_kernel        (elementwise.cu) inverts the per-thread totals, 16 per Fermat chain
-//   C  fb_accumulate_pairs_kernel walks the pairs FIRST to LAST:  1/d_k = inv * stored_k,  inv *= d_k
-// A pair with x_a = x_b (same or opposite points) or with a zero x (the identity's encoding) is not added in affine form:
-// both points go through the complete mixed addition one after the other, so every input the kernel above handles is
-// handled here with the same result.
-template <class BP> __device__ __forceinline__ bool fb_pair_ok(const Fe<BP>& xa, const Fe<BP>& xb, Fe<BP>& d) {
-  d = fe_sub(xb, xa);
-  return !(fe_is_zero(xa) || fe_is_zero(xb) || fe_is_zero(d));
-}
-// out-of-line complete mixed addition for the rare / once-per-piece cases (keeps the hot loop's code small)
-template <class BP> __device__ __noinline__ void fb_add_mixed_slow(Xyzz<BP>& acc, const Affine<BP>& q) { xyzz_add_mixed(acc, q); }
-// entries of lane `lane` in the piece [pb, pe): pb + lane + 32 j, j < count
-__device__ __forceinline__ uint32_t fb_lane_count(uint32_t pb, uint32_t pe, uint32_t lane) { return pe > pb + lane ? (pe - pb - lane + 31u) >> 5 : 0u; }
-
-template <class BP>
-__global__ void __launch_bounds__(FB_THREADS) fb_pair_prefix_kernel(const Affine<BP>* __restrict__ table, const uint32_t* __restrict__ lists,
-                                 uint32_t list_stride, const uint32_t* __restrict__ list_count, uint32_t n_msm,
-                                 Fe<BP>* __restrict__ pre, Fe<BP>* __restrict__ totals) {
-  extern __shared__ uint32_t fb_off[];
-  __shared__ uint32_t wsum[33];
-  const uint32_t T = gridDim.x * FB_THREADS, t = blockIdx.x * FB_THREADS + threadIdx.x, lane = threadIdx.x & 31, W = t >> 5;
-  const uint32_t q = fb_plan(list_count, n_msm, T, fb_off, wsum);
-  const uint32_t total = fb_off[n_msm];
-  const uint64_t base64 = (uint64_t)W * 32u * q;
-  Fe<BP> prod = fe_one<BP>();
-  if (base64 < total) {
-    const uint32_t base = (uint32_t)base64, end = (uint32_t)min((uint64_t)total, base64 + (uint64_t)32 * q);
-    uint32_t lo = 0, hi = n_msm;                     // m_lo = last MSM with off[m] <= base
-    while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (fb_off[mid] <= base) lo = mid; else hi = mid; }
-    const uint32_t m_lo = lo;
-    lo = m_lo; hi = n_msm;                           // m_hi = last MSM with off[m] < end
-    while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (fb_off[mid] < end) lo = mid; else hi = mid; }
-    const uint32_t m_hi = lo;
-    uint32_t k = 0;                                  // number of pairs of this thread
-    for (uint32_t m = m_lo; m <= m_hi; ++m) k += fb_lane_count(max(base, fb_off[m]), min(end, fb_off[m + 1]), lane) >> 1;
-    for (uint32_t m = m_hi + 1; m-- > m_lo;) {
-      const uint32_t pb = max(base, fb_off[m]), pe = min(end, fb_off[m + 1]);
-      const uint32_t npair = fb_lane_count(pb, pe, lane) >> 1;
-      if (!npair) continue;
-      const uint32_t* list = lists + (size_t)m * list_stride - fb_off[m];
-      uint32_t p = pb + lane + 64u * (npair - 1);
-      uint32_t ea = list[p], eb = list[p + 32];
-      for (uint32_t j = npair; j-- > 0;) {
-        const Fe<BP> xa = fe_load(&table[ea & 0x7fffffffu].x), xb = fe_load(&table[eb & 0x7fffffffu].x);
-        if (j) { p -= 64u; ea = list[p]; eb = list[p + 32]; }
-        --k;
-        Fe<BP> d;
-        if (fb_pair_ok(xa, xb, d)) { fe_store(pre + (size_t)k * T + t, prod); prod = fe_mul(prod, d); }
-      }
-    }
-  }
-  fe_store(totals + t, prod);
-}
-
-template <class BP>
-__global__ void __launch_bounds__(FB_THREADS, 3) fb_accumulate_pairs_kernel(const Affine<BP>* __restrict__ table, const uint32_t* __restrict__ lists,
-                                 uint32_t list_stride, const uint32_t* __restrict__ list_count, uint32_t n_msm,
-                                 const Fe<BP>* __restrict__ pre, const Fe<BP>* __restrict__ inv_totals,
-                                 Xyzz<BP>* __restrict__ partial, unsigned long long* __restrict__ add_counter) {
-  extern __shared__ uint32_t fb_off[];
-  __shared__ uint32_t wsum[33];
-  const uint32_t T = gridDim.x * FB_THREADS, t = blockIdx.x * FB_THREADS + threadIdx.x, lane = threadIdx.x & 31, W = t >> 5;
-  const uint32_t q = fb_plan(list_count, n_msm, T, fb_off, wsum);
-  const uint32_t total = fb_off[n_msm];
-  const uint64_t base64 = (uint64_t)W * 32u * q;
-  uint32_t my_adds = 0;
-  if (base64 < total) {
-    const uint32_t base = (uint32_t)base64, end = (uint32_t)min((uint64_t)total, base64 + (uint64_t)32 * q);
-    uint32_t lo = 0, hi = n_msm;
-    while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (fb_off[mid] <= base) lo = mid; else hi = mid; }
-    uint32_t m = lo, pbeg = base, k = 0;
-    Fe<BP> inv = fe_load(inv_totals + t);
-    while (pbeg < end) {
-      while (fb_off[m + 1] <= pbeg) ++m;
-      const uint32_t pend = min(end, fb_off[m + 1]);
-      const uint32_t* list = lists + (size_t)m * list_stride - fb_off[m];
-      const uint32_t cnt = fb_lane_count(pbeg, pend, lane), npair = cnt >> 1;
-      Xyzz<BP> acc = xyzz_identity<BP>();
-      uint32_t p = pbeg + lane;
-      uint32_t ea = 0, eb = 0;
-      Affine<BP> pa, pb;
-      if (npair) { ea = list[p]; eb = list[p + 32]; pa = aff_load(table + (ea & 0x7fffffffu)); pb = aff_load(table + (eb & 0x7fffffffu)); }
-      for (uint32_t j = 0; j < npair; ++j) {
-        const bool more = j + 1 < npair;
-        uint32_t ea_n = 0, eb_n = 0;
-        Affine<BP> pa_n, pb_n;
-        if (more) { ea_n = list[p + 64]; eb_n = list[p + 96]; pa_n = aff_load(table + (ea_n & 0x7fffffffu)); pb_n = aff_load(table + (eb_n & 0x7fffffffu)); }
-        if (ea >> 31) pa.y = fe_neg(pa.y);
-        if (eb >> 31) pb.y = fe_neg(pb.y);
-        Fe<BP> d;
-        Affine<BP> s;
-        if (fb_pair_ok(pa.x, pb.x, d)) {
-          const Fe<BP> invd = fe_mul(inv, fe_load(pre + (size_t)k * T + t));
-          inv = fe_mul(inv, d);
-          const Fe<BP> lam = fe_mul(fe_sub(pb.y, pa.y), invd);
-          s.x = fe_sub(fe_sub(fe_sqr(lam), pa.x), pb.x);
-          s.y = fe_sub(fe_mul(lam, fe_sub(pa.x, s.x)), pa.y);
-        } else {
-          fb_add_mixed_slow(acc, pa);
-          s = pb;
-        }
-        xyzz_add_mixed(acc, s);
-        my_adds += 2;
-        ++k;
-        if (more) { pa = pa_n; pb = pb_n; }
-        ea = ea_n; eb = eb_n;
-        p += 64;
-      }
-      if (cnt & 1) {
-        const uint32_t ent = list[p];
-        Affine<BP> pt = aff_load(table + (ent & 0x7fffffffu));
-        if (ent >> 31) pt.y = fe_neg(pt.y);
-        fb_add_mixed_slow(acc, pt);
-        ++my_adds;
-      }
-      Xyzz<BP>* o = partial + ((size_t)W + m) * 32 + lane;
-      fe_store(&o->x, acc.x); fe_store(&o->y, acc.y); fe_store(&o->zz, acc.zz); fe_store(&o->zzz, acc.zzz);
-      pbeg = pend;
-    }
-  }
-  if (add_counter) {
-    uint32_t tot = __reduce_add_sync(0xffffffffu, my_adds);
-    if ((threadIdx.x & 31) == 0 && tot) atomicAdd(add_counter, (unsigned long long)tot);
-  }
-}
-
 // fold the partials of each MSM and normalise: one CTA per MSM -> affine (64 B), identity = zeros
 template <class BP, bool XYZZ_OUT, int THREADS>
 __global__ void __launch_bounds__(THREADS) fb_fold_kernel(const Xyzz<BP>* __restrict__ partial, const uint32_t* __restrict__ list_count,
@@ -497,24 +363,17 @@ __global__ void __launch_bounds__(64) fb_fold_slices_kernel(const Xyzz<BP>* __re
   }
 }
 
-void field_op_run(Ctx* ctx, int field, int op, const void* a, const void* b, void* out, uint64_t n);      // elementwise.cu (op 3 = batch inversion)
-
 template <class BP, class SP>
 static void fixed_msm_run_t(Ctx* ctx, const FixedBase& fb, const void* const* d_main, uint32_t n_main, const void* const* d_extra,
-                            uint32_t n_msm, uint32_t /*chunks*/, void* d_out, bool xyzz_out) {
+                            uint32_t n_msm, void* d_out, bool xyzz_out) {
   cudaStream_t st = ctx->stream;
   if (!ctx->counters.p) { ctx->counters.alloc(64); BZ_CUDA(cudaMemsetAsync(ctx->counters.p, 0, 64, st)); }
   const uint32_t list_stride = fb.npts * fb.W;                          // worst case: every digit non-zero
-  static int ctas_dev[BZ_MAX_DEVICES], ctas_pairs_dev[BZ_MAX_DEVICES];   // per template instantiation and device; several prover lanes (host threads) may race to set them
+  static int ctas_dev[BZ_MAX_DEVICES];   // per template instantiation and device; several prover lanes (host threads) may race to set them
   static PerDeviceOnce once;
   const int dev = ctx->device >= 0 && ctx->device < BZ_MAX_DEVICES ? ctx->device : 0;
   once.run(ctx->device, [dev] {
-    int ctas_per_sm = 0, ctas_per_sm_pairs = 0;
-    cudaFuncSetAttribute(fb_accumulate_pairs_kernel<BP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((FB_MAX_MSM + 1) * 4));
-    cudaFuncSetAttribute(fb_pair_prefix_kernel<BP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((FB_MAX_MSM + 1) * 4));
-    int vp = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&vp, fb_accumulate_pairs_kernel<BP>, FB_THREADS, (FB_MAX_MSM + 1) * 4);
-    ctas_per_sm_pairs = vp < 1 ? 1 : vp;
+    int ctas_per_sm = 0;
     cudaFuncSetAttribute(fb_accumulate_kernel<BP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((FB_MAX_MSM + 1) * 4));
     int v = 0;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, fb_accumulate_kernel<BP>, FB_THREADS, (FB_MAX_MSM + 1) * 4);
@@ -526,12 +385,9 @@ static void fixed_msm_run_t(Ctx* ctx, const FixedBase& fb, const void* const* d_
     cudaFuncSetAttribute(fb_fold_kernel<BP, false, FB_FOLD_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, fold_smem);
     // BZ_FB_CTAS_PER_SM: fewer resident CTAs of the accumulate wave than fit (A/B: leaves registers for the other prover lanes' kernels)
     if (const char* e = getenv("BZ_FB_CTAS_PER_SM")) { const int v2 = atoi(e); if (v2 >= 1 && v2 < ctas_per_sm) ctas_per_sm = v2; }
-    ctas_dev[dev] = ctas_per_sm; ctas_pairs_dev[dev] = ctas_per_sm_pairs;
+    ctas_dev[dev] = ctas_per_sm;
   });
-  const int ctas_per_sm = ctas_dev[dev], ctas_per_sm_pairs = ctas_pairs_dev[dev];
-  // pair mode needs 32 B of prefix storage per table point: only for launches whose worst case stays under 1 GB
-  const bool pairs = ctx->fb_pairs && (uint64_t)std::min<uint32_t>(n_msm, FB_MAX_MSM) * list_stride <= (1ull << 25);
-  const uint32_t acc_ctas = (uint32_t)ctx->sm_count * (uint32_t)(pairs ? ctas_per_sm_pairs : ctas_per_sm), acc_threads = acc_ctas * FB_THREADS;
+  const uint32_t acc_ctas = (uint32_t)ctx->sm_count * (uint32_t)ctas_dev[dev], acc_threads = acc_ctas * FB_THREADS;
   const uint32_t max_nm = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(FB_MAX_MSM, 0xffffffffull / list_stride));   // flat index fits 32 bits
   for (uint32_t m0 = 0; m0 < n_msm; m0 += max_nm) {
     const uint32_t nm = std::min(max_nm, n_msm - m0);
@@ -548,20 +404,7 @@ static void fixed_msm_run_t(Ctx* ctx, const FixedBase& fb, const void* const* d_
       ProfScope p(ctx, PROF_FIXED_MSM);
       fb_decode_kernel<SP><<<dim3((fb.npts + FB_THREADS - 1) / FB_THREADS, nm), FB_THREADS, 0, st>>>(
           fb.npts, fb.c, fb.W, fb.nbk, (const Fe<SP>* const*)d_main + m0, n_main, d_extra ? (const Fe<SP>* const*)d_extra + m0 : nullptr, lists, list_stride, counts);
-      if (pairs) {
-        const uint64_t q_max = std::max<uint64_t>(FB_MIN_SHARE, ((uint64_t)nm * list_stride + acc_threads - 1) / acc_threads);
-        ctx->scratch[2].ensure((q_max + 2) * (size_t)acc_threads * sizeof(Fe<BP>));
-        Fe<BP>* pre = ctx->scratch[2].as<Fe<BP>>();
-        Fe<BP>* totals = pre + q_max * (size_t)acc_threads;
-        Fe<BP>* inv_totals = totals + acc_threads;
-        fb_pair_prefix_kernel<BP><<<acc_ctas, FB_THREADS, smem, st>>>(fb.table.as<Affine<BP>>(), lists, list_stride, counts, nm, pre, totals);
-        field_op_run(ctx, BP::ID, 3, totals, nullptr, inv_totals, acc_threads);
-        fb_accumulate_pairs_kernel<BP><<<acc_ctas, FB_THREADS, smem, st>>>(fb.table.as<Affine<BP>>(), lists, list_stride, counts, nm, pre, inv_totals, partial, cnt);
-        ctx->kernel_launches += 1;
-      } else {
-        BigKernelScope bigs(ctx);
-        fb_accumulate_kernel<BP><<<acc_ctas, FB_THREADS, smem, bigs.s>>>(fb.table.as<Affine<BP>>(), lists, list_stride, counts, nm, partial, cnt);
-      }
+      fb_accumulate_kernel<BP><<<acc_ctas, FB_THREADS, smem, st>>>(fb.table.as<Affine<BP>>(), lists, list_stride, counts, nm, partial, cnt);
       // fold: offsets + one XYZZ slot per thread in dynamic shared memory.  A launch with many thread partials per MSM (a few large
       // MSMs: one big proof) folds in two levels, G CTAs per MSM first
       const uint64_t pieces_per_msm = ((uint64_t)acc_threads + 32 * (uint64_t)nm) / nm;
@@ -590,12 +433,11 @@ static void fixed_msm_run_t(Ctx* ctx, const FixedBase& fb, const void* const* d_
 }
 
 void fixed_msm_run(Ctx* ctx, const FixedBase& fb, const void* const* d_main, uint32_t n_main, const void* const* d_extra,
-                   uint32_t n_msm, uint32_t chunks, void* d_out, bool xyzz_out) {
+                   uint32_t n_msm, void* d_out, bool xyzz_out) {
   if (!n_msm) return;
   BZ_CHECK(n_main <= fb.npts, "fixed msm: more scalars than table points");
-  if (chunks < 1) chunks = 1;
-  if (fb.curve == 0) fixed_msm_run_t<FqP, FpP>(ctx, fb, d_main, n_main, d_extra, n_msm, chunks, d_out, xyzz_out);
-  else fixed_msm_run_t<FpP, FqP>(ctx, fb, d_main, n_main, d_extra, n_msm, chunks, d_out, xyzz_out);
+  if (fb.curve == 0) fixed_msm_run_t<FqP, FpP>(ctx, fb, d_main, n_main, d_extra, n_msm, d_out, xyzz_out);
+  else fixed_msm_run_t<FpP, FqP>(ctx, fb, d_main, n_main, d_extra, n_msm, d_out, xyzz_out);
 }
 
 }  // namespace bz

@@ -11,5 +11,5 @@ void fixed_base_build(Ctx* ctx, FixedBase& fb, int curve, const void* bases_dev,
 // each), or -- xyzz_out -- the unnormalised XYZZ sums (128 B each: X, Y, ZZ, ZZZ) for callers that normalise on the host
 // (one batched inversion there beats a single-thread Fermat chain per commitment on the device)
 void fixed_msm_run(Ctx* ctx, const FixedBase& fb, const void* const* d_main, uint32_t n_main, const void* const* d_extra,
-                   uint32_t n_msm, uint32_t chunks, void* d_out, bool xyzz_out = false);
+                   uint32_t n_msm, void* d_out, bool xyzz_out = false);
 }  // namespace bz

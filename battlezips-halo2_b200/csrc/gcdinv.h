@@ -2,8 +2,8 @@
 // (both Pasta primes; field.cuh `mod_limb`).  Groundwork for round 2: `fe_inv` is a Fermat chain of ~320 DEPENDENT field
 // multiplications (~77 K instructions, half of them on the fma-heavy pipe every kernel of this library is bound by, and
 // 130 - 180 us of latency on a lone warp); this routine needs ~30 K instructions, practically all of them on the ALU pipe
-// (which sits at ~33 %), so the inversions inside the grand-product finish, the batch-inversion kernels, the table build
-// and the table MSM's pair mode (DESIGN.md section 6) stop competing with the multiplications.  Used through `fe_inv_gcd`
+// (which sits at ~33 %), so the inversions inside the grand-product finish, the batch-inversion kernels and the table build
+// stop competing with the multiplications.  Used through `fe_inv_gcd`
 // (field.cuh) wherever ONE lane inverts while the rest of its warp waits: the grand-product finish, XYZZ / Jacobian ->
 // affine, and `bz_field_op` op 9.  Checked on the CPU (tests/test_gcdinv_host.py runs this very code, compiled for the
 // host, against big-integer inverses) and on the device against the Fermat chain and the oracle

@@ -13,7 +13,6 @@
 // Fusions: zero-padding + zeta^(i mod 3) coset pre-scale on the first pass (coeff_to_extended),
 // N^-1 and zeta^-(i mod 3) post-scale on the last pass (ifft / extended_to_coeff).
 #include "common.h"
-#include <cstdlib>
 #include "field.cuh"
 
 namespace bz {
@@ -191,8 +190,7 @@ template <class P> static void launch_pass(Ctx* ctx, NttPassArgs<P>& a, uint64_t
   once.run(ctx->device, [] { cudaFuncSetAttribute(ntt_pass_kernel<P>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024); });
   dim3 grid((unsigned)(nlines >> a.logT), (unsigned)batch, (unsigned)batch2);
   ProfScope prof(ctx, PROF_NTT_PASS);
-  BigKernelScope bigs(ctx);
-  ntt_pass_kernel<P><<<grid, threads, smem, bigs.s>>>(a);
+  ntt_pass_kernel<P><<<grid, threads, smem, ctx->stream>>>(a);
   ctx->kernel_launches++;
   BZ_CUDA(cudaGetLastError());
 }
@@ -220,8 +218,7 @@ static void ntt_run_t(Ctx* ctx, int field, const Fe<P>* in, Fe<P>* out, int logN
   }
   for (int i = 0; i < 3; ++i) { base.pre[i] = pre[i]; base.post[i] = post[i]; }
 
-  static const int two_pass_max = [] { const char* e = getenv("BZ_NTT_2PASS_MAX"); return e ? atoi(e) : 20; }();      // A/B knob
-  int npass = logN <= 12 ? 1 : (logN <= two_pass_max ? 2 : 3);
+  int npass = logN <= 12 ? 1 : (logN <= 20 ? 2 : 3);      // two passes above 2^20 were probed and dropped (DESIGN.md section 6)
   if (npass == 1) {
     NttPassArgs<P> a = base;
     a.in = in; a.out = out;

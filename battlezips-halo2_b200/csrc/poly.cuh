@@ -407,9 +407,10 @@ __global__ void grand_product_finish_kernel(const Fe<P>* __restrict__ pnum, cons
 // chained through z_s[0] = z_{s-1}[u] (u = first unusable row); the others (lookups) start at 1.
 //   z_g[i] = z0_g * pnum_g[i] * sden_g[i] / sden_g[0],   z0_s = prod_{s' < s} pnum_s'[u] * sden_s'[u] / sden_s'[0]
 // The <= 8 inversions a product needs share one Fermat chain (Montgomery's trick, zeros skipped), so a batch pays the
-// inversion latency once instead of once per product.
+// inversion latency once instead of once per product.  ONE CTA per (proof, product) walks all rows: B x G inversions per batch
+// (launch site in prover.cu).
 struct GpBatchDesc { uint32_t nprod, nsets; PolyRef zref[8]; };
-template <class P, bool NARROW>
+template <class P>
 __global__ void grand_product_finish_batch_kernel(const Fe<P>* __restrict__ pnum, const Fe<P>* __restrict__ sden, uint64_t prod_stride, uint64_t nd_stride,
                                                   Regions reg, GpBatchDesc d, uint32_t n, uint32_t u) {
   __shared__ Fe<P> scale_sh;
@@ -437,17 +438,10 @@ __global__ void grand_product_finish_batch_kernel(const Fe<P>* __restrict__ pnum
     scale_sh = fe_mul(z0, mine);
   }
   __syncthreads();
-  if (!NARROW) {                        // validated geometry: one thread per row, the chain above once per 128 rows
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
+  const Fe<P> scale = scale_sh;
+  for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
     const uint64_t at = (uint64_t)g * prod_stride + (uint64_t)b * nd_stride + i;
-    fe_store(region_ptr<P>(reg, d.zref[g], b, n) + i, fe_mul(fe_mul(fe_load(pnum + at), fe_load(sden + at)), scale_sh));
-  } else {                              // ONE CTA per (proof, product) walks all rows: B x G Fermat chains per batch (launch site in prover.cu)
-    const Fe<P> scale = scale_sh;
-    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
-      const uint64_t at = (uint64_t)g * prod_stride + (uint64_t)b * nd_stride + i;
-      fe_store(region_ptr<P>(reg, d.zref[g], b, n) + i, fe_mul(fe_mul(fe_load(pnum + at), fe_load(sden + at)), scale));
-    }
+    fe_store(region_ptr<P>(reg, d.zref[g], b, n) + i, fe_mul(fe_mul(fe_load(pnum + at), fe_load(sden + at)), scale));
   }
 }
 

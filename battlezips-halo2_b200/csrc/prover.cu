@@ -48,8 +48,7 @@ static void emit_tokens(ProgBuilder& pb, const CircuitCopy& cs, const std::vecto
 static void emit_expr(ProgBuilder& pb, const CircuitCopy& cs, uint32_t lo, uint32_t hi) { emit_tokens(pb, cs, cs.tokens, lo, hi); }
 
 static void derive_fixed_subexpressions(PkImpl& pk) {
-  const char* env = getenv("BZ_QUOTIENT_DERIVED");            // =0: evaluate the compressed selector products per point (A/B)
-  split_fixed_subexpressions(pk.cs.tokens, pk.cs.gate_off, pk.cs.F + pk.M + 5, !(env && atoi(env) == 0), pk.derived, pk.qtokens, pk.qgate_off);
+  split_fixed_subexpressions(pk.cs.tokens, pk.cs.gate_off, pk.cs.F + pk.M + 5, pk.derived, pk.qtokens, pk.qgate_off);
 }
 
 static void emit_compressed(ProgBuilder& pb, const CircuitCopy& cs, const std::vector<std::pair<uint32_t, uint32_t>>& exprs, uint32_t c_theta) {
@@ -92,7 +91,8 @@ static void build_programs(PkImpl& pk) {
   // expr_e / t has degree < (deg_e - 1) n.  Terms with (deg_e - 1) n <= ext_n / 2 are therefore evaluated on every SECOND
   // point of the extended coset only (that is the coset of the half-size domain), interpolated by a half-size inverse NTT
   // and added to the rest in coefficient form: same h(X), about a third fewer field multiplications for Shot / Board.
-  // (For a witness that violates a gate neither variant is a polynomial identity; both proofs are rejected, their bytes differ.)
+  // (For a witness that violates a gate this is not a polynomial identity: the proof differs from that of a single full-coset
+  // evaluation, and both are rejected.)
   {
     struct Term { uint32_t degree; std::function<void(ProgBuilder&)> emit; bool gate = false; uint32_t lo = 0, hi = 0; };
     std::vector<Term> terms;
@@ -153,8 +153,7 @@ static void build_programs(PkImpl& pk) {
       terms.push_back({3, [&pk, a, sp](ProgBuilder& pb) { pb.pp(a, 0); pb.pp(sp, 0); pb.sub(); pb.pp(a, 0); pb.pp(a, -1); pb.sub(); pb.mul(); pb.ps(shslot_active(pk), 0); pb.mul(); }});
     }
     BZ_CHECK(terms.size() == pk.n_exprs, "internal: expression count mismatch");
-    const char* tier_env = getenv("BZ_QUOTIENT_TIERS");
-    const bool tiers = !(tier_env && atoi(tier_env) == 0) && pk.ext_k > cs.k;
+    const bool tiers = pk.ext_k > cs.k;
     // tier of a term: the largest t <= 2 with (deg - 1) n <= ext_n >> t  (and at least n points)
     auto tier_of = [&](uint32_t degree) {
       uint32_t t = 0;
@@ -369,7 +368,7 @@ API int bz_params_commit(bz_ctx* ctx, bz_params* params, int lagrange_basis, con
     void* ptrs[2] = {d_poly.p, d_extra.p};
     BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, ptrs, sizeof(ptrs), cudaMemcpyHostToDevice, st));
     const FixedBase& fb = lagrange_basis ? p.fb_gl : p.fb_g;
-    if (p.use_tables) fixed_msm_run(C, fb, (const void* const*)d_ptrs.p, p.n, (const void* const*)((void**)d_ptrs.p + 1), 1, 16, d_out.p);
+    if (p.use_tables) fixed_msm_run(C, fb, (const void* const*)d_ptrs.p, p.n, (const void* const*)((void**)d_ptrs.p + 1), 1, d_out.p);
     else {
       DevBuf d_in, d_jac; d_in.alloc((size_t)fb.npts * 32); d_jac.alloc(96);
       BZ_CUDA(cudaMemcpyAsync(d_in.p, d_poly.p, (size_t)p.n * 32, cudaMemcpyDeviceToDevice, st));
@@ -405,7 +404,7 @@ API int bz_params_commit_batch_dev(bz_ctx* ctx, bz_params* params, int lagrange_
     for (uint32_t j = 0; j < count; ++j) { ptrs[j] = (char*)d_polys + (size_t)j * p.n * 32; ptrs[count + j] = (char*)d_extra.p + (size_t)j * nextra * 32; }
     BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, ptrs.data(), ptrs.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
     if (p.use_tables) {
-      fixed_msm_run(C, fb, (const void* const*)d_ptrs.p, p.n, (const void* const*)((void**)d_ptrs.p + count), count, 1, d_out_affine);
+      fixed_msm_run(C, fb, (const void* const*)d_ptrs.p, p.n, (const void* const*)((void**)d_ptrs.p + count), count, d_out_affine);
     } else {
       DevBuf& d_jac = C->stage[0];
       d_jac.ensure((size_t)count * 96);
@@ -697,7 +696,7 @@ API int bz_pk_vk_commitments(bz_ctx* ctx, bz_pk* pkh, void* fixed_commitments, v
       if (pr.use_tables) {
         BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, mainp.data(), (size_t)FM * sizeof(void*), cudaMemcpyHostToDevice, st));
         BZ_CUDA(cudaMemcpyAsync((void**)d_ptrs.p + FM, extrap.data(), (size_t)FM * sizeof(void*), cudaMemcpyHostToDevice, st));
-        fixed_msm_run(C, pr.fb_gl, (const void* const*)d_ptrs.p, n, (const void* const*)((void**)d_ptrs.p + FM), FM, 1, d_out.p);
+        fixed_msm_run(C, pr.fb_gl, (const void* const*)d_ptrs.p, n, (const void* const*)((void**)d_ptrs.p + FM), FM, d_out.p);
       } else {
         DevBuf d_in, d_jac;
         d_in.alloc((size_t)(n + 1) * 32); d_jac.alloc((size_t)FM * 96);
@@ -815,19 +814,18 @@ struct Prover {
     if (pk.params->use_tables) {
       BZ_CUDA(cudaMemcpyAsync(w.ptrs.p, mainp.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
       BZ_CUDA(cudaMemcpyAsync((void**)w.ptrs.p + n_msm, extrap.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
-      uint32_t chunks = std::max(1u, std::min(16u, (uint32_t)(4 * C->sm_count / std::max(1u, n_msm))));
       if (world > 1 && n_msm >= world) {
         // one large proof across GPUs, table path: rank r sums the contiguous MSMs [r * per, (r + 1) * per) and the 128-byte
         // XYZZ results are all-gathered (every rank holds the same tables); fewer MSMs than ranks are computed redundantly
         const uint32_t per = (n_msm + world - 1) / world, lo = std::min(n_msm, rank * per), hi = std::min(n_msm, lo + per);
         BZ_CHECK((size_t)per * 128 <= C->shard_cap, "sharding exchange buffer too small");
         BZ_CUDA(cudaMemsetAsync(C->shard_send, 0, (size_t)per * 128, st));
-        if (hi > lo) fixed_msm_run(C, fb, (const void* const*)w.ptrs.p + lo, n, (const void* const*)((void**)w.ptrs.p + n_msm) + lo, hi - lo, chunks, C->shard_send, true);
+        if (hi > lo) fixed_msm_run(C, fb, (const void* const*)w.ptrs.p + lo, n, (const void* const*)((void**)w.ptrs.p + n_msm) + lo, hi - lo, C->shard_send, true);
         if (C->shard_exchange(C->shard_user, (size_t)per * 128) != 0) throw Error(BZ_ERR_CUDA, "sharding: all-gather callback failed");
         BZ_CUDA(cudaMemcpyAsync(w.commits.p, C->shard_recv, (size_t)n_msm * 128, cudaMemcpyDeviceToDevice, st));
         return;
       }
-      fixed_msm_run(C, fb, (const void* const*)w.ptrs.p, n, (const void* const*)((void**)w.ptrs.p + n_msm), n_msm, chunks, w.commits.p, true);
+      fixed_msm_run(C, fb, (const void* const*)w.ptrs.p, n, (const void* const*)((void**)w.ptrs.p + n_msm), n_msm, w.commits.p, true);
       return;
     }
     // bucket MSM (k >= 20, or forced): the MSMs of the call go through the sort / accumulate / reduce pipeline as ONE batch
@@ -984,12 +982,11 @@ void Prover::compute_h() {
     const bool split = world > 1 && B == 1 && (en >> (PkImpl::Q_TIERS - 1)) >= 128u * world && (en >> (PkImpl::Q_TIERS - 1)) % world == 0 && slice_bytes <= C->shard_cap;
     {
       ProfScope prof(C, PROF_QUOTIENT);
-      BigKernelScope bigs(C);
       auto launch = [&](uint32_t t, EvalArgs<FpP> args, uint32_t points) {
         if (split) { points /= world; args.first = rank * points; }
         const dim3 grid((points + 127) / 128, B);
-        if (pk.q_gen[t]) pk.q_gen[t](args, grid, bigs.s);                   // circuit-specialised straight-line code (gen_quotient.cu)
-        else eval_program_kernel<FpP><<<grid, 128, pk.q_ninstr[t] * 4, bigs.s>>>(args);
+        if (pk.q_gen[t]) pk.q_gen[t](args, grid, st);                   // circuit-specialised straight-line code (gen_quotient.cu)
+        else eval_program_kernel<FpP><<<grid, 128, pk.q_ninstr[t] * 4, st>>>(args);
         C->kernel_launches++;
       };
       launch(0, a, en);
@@ -1137,9 +1134,7 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
       eval_program_kernel<FpP><<<dim3((n + 127) / 128, B), 128, pk.lk_ninstr * 4, st>>>(a);
       C->kernel_launches++;
     }
-    const bool device_permute = !getenv("BZ_LOOKUP_HOST");      // the host permutation is kept for A/B checks only
-    std::vector<HFe> up;
-    if (device_permute && n > LKP_MAX_N) {
+    if (n > LKP_MAX_N) {
       // large domains: device-wide radix sort / scans per (proof, lookup) (lookup.cu)
       BZ_CUDA(cudaMemsetAsync(w.lk_err.p, 0, (size_t)B * 4, st));
       ProfScope prof(C, PROF_SCAN);
@@ -1147,7 +1142,7 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
         for (uint32_t l = 0; l < L; ++l)
           lookup_permute_large_run(C, misc(b, pk.m_cin0 + 2 * l), misc(b, pk.m_cin0 + 2 * l + 1), val(b, pk.slot_lk(l, 0)), val(b, pk.slot_lk(l, 1)), usable, (uint32_t*)w.lk_err.p + b);
       BZ_CUDA(cudaMemcpyAsync(w.h_err, w.lk_err.p, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
-    } else if (device_permute) {
+    } else {
       // device: sort / permute (U: lookup/prover.rs::permute_expression_pair), one CTA per (lookup, proof)
       static PerDeviceOnce once;
       once.run(C->device, [] { cudaFuncSetAttribute(lookup_permute_kernel<FpP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lookup_permute_smem(LKP_MAX_N)); });
@@ -1162,46 +1157,6 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
         C->kernel_launches++;
       }
       BZ_CUDA(cudaMemcpyAsync(w.h_err, w.lk_err.p, (size_t)B * 4, cudaMemcpyDeviceToHost, st));     // read after the commitments' sync below
-    } else {
-      // host: sort / permute (U: lookup/prover.rs::permute_expression_pair)
-      const size_t per = (size_t)2 * L * n * 32;
-      BZ_CHECK((size_t)B * per <= w.h_pinned_bytes, "pinned staging too small");
-      for (uint32_t b = 0; b < B; ++b) BZ_CUDA(cudaMemcpyAsync((char*)w.h_pinned + b * per, misc(b, pk.m_cin0), per, cudaMemcpyDeviceToHost, st));
-      BZ_CUDA(cudaStreamSynchronize(st));
-      up.assign((size_t)B * L * 2 * n, F.zero());
-      for (uint32_t b = 0; b < B; ++b)
-        for (uint32_t l = 0; l < L; ++l) {
-          const HFe* cinp = (const HFe*)((char*)w.h_pinned + b * per) + (size_t)(2 * l) * n;
-          const HFe* ctab = cinp + n;
-          struct Key { std::array<uint64_t, 4> v; uint32_t idx; };
-          auto canon = [&](const HFe& x) { std::array<uint64_t, 4> r; F.to_raw(x, r.data()); return r; };
-          auto less = [](const std::array<uint64_t, 4>& a, const std::array<uint64_t, 4>& c) { for (int i = 3; i >= 0; --i) { if (a[i] != c[i]) return a[i] < c[i]; } return false; };
-          std::vector<Key> a(usable);
-          for (uint32_t i = 0; i < usable; ++i) a[i] = Key{canon(cinp[i]), i};
-          std::stable_sort(a.begin(), a.end(), [&](const Key& x, const Key& y) { return less(x.v, y.v); });
-          std::map<std::array<uint64_t, 4>, std::pair<uint32_t, HFe>, decltype(less)> leftover(less);
-          for (uint32_t i = 0; i < usable; ++i) { auto key = canon(ctab[i]); auto it = leftover.find(key); if (it == leftover.end()) leftover.emplace(key, std::make_pair(1u, ctab[i])); else it->second.first++; }
-          HFe* ap = &up[((size_t)b * L + l) * 2 * n];
-          HFe* sp = ap + n;
-          std::vector<uint32_t> repeated;
-          for (uint32_t row = 0; row < usable; ++row) {
-            ap[row] = cinp[a[row].idx];
-            if (row == 0 || a[row].v != a[row - 1].v) {
-              sp[row] = ap[row];
-              auto it = leftover.find(a[row].v);
-              if (it == leftover.end() || it->second.first == 0) throw Error(BZ_ERR_SYNTHESIS, "lookup input not in table (Error::ConstraintSystemFailure)");
-              it->second.first--;
-            } else repeated.push_back(row);
-          }
-          for (auto& kv : leftover)
-            for (uint32_t c = 0; c < kv.second.first; ++c) { BZ_CHECK(!repeated.empty(), "lookup permutation underflow"); sp[repeated.back()] = kv.second.second; repeated.pop_back(); }
-          BZ_CHECK(repeated.empty(), "lookup permutation leftover");
-        }
-      for (uint32_t b = 0; b < B; ++b)
-        for (uint32_t l = 0; l < L; ++l) {
-          BZ_CUDA(cudaMemcpyAsync(val(b, pk.slot_lk(l, 0)), &up[((size_t)b * L + l) * 2 * n], (size_t)n * 32, cudaMemcpyHostToDevice, st));
-          BZ_CUDA(cudaMemcpyAsync(val(b, pk.slot_lk(l, 1)), &up[((size_t)b * L + l) * 2 * n + n], (size_t)n * 32, cudaMemcpyHostToDevice, st));
-        }
     }
     std::vector<CopyDesc> cd;
     std::vector<CommitReq> reqs;
@@ -1219,11 +1174,9 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
       }
     }
     launch_copy(cd, n);
-    if (!device_permute) BZ_CUDA(cudaStreamSynchronize(st));      // `up` must outlive the async copies
     commit(reqs, bl, pts);
-    if (device_permute)
-      for (uint32_t b = 0; b < B; ++b)
-        if (w.h_err[b]) throw Error(BZ_ERR_SYNTHESIS, "lookup input not in table (Error::ConstraintSystemFailure) in proof " + std::to_string(b) + " of the batch");
+    for (uint32_t b = 0; b < B; ++b)
+      if (w.h_err[b]) throw Error(BZ_ERR_SYNTHESIS, "lookup input not in table (Error::ConstraintSystemFailure) in proof " + std::to_string(b) + " of the batch");
     for (uint32_t b = 0; b < B; ++b) for (uint32_t j = 0; j < 2 * L; ++j) t_write_point(ps[b], pts[b][j]);
   }
   // ---- step 6
@@ -1280,10 +1233,8 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
         product_scan_kernel<FpP><<<dim3(1, NG * B), SCAN_THREADS, 0, st>>>(den, sden, n, n, 1);
         // One CTA per (proof, product), i.e. B x NG inversions per batch instead of one per 128 rows (the r1h launch list shows
         // the 3 072 single-lane chains of the wide geometry costing the fma pipe as much as an IPA-round MSM; r2 A/B on B200:
-        // scan scope 5.77 -> 2.78 ms per 5 x 64 proofs, Shot 3 469 -> 3 600 proofs/s).  BZ_GP_FINISH_NARROW=0 selects the wide geometry.
-        const bool narrow = [] { const char* e = getenv("BZ_GP_FINISH_NARROW"); return !(e && atoi(e) == 0); }();
-        if (narrow) grand_product_finish_batch_kernel<FpP, true><<<dim3(1, B, NG), 256, 0, st>>>(pnum, sden, PS, n, reg, gd, n, n - (bf + 1));
-        else grand_product_finish_batch_kernel<FpP, false><<<dim3((n + 127) / 128, B, NG), 128, 0, st>>>(pnum, sden, PS, n, reg, gd, n, n - (bf + 1));
+        // scan scope 5.77 -> 2.78 ms per 5 x 64 proofs, Shot 3 469 -> 3 600 proofs/s).
+        grand_product_finish_batch_kernel<FpP><<<dim3(1, B, NG), 256, 0, st>>>(pnum, sden, PS, n, reg, gd, n, n - (bf + 1));
         C->kernel_launches += NG + 3;
       }
       launch_copy(cd, n);
@@ -1723,7 +1674,7 @@ API int bz_ipa_round(bz_ctx* ctx, bz_ipa* ipa, const void* z, const void* l_rand
                                                     (const DFe*)ipa->rnd.p, 0, 0, 1, (DFe*)ipa->extras.p);
     C->kernel_launches += 2;
     ParamsImpl& pr = *ipa->params;
-    if (pr.use_tables) fixed_msm_run(C, pr.fb_g, (const void* const*)ipa->ptrs.p, n, (const void* const*)((void**)ipa->ptrs.p + 2), 2, 16, ipa->out.p, false);
+    if (pr.use_tables) fixed_msm_run(C, pr.fb_g, (const void* const*)ipa->ptrs.p, n, (const void* const*)((void**)ipa->ptrs.p + 2), 2, ipa->out.p, false);
     else {
       // extras are [blind (w), z <p', b> (u)] in the order of g || w || u
       ipa->msm_jac.ensure(2 * 96);

@@ -143,7 +143,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
     if (pr.use_tables) {
       BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, mainp.data(), mainp.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
       BZ_CUDA(cudaMemcpyAsync((void**)d_ptrs.p + B * I, extrap.data(), extrap.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
-      fixed_msm_run(C, pr.fb_gl, (const void* const*)d_ptrs.p, n, (const void* const*)((void**)d_ptrs.p + B * I), B * I, 1, d_icomm.p);
+      fixed_msm_run(C, pr.fb_gl, (const void* const*)d_ptrs.p, n, (const void* const*)((void**)d_ptrs.p + B * I), B * I, d_icomm.p);
     } else {
       DevBuf d_in, d_jac; d_in.alloc((size_t)(n + 1) * 32); d_jac.alloc((size_t)B * I * 96);
       for (size_t j = 0; j < (size_t)B * I; ++j) {
@@ -383,7 +383,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
   if (pr.use_tables) {
     BZ_CUDA(cudaMemcpyAsync(d_fptrs.p, mainp.data(), (size_t)B * sizeof(void*), cudaMemcpyHostToDevice, st));
     BZ_CUDA(cudaMemcpyAsync((void**)d_fptrs.p + B, extrap.data(), (size_t)B * sizeof(void*), cudaMemcpyHostToDevice, st));
-    fixed_msm_run(C, pr.fb_g, (const void* const*)d_fptrs.p, n, (const void* const*)((void**)d_fptrs.p + B), B, 1, d_fpart.p);
+    fixed_msm_run(C, pr.fb_g, (const void* const*)d_fptrs.p, n, (const void* const*)((void**)d_fptrs.p + B), B, d_fpart.p);
   } else {
     DevBuf d_in, d_jac; d_in.alloc((size_t)(n + 2) * 32); d_jac.alloc((size_t)B * 96);
     for (uint32_t b = 0; b < B; ++b) {

@@ -134,7 +134,7 @@ static int file_mode(const char* path) {
     std::vector<DerivedColumn> derived; std::vector<Token> qtokens; std::vector<uint32_t> goff{0}, qoff;
     for (size_t i = 0; i < eidx.size(); ++i) goff.push_back(hi[i]);
     g_derived_base = 0xffffffffu; g_derived.clear();
-    split_fixed_subexpressions(tokens, goff, 2000, getenv("BZ_NO_DERIVED") == nullptr, derived, qtokens, qoff);
+    split_fixed_subexpressions(tokens, goff, 2000, derived, qtokens, qoff);
     { u64 dm = 0; std::vector<u64> vals; for (const DerivedColumn& d : derived) vals.push_back(eval_tokens(d.tokens, 0, (uint32_t)d.tokens.size(), dm)); g_derived = vals; g_derived_base = 2000; }
     tokens = qtokens;
     for (size_t i = 0; i < eidx.size(); ++i) { lo[i] = qoff[i]; hi[i] = qoff[i + 1]; }

@@ -1,9 +1,8 @@
 """Both MSM engines against the oracle at every window width, on scalars at the digit boundaries of the signed recoding
 (tests/util_msm.py) and in every launch shape:
 
-  - the table MSM (fixedmsm.cu) through Params.commit at c = 4 .. 16, in both accumulation modes (BZ_FB_PAIRS, read when
-    a Context is created), and through Params.commit_batch_dev across its chunk loop, both fold widths, the two-level
-    fold and empty MSMs in the flat entry space;
+  - the table MSM (fixedmsm.cu) through Params.commit at c = 4 .. 16, and through Params.commit_batch_dev across its
+    chunk loop, both fold widths, the two-level fold and empty MSMs in the flat entry space;
   - the bucket MSM (msm.cu) through bz_msm_dev at window_bits = 2 .. 16 and at its own choice, on skewed scalars, and as
     the batched commit of Params built with BZ_FORCE_GENERAL_MSM=1;
   - bz_batch_normalize_dev (Jacobian -> affine).
@@ -23,22 +22,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 K5 = 5
 N5 = 1 << K5
-
-
-@pytest.fixture(scope="module")
-def pair_ctx():
-    """A Context in pair mode (BZ_FB_PAIRS=1: affine pre-addition of consecutive table points)."""
-    old = os.environ.get("BZ_FB_PAIRS")
-    os.environ["BZ_FB_PAIRS"] = "1"
-    try:
-        c = bz.Context(0)
-    finally:
-        if old is None:
-            del os.environ["BZ_FB_PAIRS"]
-        else:
-            os.environ["BZ_FB_PAIRS"] = old
-    yield c
-    c.close()
 
 
 _URS = {}
@@ -75,9 +58,9 @@ def _free(*bufs):
 # ---- 1. table MSM at every width ------------------------------------------------------------------------------------
 @pytest.mark.parametrize("c", range(4, 17))
 @pytest.mark.parametrize("curve", [0, 1])
-def test_table_msm_every_width(curve, c, ctx, pair_ctx, oracle_c):
-    """Params(k = 5, window_bits = c).commit(poly, blind) for every scalar family, both bases (lagrange) and both
-    accumulation modes.  Odd widths on Vesta and even widths on Pallas run over degenerate bases."""
+def test_table_msm_every_width(curve, c, ctx, oracle_c):
+    """Params(k = 5, window_bits = c).commit(poly, blind) for every scalar family and both bases (lagrange).  Odd widths
+    on Vesta and even widths on Pallas run over degenerate bases."""
     from battlezips_halo2_b200.plonk import prover as PR
     co = oracle_c
     sf = co.CURVES[curve][1]
@@ -91,15 +74,14 @@ def test_table_msm_every_width(curve, c, ctx, pair_ctx, oracle_c):
             keys.append((label, lagrange))
     exp = oracle_msms(co, curve, jobs)
     bad = []
-    for mode, cx in (("default", ctx), ("pairs", pair_ctx)):
-        params = PR.Params(cx, K5, g, gl, w, u, curve=curve, window_bits=c)
-        try:
-            for (label, lagrange), e in zip(keys, exp):
-                got = params.commit(fams[label][:N5], fams[label][N5], lagrange=lagrange)
-                if not np.array_equal(got, e):
-                    bad.append((label, f"c={c}", mode, f"lagrange={lagrange}"))
-        finally:
-            params.close()
+    params = PR.Params(ctx, K5, g, gl, w, u, curve=curve, window_bits=c)
+    try:
+        for (label, lagrange), e in zip(keys, exp):
+            got = params.commit(fams[label][:N5], fams[label][N5], lagrange=lagrange)
+            if not np.array_equal(got, e):
+                bad.append((label, f"c={c}", f"lagrange={lagrange}"))
+    finally:
+        params.close()
     assert not bad, bad
 
 
@@ -148,12 +130,11 @@ def _check_batch(got, exp, labels, what):
 
 
 @pytest.mark.parametrize("c", [4, 16])
-def test_table_msm_launch_shapes(c, ctx, pair_ctx, oracle_c):
+def test_table_msm_launch_shapes(c, ctx, oracle_c):
     """commit_batch_dev at count 1, 2, 47, 48, 64, 65, 4 096 and 4 097 (the second pass of the chunk loop) with empty
-    MSMs interleaved; pair mode at 1, 48 and 4 097.  Vesta at c = 4, Pallas at c = 16.
+    MSMs interleaved.  Vesta at c = 4, Pallas at c = 16.
 
-    Which fold runs depends on how many threads the accumulation wave has.  On a B200 (4 resident CTAs per SM, 3 in pair
-    mode) every count up to 65 leaves each MSM enough thread partials for the two-level fold; 4 096 MSMs always fold in a
+    Which fold runs depends on how many threads the accumulation wave has.  On a B200 (4 resident CTAs per SM) every count up to 65 leaves each MSM enough thread partials for the two-level fold; 4 096 MSMs always fold in a
     single level, by the narrow fold (asserted through the launch count).  The single-level folds of fewer MSMs, the wide
     one among them, are tested by test_table_msm_single_level_fold_widths."""
     from battlezips_halo2_b200.plonk import prover as PR
@@ -166,16 +147,15 @@ def test_table_msm_launch_shapes(c, ctx, pair_ctx, oracle_c):
     for lagrange in (False, True):
         bases = np.concatenate([gl if lagrange else g, w[None]])
         exp[lagrange] = oracle_msms(co, curve, [(np.concatenate([polys[j], blinds[j][None]]), bases) for j in range(len(polys))])
-    for mode, cx, mode_counts in (("default", ctx, counts), ("pairs", pair_ctx, [1, 48, 4097])):
-        params = PR.Params(cx, K5, g, gl, w, u, curve=curve, window_bits=c)
-        try:
-            for count in mode_counts:
-                for lagrange in (False, True):
-                    launches = 3 if (mode, count) == ("default", 4096) else None
-                    got = _commit_batch(cx, params, polys, blinds, count, lagrange, launches)
-                    _check_batch(got, exp[lagrange][:count], labels, (f"c={c}", mode, f"count={count}", f"lagrange={lagrange}"))
-        finally:
-            params.close()
+    params = PR.Params(ctx, K5, g, gl, w, u, curve=curve, window_bits=c)
+    try:
+        for count in counts:
+            for lagrange in (False, True):
+                launches = 3 if count == 4096 else None
+                got = _commit_batch(ctx, params, polys, blinds, count, lagrange, launches)
+                _check_batch(got, exp[lagrange][:count], labels, (f"c={c}", f"count={count}", f"lagrange={lagrange}"))
+    finally:
+        params.close()
 
 
 def _single_level_fold_child():
@@ -204,7 +184,6 @@ def test_table_msm_single_level_fold_widths():
     and 48 MSMs with the narrow one.  The launch count shows that no two-level fold ran.  BZ_FB_CTAS_PER_SM is read once
     per process, so this runs in a child process."""
     env = dict(os.environ, BZ_FB_CTAS_PER_SM="1")
-    env.pop("BZ_FB_PAIRS", None)
     cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + \
           ["-c", "from tests.test_gpu_msm_windows import _single_level_fold_child as f; f()"]
     out = subprocess.run(cmd, cwd=ROOT, env=env, capture_output=True, text=True, timeout=600)

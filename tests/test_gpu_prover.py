@@ -146,27 +146,21 @@ def test_keygen_on_device_matches_oracle(ctx, oracle_c, which):
     pk2.close(); pk.close(); params.close()
 
 
-def test_lookup_permutation_paths_agree(ctx, monkeypatch):
-    """permute_expression_pair: the one-CTA kernel (n <= 4096), the device-wide radix-sort path (n = 8192) and the C++ host
-    permutation (BZ_LOOKUP_HOST, kept for A/B checks) give the same proof bytes; a lookup input missing from the table is
-    Error::ConstraintSystemFailure on every path."""
+def test_lookup_permutation_paths_agree(ctx):
+    """permute_expression_pair: the one-CTA kernel (n <= 4096) and the device-wide radix-sort path (n = 8192) give the
+    oracle's proof bytes; a lookup input missing from the table is Error::ConstraintSystemFailure."""
     import battlezips_halo2_b200 as bz
     from battlezips_halo2_b200.plonk import prover as PR
     from battlezips_halo2_b200.circuits import board_circuit_scaled
     job = Job(*tiny_circuit(5))
     params, pk = job.device_keys(ctx, window_bits=6)
-    dev = _prove(job, pk, [4])[0]
-    monkeypatch.setenv("BZ_LOOKUP_HOST", "1")
-    assert _prove(job, pk, [4])[0] == dev == job.oracle_proof(index=4)
-    monkeypatch.delenv("BZ_LOOKUP_HOST")
+    assert _prove(job, pk, [4])[0] == job.oracle_proof(index=4)
     pk.close(); params.close()
     cs, cfg, asg = board_circuit_scaled(13)
     job = Job(cs, asg)
     params, pk = job.device_keys(ctx)
     dev = _prove(job, pk, [1])[0]
-    monkeypatch.setenv("BZ_LOOKUP_HOST", "1")
-    assert _prove(job, pk, [1])[0] == dev
-    monkeypatch.delenv("BZ_LOOKUP_HOST")
+    assert first_diff(dev, job.oracle_proof(index=1)) is None, first_diff(dev, job.oracle_proof(index=1))
     # break the range-check lookup: input = q_lookup * (...advice...), so poison the advice column it reads on the rows
     # where the lookup selector is on (a value far outside the 10-bit table)
     adv = job.advice.copy()
@@ -231,21 +225,6 @@ def test_grand_products_batched_and_sequential_agree(ctx, monkeypatch):
     pk.close(); params.close()
 
 
-def test_grand_product_finish_narrow_geometry(ctx, monkeypatch):
-    """BZ_GP_FINISH_NARROW=1 (one CTA per (proof, product) walks all rows) writes the same proofs as the default geometry."""
-    from battlezips_halo2_b200.circuits import shot_circuit, board_circuit
-    for make in (shot_circuit, board_circuit):
-        cs, cfg, asg = make(2)
-        job = Job(cs, asg)
-        params, pk = job.device_keys(ctx, window_bits=10)
-        a = _prove(job, pk, [0, 5])
-        monkeypatch.setenv("BZ_GP_FINISH_NARROW", "1")
-        b = _prove(job, pk, [0, 5])
-        monkeypatch.delenv("BZ_GP_FINISH_NARROW")
-        assert a == b
-        pk.close(); params.close()
-
-
 @pytest.mark.parametrize("which", ["shot", "board"])
 def test_quotient_dag_and_tree_programs_agree(ctx, which, monkeypatch):
     """h(X) compiled as one DAG per tier (shared sub-expressions, hoisted factors: csrc/evalprog.h) and as the
@@ -294,21 +273,15 @@ def test_generated_quotient_matches_interpreter(ctx, which, monkeypatch):
     k2.close(); p2.close()
 
 
-@pytest.mark.parametrize("pairs", ["0", "1"])
-def test_table_msm_degenerate_bases_and_pair_mode_parity(oracle_c, monkeypatch, pairs):
-    """The table MSM in both accumulation modes -- default, and BZ_FB_PAIRS=1 (affine pre-addition of consecutive table points with one shared inversion per thread, fixedmsm.cu) --:
-    same commitments as the oracle's best_multiexp on a URS with repeated, opposite and identity bases (the pairs that must
-    take the complete-addition path), and the Shot golden proof bytes."""
+def test_table_msm_degenerate_bases_parity(ctx, oracle_c):
+    """The table MSM (fixedmsm.cu): same commitments as the oracle's best_multiexp on a URS with repeated, opposite and
+    identity bases, and the Shot golden proof bytes."""
     import os
-    import battlezips_halo2_b200 as bz
     from battlezips_halo2_b200.plonk import prover as PR
     from battlezips_halo2_b200.circuits import shot_circuit
     from tests.util_prover import VK_REPR
     from oracle import halo2 as H
     co = oracle_c
-    monkeypatch.setenv("BZ_FB_PAIRS", pairs)
-    c2 = bz.Context(0)
-    monkeypatch.delenv("BZ_FB_PAIRS")
     C = co.CURVES[0][0]
     h = C.hash_to_curve("bz-pairs")
     k, n = 6, 64
@@ -316,7 +289,7 @@ def test_table_msm_degenerate_bases_and_pair_mode_parity(oracle_c, monkeypatch, 
     pts[1] = pts[0]; pts[2] = C.neg(pts[0]); pts[3] = None; pts[40] = pts[8]; pts[41] = pts[8]
     g = co.points_to_mont(0, pts[:n])
     w, u = co.points_to_mont(0, [pts[n]])[0], co.points_to_mont(0, [pts[n + 1]])[0]
-    params = PR.Params(c2, k, g, g, w, u, window_bits=5)
+    params = PR.Params(ctx, k, g, g, w, u, window_bits=5)
     rng = np.random.default_rng(5)
     for trial in range(4):
         poly = co.from_u512(0, rng.integers(0, 2**63, size=(n, 8), dtype=np.uint64))
@@ -331,13 +304,13 @@ def test_table_msm_degenerate_bases_and_pair_mode_parity(oracle_c, monkeypatch, 
     gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "proofs.npz"))
     cs, _, asg = shot_circuit(0)
     fx = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", f"params_vesta_k{asg.k}.npz"))
-    params = PR.Params(c2, asg.k, fx["g"], fx["g_lagrange"], fx["w"], fx["u"], window_bits=12)
-    pk = PR.ProvingKey(c2, params, cs.to_ir(), asg.fixed, asg.permutation_mapping(), VK_REPR)
+    params = PR.Params(ctx, asg.k, fx["g"], fx["g_lagrange"], fx["w"], fx["u"], window_bits=12)
+    pk = PR.ProvingKey(ctx, params, cs.to_ir(), asg.fixed, asg.permutation_mapping(), VK_REPR)
     advice = np.stack([PR.mont(col) for col in asg.advice])
     wide = H.splitmix64_wide(0xB200B200B200B200, pk.num_random)
     proof = PR.create_proofs(pk, [asg.instance], advice[None], wide[None])[0]
     assert proof == bytes(gold["shot_w0_idx0"])
-    pk.close(); params.close(); c2.close()
+    pk.close(); params.close()
 
 
 def test_device_proofs_equal_committed_goldens(ctx):
