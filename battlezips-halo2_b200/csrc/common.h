@@ -91,6 +91,7 @@ struct Ctx {
   DevBuf ntt_tmp;          // ping-pong scratch for multi-pass transforms
   DevBuf scratch[4];       // general reusable scratch (msm, staging)
   DevBuf stage[6];         // device staging of the host-buffer entry points (kept across calls: no cudaMalloc/cudaFree per call)
+  DevBuf commit_jac;       // Jacobian results of params_commit_run's bucket MSM
   uint64_t kernel_launches = 0;   // counted by every launch site (bench.py's gpu_launches)
   bool profiling = false;
   DevBuf counters;        // [0] = mixed additions done by fixed_msm_kernel while profiling

@@ -284,7 +284,6 @@ static void ensure_work(Ctx* ctx, PkImpl& pk, uint32_t B) {
   w.commits.alloc(B * max_req * 128);
   w.ptrs.alloc(B * max_req * 2 * sizeof(void*));
   w.descs.alloc(64 * 1024);
-  w.adv_in.alloc(1);
   w.lk_sorted.alloc(std::max<size_t>(1, (size_t)B * pk.L * n * E));
   w.lk_err.alloc((size_t)B * 4 + 64);
   if (w.h_err) cudaFreeHost(w.h_err);
@@ -293,6 +292,28 @@ static void ensure_work(Ctx* ctx, PkImpl& pk, uint32_t B) {
   w.h_pinned_bytes = std::max<size_t>(B * std::max<size_t>(2 * n * E * std::max<uint32_t>(1, pk.L), std::max<size_t>(max_req * 128, (pk.evals.size() + 16) * E)), 1 << 20);
   BZ_CUDA(cudaMallocHost(&w.h_pinned, w.h_pinned_bytes));
   w.batch = B;
+}
+
+void params_commit_run(Ctx* C, const ParamsImpl& p, bool lagrange, const void* const* d_main, const void* const* d_extra,
+                       uint32_t n_msm, void* d_out, bool xyzz_out) {
+  const FixedBase& fb = lagrange ? p.fb_gl : p.fb_g;
+  if (p.use_tables) {
+    fixed_msm_run(C, fb, d_main, p.n, d_extra, n_msm, d_out, xyzz_out);
+    return;
+  }
+  // bucket MSM (k >= 20, or forced): the MSMs of the call are sorted, accumulated and reduced as ONE batch
+  BZ_CHECK(!xyzz_out, "internal: the bucket MSM returns affine commitments only");
+  C->commit_jac.ensure((size_t)n_msm * 96);
+  msm_run_batch(C, p.curve, d_main, d_extra, p.n, 0, fb.npts, lagrange ? p.gl_w.p : p.g_w_u.p, n_msm, C->commit_jac.p);
+  jac_to_affine_run(C, p.curve, C->commit_jac.p, d_out, n_msm);
+}
+
+const void* const* upload_msm_ptrs(Ctx* C, DevBuf& d, const std::vector<void*>& mainp, const std::vector<void*>& extrap) {
+  const size_t bytes = mainp.size() * sizeof(void*);
+  d.ensure(2 * bytes);
+  BZ_CUDA(cudaMemcpyAsync(d.p, mainp.data(), bytes, cudaMemcpyHostToDevice, C->stream));
+  BZ_CUDA(cudaMemcpyAsync((char*)d.p + bytes, extrap.data(), bytes, cudaMemcpyHostToDevice, C->stream));
+  return (const void* const*)d.p;
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -359,24 +380,14 @@ API int bz_params_commit(bz_ctx* ctx, bz_params* params, int lagrange_basis, con
   PV_TRY(ctx, {
     BZ_CHECK(params && poly && blind && out_affine, "null argument");
     ParamsImpl& p = params->p;
-    DevBuf d_poly, d_extra, d_ptrs, d_out;
-    d_poly.alloc((size_t)p.n * 32); d_extra.alloc(64); d_ptrs.alloc(2 * sizeof(void*)); d_out.alloc(64);
     cudaStream_t st = C->stream;
+    DevBuf &d_poly = C->stage[0], &d_out = C->stage[1], &d_extra = C->stage[3], &d_ptrs = C->stage[4];
+    d_poly.ensure((size_t)p.n * 32); d_out.ensure(64); d_extra.ensure(64);
     BZ_CUDA(cudaMemcpyAsync(d_poly.p, poly, (size_t)p.n * 32, cudaMemcpyHostToDevice, st));
     BZ_CUDA(cudaMemsetAsync(d_extra.p, 0, 64, st));
     BZ_CUDA(cudaMemcpyAsync(d_extra.p, blind, 32, cudaMemcpyHostToDevice, st));
-    void* ptrs[2] = {d_poly.p, d_extra.p};
-    BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, ptrs, sizeof(ptrs), cudaMemcpyHostToDevice, st));
-    const FixedBase& fb = lagrange_basis ? p.fb_gl : p.fb_g;
-    if (p.use_tables) fixed_msm_run(C, fb, (const void* const*)d_ptrs.p, p.n, (const void* const*)((void**)d_ptrs.p + 1), 1, d_out.p);
-    else {
-      DevBuf d_in, d_jac; d_in.alloc((size_t)fb.npts * 32); d_jac.alloc(96);
-      BZ_CUDA(cudaMemcpyAsync(d_in.p, d_poly.p, (size_t)p.n * 32, cudaMemcpyDeviceToDevice, st));
-      BZ_CUDA(cudaMemcpyAsync((char*)d_in.p + (size_t)p.n * 32, d_extra.p, (size_t)(fb.npts - p.n) * 32, cudaMemcpyDeviceToDevice, st));
-      msm_run(C, p.curve, d_in.p, lagrange_basis ? p.gl_w.p : p.g_w_u.p, fb.npts, d_jac.p, 0);
-      jac_to_affine_run(C, p.curve, d_jac.p, d_out.p, 1);
-      BZ_CUDA(cudaStreamSynchronize(st));
-    }
+    const void* const* d = upload_msm_ptrs(C, d_ptrs, {d_poly.p}, {d_extra.p});
+    params_commit_run(C, p, lagrange_basis, d, d + 1, 1, d_out.p);
     BZ_CUDA(cudaMemcpyAsync(out_affine, d_out.p, 64, cudaMemcpyDeviceToHost, st));
     BZ_CUDA(cudaStreamSynchronize(st));
   });
@@ -397,22 +408,14 @@ API int bz_params_commit_batch_dev(bz_ctx* ctx, bz_params* params, int lagrange_
     const uint32_t nextra = fb.npts - p.n;
     // persistent staging (no cudaMalloc / cudaFree per call: large frees stall the whole device for 100+ ms now and then)
     DevBuf &d_extra = C->stage[3], &d_ptrs = C->stage[4];
-    d_extra.ensure((size_t)count * nextra * 32); d_ptrs.ensure((size_t)2 * count * sizeof(void*));
+    d_extra.ensure((size_t)count * nextra * 32);
     BZ_CUDA(cudaMemsetAsync(d_extra.p, 0, (size_t)count * nextra * 32, st));
     BZ_CUDA(cudaMemcpy2DAsync(d_extra.p, (size_t)nextra * 32, d_blinds, 32, 32, count, cudaMemcpyDeviceToDevice, st));   // blind -> the w slot
-    std::vector<void*> ptrs((size_t)2 * count);
-    for (uint32_t j = 0; j < count; ++j) { ptrs[j] = (char*)d_polys + (size_t)j * p.n * 32; ptrs[count + j] = (char*)d_extra.p + (size_t)j * nextra * 32; }
-    BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, ptrs.data(), ptrs.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
-    if (p.use_tables) {
-      fixed_msm_run(C, fb, (const void* const*)d_ptrs.p, p.n, (const void* const*)((void**)d_ptrs.p + count), count, d_out_affine);
-    } else {
-      DevBuf& d_jac = C->stage[0];
-      d_jac.ensure((size_t)count * 96);
-      msm_run_batch(C, p.curve, (const void* const*)d_ptrs.p, (const void* const*)((void**)d_ptrs.p + count), p.n, 0, fb.npts,
-                    lagrange_basis ? p.gl_w.p : p.g_w_u.p, count, d_jac.p);
-      jac_to_affine_run(C, p.curve, d_jac.p, d_out_affine, count);
-    }
-    BZ_CUDA(cudaStreamSynchronize(st));          // ptrs goes out of scope
+    std::vector<void*> mainp(count), extrap(count);
+    for (uint32_t j = 0; j < count; ++j) { mainp[j] = (char*)d_polys + (size_t)j * p.n * 32; extrap[j] = (char*)d_extra.p + (size_t)j * nextra * 32; }
+    const void* const* d = upload_msm_ptrs(C, d_ptrs, mainp, extrap);
+    params_commit_run(C, p, lagrange_basis, d, d + count, count, d_out_affine);
+    BZ_CUDA(cudaStreamSynchronize(st));
   });
 }
 
@@ -686,27 +689,14 @@ API int bz_pk_vk_commitments(bz_ctx* ctx, bz_pk* pkh, void* fixed_commitments, v
     const uint32_t FM = pk.cs.F + pk.M, n = pk.n;
     if (FM && pk.vk_fixed_comm.size() + pk.vk_perm_comm.size() != (size_t)FM * 8) {
       cudaStream_t st = C->stream;
-      ParamsImpl& pr = *pk.params;
       std::vector<void*> mainp(FM), extrap(FM);
-      DevBuf d_ptrs, d_extra, d_out;
-      d_ptrs.alloc((size_t)2 * FM * sizeof(void*)); d_extra.alloc((size_t)FM * 64); d_out.alloc((size_t)FM * 64);
+      DevBuf &d_out = C->stage[1], &d_extra = C->stage[3], &d_ptrs = C->stage[4];
+      d_extra.ensure((size_t)FM * 64); d_out.ensure((size_t)FM * 64);
       std::vector<HFe> ex((size_t)FM * 2, C->fp.zero());
       for (uint32_t j = 0; j < FM; ++j) { mainp[j] = (DFe*)pk.lval.p + (size_t)j * n; extrap[j] = (DFe*)d_extra.p + (size_t)j * 2; ex[2 * j] = C->fp.one(); }
       BZ_CUDA(cudaMemcpyAsync(d_extra.p, ex.data(), ex.size() * 32, cudaMemcpyHostToDevice, st));
-      if (pr.use_tables) {
-        BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, mainp.data(), (size_t)FM * sizeof(void*), cudaMemcpyHostToDevice, st));
-        BZ_CUDA(cudaMemcpyAsync((void**)d_ptrs.p + FM, extrap.data(), (size_t)FM * sizeof(void*), cudaMemcpyHostToDevice, st));
-        fixed_msm_run(C, pr.fb_gl, (const void* const*)d_ptrs.p, n, (const void* const*)((void**)d_ptrs.p + FM), FM, d_out.p);
-      } else {
-        DevBuf d_in, d_jac;
-        d_in.alloc((size_t)(n + 1) * 32); d_jac.alloc((size_t)FM * 96);
-        for (uint32_t j = 0; j < FM; ++j) {
-          BZ_CUDA(cudaMemcpyAsync(d_in.p, mainp[j], (size_t)n * 32, cudaMemcpyDeviceToDevice, st));
-          BZ_CUDA(cudaMemcpyAsync((char*)d_in.p + (size_t)n * 32, extrap[j], 32, cudaMemcpyDeviceToDevice, st));
-          msm_run(C, pr.curve, d_in.p, pr.gl_w.p, n + 1, (char*)d_jac.p + (size_t)j * 96, 0);
-        }
-        jac_to_affine_run(C, pr.curve, d_jac.p, d_out.p, FM);
-      }
+      const void* const* d = upload_msm_ptrs(C, d_ptrs, mainp, extrap);
+      params_commit_run(C, *pk.params, true, d, d + FM, FM, d_out.p);
       std::vector<uint64_t> all((size_t)FM * 8);
       BZ_CUDA(cudaMemcpyAsync(all.data(), d_out.p, all.size() * 8, cudaMemcpyDeviceToHost, st));
       BZ_CUDA(cudaStreamSynchronize(st));
@@ -807,62 +797,50 @@ struct Prover {
     run_msms(lag, mainp, extrap, n_msm);
     read_points(n_msm, nr, pts);
   }
-  // one batch of commitments: fixed-base tables when available, otherwise the bucket MSM per polynomial
+  // one batch of commitments into w.commits: the table MSM's XYZZ sums, or affine points from the bucket MSM (read_points)
   void run_msms(bool lagrange, const std::vector<void*>& mainp, const std::vector<void*>& extrap, uint32_t n_msm) {
-    const FixedBase& fb = lagrange ? pk.params->fb_gl : pk.params->fb_g;
+    const ParamsImpl& pr = *pk.params;
     const uint32_t world = C->shard_world, rank = C->shard_rank;
-    if (pk.params->use_tables) {
-      BZ_CUDA(cudaMemcpyAsync(w.ptrs.p, mainp.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
-      BZ_CUDA(cudaMemcpyAsync((void**)w.ptrs.p + n_msm, extrap.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
-      if (world > 1 && n_msm >= world) {
-        // one large proof across GPUs, table path: rank r sums the contiguous MSMs [r * per, (r + 1) * per) and the 128-byte
-        // XYZZ results are all-gathered (every rank holds the same tables); fewer MSMs than ranks are computed redundantly
+    const void* const* dm = upload_msm_ptrs(C, w.ptrs, mainp, extrap);
+    const void* const* de = dm + n_msm;
+    if (world > 1 && pr.use_tables && n_msm >= world) {
+      // one large proof across GPUs, table path: rank r sums the contiguous MSMs [r * per, (r + 1) * per) and the 128-byte
+      // XYZZ results are all-gathered (every rank holds the same tables); fewer MSMs than ranks are computed redundantly
+      const uint32_t per = (n_msm + world - 1) / world, lo = std::min(n_msm, rank * per), hi = std::min(n_msm, lo + per);
+      BZ_CHECK((size_t)per * 128 <= C->shard_cap, "sharding exchange buffer too small");
+      BZ_CUDA(cudaMemsetAsync(C->shard_send, 0, (size_t)per * 128, st));
+      if (hi > lo) params_commit_run(C, pr, lagrange, dm + lo, de + lo, hi - lo, C->shard_send, true);
+      if (C->shard_exchange(C->shard_user, (size_t)per * 128) != 0) throw Error(BZ_ERR_CUDA, "sharding: all-gather callback failed");
+      BZ_CUDA(cudaMemcpyAsync(w.commits.p, C->shard_recv, (size_t)n_msm * 128, cudaMemcpyDeviceToDevice, st));
+      return;
+    }
+    if (world > 1 && !pr.use_tables) {
+      const uint32_t npts = (lagrange ? pr.fb_gl : pr.fb_g).npts;
+      const void* bases = lagrange ? pr.gl_w.p : pr.g_w_u.p;
+      if (n_msm >= world) {
+        // column deal: rank r owns the contiguous MSMs [r * per, (r + 1) * per); one all-gather of per x 96 B per rank
         const uint32_t per = (n_msm + world - 1) / world, lo = std::min(n_msm, rank * per), hi = std::min(n_msm, lo + per);
-        BZ_CHECK((size_t)per * 128 <= C->shard_cap, "sharding exchange buffer too small");
-        BZ_CUDA(cudaMemsetAsync(C->shard_send, 0, (size_t)per * 128, st));
-        if (hi > lo) fixed_msm_run(C, fb, (const void* const*)w.ptrs.p + lo, n, (const void* const*)((void**)w.ptrs.p + n_msm) + lo, hi - lo, C->shard_send, true);
-        if (C->shard_exchange(C->shard_user, (size_t)per * 128) != 0) throw Error(BZ_ERR_CUDA, "sharding: all-gather callback failed");
-        BZ_CUDA(cudaMemcpyAsync(w.commits.p, C->shard_recv, (size_t)n_msm * 128, cudaMemcpyDeviceToDevice, st));
+        BZ_CHECK((size_t)per * 96 <= C->shard_cap, "sharding exchange buffer too small");
+        BZ_CUDA(cudaMemsetAsync(C->shard_send, 0, (size_t)per * 96, st));
+        msm_run_batch(C, pr.curve, dm + lo, de + lo, n, 0, npts, bases, hi - lo, C->shard_send);
+        if (C->shard_exchange(C->shard_user, (size_t)per * 96) != 0) throw Error(BZ_ERR_CUDA, "sharding: all-gather callback failed");
+        jac_to_affine_run(C, pr.curve, C->shard_recv, w.commits.p, n_msm);          // rank-major = MSM order
         return;
       }
-      fixed_msm_run(C, fb, (const void* const*)w.ptrs.p, n, (const void* const*)((void**)w.ptrs.p + n_msm), n_msm, w.commits.p, true);
-      return;
-    }
-    // bucket MSM (k >= 20, or forced): the MSMs of the call go through the sort / accumulate / reduce pipeline as ONE batch
-    const uint32_t npts = fb.npts;
-    const int curve = pk.params->curve;
-    const void* bases = lagrange ? pk.params->gl_w.p : pk.params->g_w_u.p;
-    BZ_CUDA(cudaMemcpyAsync(w.ptrs.p, mainp.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
-    BZ_CUDA(cudaMemcpyAsync((void**)w.ptrs.p + n_msm, extrap.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
-    const void* const* dm = (const void* const*)w.ptrs.p;
-    const void* const* de = dm + n_msm;
-    w.msm_jac.ensure((size_t)n_msm * 96);
-    if (world > 1 && n_msm >= world) {
-      // column deal: rank r owns the contiguous MSMs [r * per, (r + 1) * per); one all-gather of per x 96 B per rank
-      const uint32_t per = (n_msm + world - 1) / world, lo = std::min(n_msm, rank * per), hi = std::min(n_msm, lo + per);
-      BZ_CHECK((size_t)per * 96 <= C->shard_cap, "sharding exchange buffer too small");
-      BZ_CUDA(cudaMemsetAsync(C->shard_send, 0, (size_t)per * 96, st));
-      msm_run_batch(C, curve, dm + lo, de + lo, n, 0, npts, bases, hi - lo, C->shard_send);
-      if (C->shard_exchange(C->shard_user, (size_t)per * 96) != 0) throw Error(BZ_ERR_CUDA, "sharding: all-gather callback failed");
-      jac_to_affine_run(C, curve, C->shard_recv, w.commits.p, n_msm);          // rank-major = MSM order
-      return;
-    }
-    if (world > 1) {
       // fewer MSMs than ranks (random polynomial, q', S, the two IPA terms): every MSM split by point range, the partials summed
       BZ_CHECK((size_t)n_msm * 96 <= C->shard_cap, "sharding exchange buffer too small");
       const uint32_t base = npts / world, rem = npts % world, plo = rank * base + std::min(rank, rem), cnt = base + (rank < rem ? 1u : 0u);
-      msm_run_batch(C, curve, dm, de, n, plo, cnt, (const char*)bases + (size_t)plo * 64, n_msm, C->shard_send);
+      msm_run_batch(C, pr.curve, dm, de, n, plo, cnt, (const char*)bases + (size_t)plo * 64, n_msm, C->shard_send);
       if (C->shard_exchange(C->shard_user, (size_t)n_msm * 96) != 0) throw Error(BZ_ERR_CUDA, "sharding: all-gather callback failed");
       w.msm_jac.ensure((size_t)n_msm * world * 96);
       for (uint32_t j = 0; j < n_msm; ++j) {
         // partials of MSM j sit at recv[r][j]: gather them contiguously, then one kernel adds them and normalises
         BZ_CUDA(cudaMemcpy2DAsync((char*)w.msm_jac.p + (size_t)j * world * 96, 96, (const char*)C->shard_recv + (size_t)j * 96, (size_t)n_msm * 96, 96, world, cudaMemcpyDeviceToDevice, st));
-        jac_sum_run(C, curve, (const char*)w.msm_jac.p + (size_t)j * world * 96, world, (char*)w.commits.p + (size_t)j * 64);
+        jac_sum_run(C, pr.curve, (const char*)w.msm_jac.p + (size_t)j * world * 96, world, (char*)w.commits.p + (size_t)j * 64);
       }
       return;
     }
-    msm_run_batch(C, curve, dm, de, n, 0, npts, bases, n_msm, w.msm_jac.p);
-    jac_to_affine_run(C, curve, w.msm_jac.p, w.commits.p, n_msm);
+    params_commit_run(C, pr, lagrange, dm, de, n_msm, w.commits.p, pr.use_tables);
   }
   // Commitments come back unnormalised from the table MSM (XYZZ, 128 B): one batched inversion on the host for the
   // whole call (Montgomery's trick, ~9 host multiplications per point) instead of a single-thread Fermat chain per
@@ -877,24 +855,17 @@ struct Prover {
         for (uint32_t i = 0; i < nr; ++i) affine_to_host(Fq, h + ((size_t)b * nr + i) * 8, pts[b][i]);
       return;
     }
-    std::vector<HFe> pre(n_msm);
-    HFe acc = Fq.one();
+    std::vector<HFe> zi3(n_msm);                       // zzz, then 1 / zzz (0 for the identity)
+    for (uint32_t j = 0; j < n_msm; ++j) memcpy(zi3[j].l, h + (size_t)j * 16 + 12, 32);
+    host_batch_invert(Fq, zi3);
     for (uint32_t j = 0; j < n_msm; ++j) {
-      HFe zzz; memcpy(zzz.l, h + (size_t)j * 16 + 12, 32);
-      pre[j] = acc;
-      if (!zzz.is_zero()) acc = Fq.mul(acc, zzz);
-    }
-    HFe inv = Fq.inv(acc);
-    for (int j = (int)n_msm - 1; j >= 0; --j) {
-      HFe x, y, zz, zzz;
-      memcpy(x.l, h + (size_t)j * 16, 32); memcpy(y.l, h + (size_t)j * 16 + 4, 32); memcpy(zz.l, h + (size_t)j * 16 + 8, 32); memcpy(zzz.l, h + (size_t)j * 16 + 12, 32);
+      HFe x, y, zz;
+      memcpy(x.l, h + (size_t)j * 16, 32); memcpy(y.l, h + (size_t)j * 16 + 4, 32); memcpy(zz.l, h + (size_t)j * 16 + 8, 32);
       HostPoint& p = pts[j / nr][j % nr];
-      if (zzz.is_zero()) { p.identity = true; memset(p.x, 0, 32); memset(p.y, 0, 32); continue; }
-      const HFe zi3 = Fq.mul(inv, pre[j]);             // 1 / zzz
-      inv = Fq.mul(inv, zzz);
-      const HFe t = Fq.mul(zz, zi3), zi2 = Fq.sqr(t);  // (zz / zzz)^2 = 1 / zz
+      if (zi3[j].is_zero()) { p.identity = true; memset(p.x, 0, 32); memset(p.y, 0, 32); continue; }
+      const HFe t = Fq.mul(zz, zi3[j]), zi2 = Fq.sqr(t);  // (zz / zzz)^2 = 1 / zz
       p.identity = false;
-      Fq.to_repr(Fq.mul(x, zi2), p.x); Fq.to_repr(Fq.mul(y, zi3), p.y);
+      Fq.to_repr(Fq.mul(x, zi2), p.x); Fq.to_repr(Fq.mul(y, zi3[j]), p.y);
     }
   }
 
@@ -1525,10 +1496,9 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
         read_points(n_msm, 2, pts);
       } else {
         // bucket MSM of the two short vectors over G' || w || u; every rank of a sharded proof computes it (it is tiny)
-        BZ_CUDA(cudaMemcpyAsync(w.ptrs.p, mainp.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
-        BZ_CUDA(cudaMemcpyAsync((void**)w.ptrs.p + n_msm, extrap.data(), (size_t)n_msm * sizeof(void*), cudaMemcpyHostToDevice, st));
+        const void* const* dm = upload_msm_ptrs(C, w.ptrs, mainp, extrap);
         w.msm_jac.ensure((size_t)n_msm * 96);
-        msm_run_batch(C, curve, (const void* const*)w.ptrs.p, (const void* const*)w.ptrs.p + n_msm, count, 0, count + 2, w.ipa_gm.p, n_msm, w.msm_jac.p);
+        msm_run_batch(C, curve, dm, dm + n_msm, count, 0, count + 2, w.ipa_gm.p, n_msm, w.msm_jac.p);
         jac_to_affine_run(C, curve, w.msm_jac.p, w.commits.p, n_msm);
         read_points(n_msm, 2, pts, true);
       }
@@ -1626,7 +1596,7 @@ struct bz_ipa {
   bz::DevBuf consts;     // z, u, u^-1, x3
   bz::DevBuf rnd;        // l_rand, r_rand
   bz::DevBuf extras;     // [2][2] extra scalars of the two MSMs (w: blind, u: z <p', b>)
-  bz::DevBuf ptrs, out, msm_in, msm_jac;
+  bz::DevBuf ptrs, out;
   bz::Regions reg;
 };
 
@@ -1673,14 +1643,8 @@ API int bz_ipa_round(bz_ctx* ctx, bz_ipa* ipa, const void* z, const void* l_rand
     ipa_inner_kernel<FpP><<<1, IPA_THREADS, 0, st>>>(ipa->reg, n, half, PolyRef{R_MISC, 0}, PolyRef{R_MISC, 1}, (const DFe*)ipa->consts.p, 8, 0,
                                                     (const DFe*)ipa->rnd.p, 0, 0, 1, (DFe*)ipa->extras.p);
     C->kernel_launches += 2;
-    ParamsImpl& pr = *ipa->params;
-    if (pr.use_tables) fixed_msm_run(C, pr.fb_g, (const void* const*)ipa->ptrs.p, n, (const void* const*)((void**)ipa->ptrs.p + 2), 2, ipa->out.p, false);
-    else {
-      // extras are [blind (w), z <p', b> (u)] in the order of g || w || u
-      ipa->msm_jac.ensure(2 * 96);
-      msm_run_batch(C, pr.curve, (const void* const*)ipa->ptrs.p, (const void* const*)((void**)ipa->ptrs.p + 2), n, 0, n + 2, pr.g_w_u.p, 2, ipa->msm_jac.p);
-      jac_to_affine_run(C, pr.curve, ipa->msm_jac.p, ipa->out.p, 2);
-    }
+    // extras are [blind (w), z <p', b> (u)] in the order of g || w || u
+    params_commit_run(C, *ipa->params, false, (const void* const*)ipa->ptrs.p, (const void* const*)ipa->ptrs.p + 2, 2, ipa->out.p);
     BZ_CUDA(cudaMemcpyAsync(out_l_affine, ipa->out.p, 64, cudaMemcpyDeviceToHost, st));
     BZ_CUDA(cudaMemcpyAsync(out_r_affine, (char*)ipa->out.p + 64, 64, cudaMemcpyDeviceToHost, st));
     BZ_CUDA(cudaStreamSynchronize(st));

@@ -20,7 +20,6 @@ typedef bzh::Fe HFe;
 
 namespace bz {
 
-void msm_run(Ctx* ctx, int curve, const void* scalars, const void* bases, uint32_t n, void* out_jac, int c_override);
 void msm_run_batch(Ctx* ctx, int curve, const void* const* d_main, const void* const* d_extra, uint32_t n_main, uint32_t first, uint32_t n,
                    const void* bases, uint32_t n_msm, void* out_jac);
 void msm_multi_run(Ctx* ctx, int curve, const void* scalars, uint32_t nq, const void* bases, uint32_t stride, uint32_t outputs, void* out_jac);
@@ -52,8 +51,18 @@ struct ParamsImpl {
   DevBuf g_w_u;         // n + 2 affine points: g || w || u
   DevBuf gl_w;          // n + 1 affine points: g_lagrange || w
   FixedBase fb_g, fb_gl;
-  bool use_tables = true;   // small n: fixed-base window tables; large n (k >= 15): bucket MSM over the raw bases
+  bool use_tables = true;   // k <= 19: fixed-base window tables; k >= 20 (or BZ_FORCE_GENERAL_MSM=1): bucket MSM over the raw bases
 };
+
+// The n_msm commitments of one call over the basis of p: g || w || u, or g_lagrange || w when `lagrange`.  MSM m sums
+// d_main[m][0 .. p.n) and d_extra[m][0 .. npts - p.n) (the blind, and over g the U term) against that basis; d_main / d_extra
+// are DEVICE arrays of device pointers.  d_out: n_msm affine points (64 B each), or with `xyzz_out` the table MSM's
+// unnormalised XYZZ sums (128 B each).  The bucket path only returns affine points and rejects `xyzz_out`.  Stream-ordered
+// on C->stream; its only allocation is the context's Jacobian scratch, grown as needed.
+void params_commit_run(Ctx* C, const ParamsImpl& p, bool lagrange, const void* const* d_main, const void* const* d_extra,
+                       uint32_t n_msm, void* d_out, bool xyzz_out = false);
+// Copies the host pointer arrays into d (grown as needed) as [main... | extra...]; returns the device array (extras at + main.size())
+const void* const* upload_msm_ptrs(Ctx* C, DevBuf& d, const std::vector<void*>& mainp, const std::vector<void*>& extrap);
 
 
 struct CircuitCopy {
@@ -130,7 +139,7 @@ struct PkImpl {
   // workspace cache
   struct Work {
     uint32_t batch = 0;
-    DevBuf val, poly, coset, misc, rnd, wide, hext, hcoef, hext_low, hcoef_low, nd, consts, extras, evalout, commits, ptrs, descs, adv_in, inst_in, msm_in, msm_jac, ipa_coefq, ipa_gm, ipa_tmp, lk_sorted, lk_err, scan_tmp, eval_tmp;
+    DevBuf val, poly, coset, misc, rnd, wide, hext, hcoef, hext_low, hcoef_low, nd, consts, extras, evalout, commits, ptrs, descs, msm_jac, ipa_coefq, ipa_gm, ipa_tmp, lk_sorted, lk_err, scan_tmp, eval_tmp;
     void* h_pinned = nullptr; size_t h_pinned_bytes = 0;
     uint32_t* h_err = nullptr;      // pinned: error word of the device lookup permutation
   } work;

@@ -128,7 +128,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
   BZ_CUDA(cudaMemcpyAsync(h_pts.data(), d_pts.p, h_pts.size() * 8, cudaMemcpyDeviceToHost, st));
   BZ_CUDA(cudaMemcpyAsync(h_stat.data(), d_stat.p, h_stat.size(), cudaMemcpyDeviceToHost, st));
   if (I) {
-    d_inst.ensure((size_t)B * I * n * 32); d_ptrs.ensure((size_t)2 * B * I * sizeof(void*)); d_extra.ensure((size_t)B * I * 64); d_icomm.ensure((size_t)B * I * 64);
+    d_inst.ensure((size_t)B * I * n * 32); d_extra.ensure((size_t)B * I * 64); d_icomm.ensure((size_t)B * I * 64);
     BZ_CUDA(cudaMemsetAsync(d_inst.p, 0, (size_t)B * I * n * 32, st));
     std::vector<void*> mainp((size_t)B * I), extrap((size_t)B * I);
     std::vector<HFe> ex((size_t)B * I * 2, F.zero());
@@ -140,19 +140,8 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
         mainp[j] = (char*)d_inst.p + j * n * 32; extrap[j] = (char*)d_extra.p + j * 64; ex[2 * j] = F.one();
       }
     BZ_CUDA(cudaMemcpyAsync(d_extra.p, ex.data(), ex.size() * 32, cudaMemcpyHostToDevice, st));
-    if (pr.use_tables) {
-      BZ_CUDA(cudaMemcpyAsync(d_ptrs.p, mainp.data(), mainp.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
-      BZ_CUDA(cudaMemcpyAsync((void**)d_ptrs.p + B * I, extrap.data(), extrap.size() * sizeof(void*), cudaMemcpyHostToDevice, st));
-      fixed_msm_run(C, pr.fb_gl, (const void* const*)d_ptrs.p, n, (const void* const*)((void**)d_ptrs.p + B * I), B * I, d_icomm.p);
-    } else {
-      DevBuf d_in, d_jac; d_in.alloc((size_t)(n + 1) * 32); d_jac.alloc((size_t)B * I * 96);
-      for (size_t j = 0; j < (size_t)B * I; ++j) {
-        BZ_CUDA(cudaMemcpyAsync(d_in.p, mainp[j], (size_t)n * 32, cudaMemcpyDeviceToDevice, st));
-        BZ_CUDA(cudaMemcpyAsync((char*)d_in.p + (size_t)n * 32, extrap[j], 32, cudaMemcpyDeviceToDevice, st));
-        msm_run(C, pr.curve, d_in.p, pr.gl_w.p, n + 1, (char*)d_jac.p + j * 96, 0);
-      }
-      jac_to_affine_run(C, pr.curve, d_jac.p, d_icomm.p, B * I);
-    }
+    const void* const* d = upload_msm_ptrs(C, d_ptrs, mainp, extrap);
+    params_commit_run(C, pr, true, d, d + B * I, B * I, d_icomm.p);
     BZ_CUDA(cudaMemcpyAsync(h_icomm.data(), d_icomm.p, (size_t)B * I * 64, cudaMemcpyDeviceToHost, st));
   }
   BZ_CUDA(cudaStreamSynchronize(st));
@@ -370,7 +359,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
   }
   // ---- device: compute_s, the fixed-base part, the final check
   DevBuf &d_sc = pk.vwork[7], &d_s = pk.vwork[8], &d_fx = pk.vwork[9], &d_fptrs = pk.vwork[10], &d_fpart = pk.vwork[11], &d_vp = pk.vwork[12], &d_vs = pk.vwork[13], &d_ok = pk.vwork[14];
-  d_sc.ensure(s_consts.size() * 32); d_s.ensure((size_t)B * n * 32); d_fx.ensure((size_t)B * 64); d_fptrs.ensure((size_t)2 * B * sizeof(void*));
+  d_sc.ensure(s_consts.size() * 32); d_s.ensure((size_t)B * n * 32); d_fx.ensure((size_t)B * 64);
   d_fpart.ensure((size_t)B * 64); d_vp.ensure(v_pts.size() * 8); d_vs.ensure(v_scal.size() * 8); d_ok.ensure(B);
   BZ_CUDA(cudaMemcpyAsync(d_sc.p, s_consts.data(), s_consts.size() * 32, cudaMemcpyHostToDevice, st));
   BZ_CUDA(cudaMemcpyAsync(d_fx.p, fx_extra.data(), fx_extra.size() * 32, cudaMemcpyHostToDevice, st));
@@ -380,19 +369,8 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
   C->kernel_launches++;
   std::vector<void*> mainp(B), extrap(B);
   for (uint32_t b = 0; b < B; ++b) { mainp[b] = (char*)d_s.p + (size_t)b * n * 32; extrap[b] = (char*)d_fx.p + (size_t)b * 64; }
-  if (pr.use_tables) {
-    BZ_CUDA(cudaMemcpyAsync(d_fptrs.p, mainp.data(), (size_t)B * sizeof(void*), cudaMemcpyHostToDevice, st));
-    BZ_CUDA(cudaMemcpyAsync((void**)d_fptrs.p + B, extrap.data(), (size_t)B * sizeof(void*), cudaMemcpyHostToDevice, st));
-    fixed_msm_run(C, pr.fb_g, (const void* const*)d_fptrs.p, n, (const void* const*)((void**)d_fptrs.p + B), B, d_fpart.p);
-  } else {
-    DevBuf d_in, d_jac; d_in.alloc((size_t)(n + 2) * 32); d_jac.alloc((size_t)B * 96);
-    for (uint32_t b = 0; b < B; ++b) {
-      BZ_CUDA(cudaMemcpyAsync(d_in.p, mainp[b], (size_t)n * 32, cudaMemcpyDeviceToDevice, st));
-      BZ_CUDA(cudaMemcpyAsync((char*)d_in.p + (size_t)n * 32, extrap[b], 64, cudaMemcpyDeviceToDevice, st));
-      msm_run(C, pr.curve, d_in.p, pr.g_w_u.p, n + 2, (char*)d_jac.p + (size_t)b * 96, 0);
-    }
-    jac_to_affine_run(C, pr.curve, d_jac.p, d_fpart.p, B);
-  }
+  const void* const* d = upload_msm_ptrs(C, d_fptrs, mainp, extrap);
+  params_commit_run(C, pr, false, d, d + B, B, d_fpart.p);
   verify_final_kernel<<<B, VFY_THREADS, 0, st>>>((const Affine<FqP>*)d_vp.p, (const uint32_t*)d_vs.p, NV, (const Affine<FqP>*)d_fpart.p, (uint8_t*)d_ok.p);
   C->kernel_launches++;
   std::vector<uint8_t> h_ok(B);
