@@ -111,7 +111,8 @@ def load_library():
         "bz_ctx_set_sharding": (i32, [vp, u32, u32, vp, vp, ctypes.c_size_t, ALLGATHER_FN, vp]),
     }
     declared_elsewhere = {"bz_params_create", "bz_params_destroy", "bz_params_commit", "bz_pk_create", "bz_pk_destroy",
-                          "bz_pk_num_random", "bz_pk_proof_size", "bz_pk_quotient_muls", "bz_create_proofs", "bz_pk_create_from_assembly", "bz_pk_vk_commitments", "bz_verify_proofs", "bz_params_commit_batch_dev"}     # bound in plonk/prover.py
+                          "bz_pk_num_random", "bz_pk_proof_size", "bz_pk_quotient_muls", "bz_create_proofs", "bz_pk_create_from_assembly", "bz_pk_vk_commitments", "bz_verify_proofs", "bz_params_commit_batch_dev",
+                          "bz_vk_create", "bz_vk_destroy", "bz_vk_proof_size", "bz_verify_proofs_vk"}     # bound in plonk/prover.py
     missing = [n for n in EXPORTS if n not in sigs and n not in declared_elsewhere]
     assert not missing, f"unbound C-ABI symbols: {missing}"
     for name, (res, args) in sigs.items():

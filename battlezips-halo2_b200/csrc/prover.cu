@@ -234,11 +234,11 @@ static void upload_programs(PkImpl& pk) {
 }
 
 // ------------------------------------------------------------------------------------------------------
-static void add_query(PkImpl& pk, int cid, int rot, PolyRef poly, int bk, int bi, int ev = -1) { pk.queries.push_back(Query{cid, rot, poly, bk, bi, ev}); }
+static void add_query(VkImpl& pk, int cid, int rot, PolyRef poly, int bk, int bi, int ev = -1) { pk.queries.push_back(Query{cid, rot, poly, bk, bi, ev}); }
 
 // static structure of the multiopen argument (U: multiopen.rs::construct_intermediate_sets); points are
 // identified by their rotation (x * omega^rot are distinct for distinct rotations)
-static void build_multiopen(PkImpl& pk) {
+static void build_multiopen(VkImpl& pk) {
   std::vector<int> point_order;                       // rotation -> point index = position
   auto point_index = [&](int rot) { for (size_t i = 0; i < point_order.size(); ++i) if (point_order[i] == rot) return (int)i; point_order.push_back(rot); return (int)point_order.size() - 1; };
   struct Tmp { int cid; PolyRef poly; int bk, bi; std::vector<int> pidx; };
@@ -255,7 +255,7 @@ static void build_multiopen(PkImpl& pk) {
     int idx = -1;
     for (size_t i = 0; i < sets.size(); ++i) if (sets[i] == s) idx = (int)i;
     if (idx < 0) { sets.push_back(s); idx = (int)sets.size() - 1; }
-    pk.cmap.push_back(PkImpl::CommInfo{t.poly, t.bk, t.bi, idx, t.cid});
+    pk.cmap.push_back(VkImpl::CommInfo{t.poly, t.bk, t.bi, idx, t.cid});
   }
   for (auto& s : sets) { std::vector<int> r; for (int pi : s) r.push_back(point_order[pi]); pk.point_sets.push_back(r); }
 }
@@ -428,11 +428,14 @@ API uint32_t bz_pk_quotient_muls(const bz_pk* pk, uint32_t tier, uint32_t* point
   return pk->p.q_muls[tier];
 }
 
-// Everything of keygen_pk's image that needs no GPU: the flattened constraint system, domain constants, the layouts of the per-proof
-// constants / randomness / polynomial slots, the query and evaluation lists, the multiopen structure and the compiled programs.
-// (Also what bz_quotient_program runs at build time to emit the circuit-specialised kernels.)
-static void pk_host_setup(const bzh::Field& F, PkImpl& pk, const bz_circuit* cin) {
-  CircuitCopy& cs = pk.cs;
+}  // extern "C"
+
+namespace bz {
+
+// The verifying key's part of keygen: the flattened constraint system, domain constants, the query list, the multiopen
+// structure, the number of evaluations and the proof size.  Needs no GPU.
+void vk_host_setup(const bzh::Field& F, VkImpl& vk, const bz_circuit* cin) {
+  CircuitCopy& cs = vk.cs;
   cs.k = cin->k; cs.G = cin->num_advice; cs.F = cin->num_fixed; cs.I = cin->num_instance; cs.degree = cin->degree; cs.bf = cin->blinding_factors;
   for (uint32_t i = 0; i < cin->n_advice_queries; ++i) cs.aq.push_back({cin->advice_queries[2 * i], cin->advice_queries[2 * i + 1]});
   for (uint32_t i = 0; i < cin->n_fixed_queries; ++i) cs.fq.push_back({cin->fixed_queries[2 * i], cin->fixed_queries[2 * i + 1]});
@@ -457,24 +460,68 @@ static void pk_host_setup(const bzh::Field& F, PkImpl& pk, const bz_circuit* cin
     cs.vk_repr = F.from_raw(raw);
   }
   BZ_CHECK(cs.degree >= 3, "cs degree must be >= 3");
-  pk.n = 1u << cs.k;
-  pk.qdeg = cs.degree - 1;
+  vk.n = 1u << cs.k;
+  vk.qdeg = cs.degree - 1;
+  vk.M = (uint32_t)cs.perm.size(); vk.L = (uint32_t)cs.lookups.size();
+  vk.chunk_len = cs.degree - 2;
+  vk.nsets = vk.M ? (vk.M + vk.chunk_len - 1) / vk.chunk_len : 0;
+  vk.usable = vk.n - (cs.bf + 1);
+  BZ_CHECK(vk.chunk_len <= 8, "permutation chunk too wide");
+  // domain constants: omega = ROOT_OF_UNITY^(2^(32-k))
+  vk.omega = F.root_of_unity();
+  for (uint32_t i = cs.k; i < 32; ++i) vk.omega = F.sqr(vk.omega);
+  vk.omega_inv = F.inv(vk.omega);
+  // ---- queries (SURVEY App. A step 19).  blind slots: advice[G], lookup (A',S',Z)[3L], perm[nsets], h, random
+  auto b_adv = [&](uint32_t g) { return (int)g; };
+  auto b_lk = [&](uint32_t l, uint32_t w) { return (int)(cs.G + 3 * l + w); };
+  auto b_pz = [&](uint32_t s) { return (int)(cs.G + 3 * vk.L + s); };
+  const int b_h = (int)(cs.G + 3 * vk.L + vk.nsets), b_rand = b_h + 1;
+  const int last_rot = -((int)cs.bf + 1);
+  // positions in the proof's evaluation list (the order pk_host_setup writes it in; steps 14-18)
+  const int e_adv0 = (int)cs.iq.size(), e_fix0 = e_adv0 + (int)cs.aq.size(), e_rand = e_fix0 + (int)cs.fq.size(), e_sig0 = e_rand + 1;
+  const int e_perm0 = e_sig0 + (int)vk.M;
+  auto e_perm = [&](uint32_t s2) { return e_perm0 + 3 * (int)s2; };                     // z, z_next, (z_last: all but the last set)
+  const int e_lk0 = e_perm0 + (vk.nsets ? 3 * (int)vk.nsets - 1 : 0);
+  for (size_t i = 0; i < cs.iq.size(); ++i) add_query(vk, cid_inst + cs.iq[i].first, cs.iq[i].second, PolyRef{R_POLY, vk.slot_inst(cs.iq[i].first)}, 0, 0, (int)i);
+  for (size_t i = 0; i < cs.aq.size(); ++i) add_query(vk, cid_adv + cs.aq[i].first, cs.aq[i].second, PolyRef{R_POLY, (uint32_t)cs.aq[i].first}, 1, b_adv(cs.aq[i].first), e_adv0 + (int)i);
+  for (uint32_t s2 = 0; s2 < vk.nsets; ++s2) {
+    add_query(vk, cid_pz + s2, 0, PolyRef{R_POLY, vk.slot_pz(s2)}, 1, b_pz(s2), e_perm(s2));
+    add_query(vk, cid_pz + s2, 1, PolyRef{R_POLY, vk.slot_pz(s2)}, 1, b_pz(s2), e_perm(s2) + 1);
+  }
+  for (int s2 = (int)vk.nsets - 2; s2 >= 0; --s2) add_query(vk, cid_pz + s2, last_rot, PolyRef{R_POLY, vk.slot_pz(s2)}, 1, b_pz(s2), e_perm(s2) + 2);
+  for (uint32_t l = 0; l < vk.L; ++l) {
+    const int e = e_lk0 + 5 * (int)l;                                                   // z, z_next, a, a_inv, s
+    add_query(vk, cid_lk + 3 * l + 2, 0, PolyRef{R_POLY, vk.slot_lk(l, 2)}, 1, b_lk(l, 2), e);
+    add_query(vk, cid_lk + 3 * l + 0, 0, PolyRef{R_POLY, vk.slot_lk(l, 0)}, 1, b_lk(l, 0), e + 2);
+    add_query(vk, cid_lk + 3 * l + 1, 0, PolyRef{R_POLY, vk.slot_lk(l, 1)}, 1, b_lk(l, 1), e + 4);
+    add_query(vk, cid_lk + 3 * l + 0, -1, PolyRef{R_POLY, vk.slot_lk(l, 0)}, 1, b_lk(l, 0), e + 3);
+    add_query(vk, cid_lk + 3 * l + 2, 1, PolyRef{R_POLY, vk.slot_lk(l, 2)}, 1, b_lk(l, 2), e + 1);
+  }
+  for (size_t i = 0; i < cs.fq.size(); ++i) add_query(vk, cid_fix + cs.fq[i].first, cs.fq[i].second, PolyRef{R_SHPOLY, (uint32_t)cs.fq[i].first}, 0, 0, e_fix0 + (int)i);
+  for (uint32_t j = 0; j < vk.M; ++j) add_query(vk, cid_sig + j, 0, PolyRef{R_SHPOLY, cs.F + j}, 0, 0, e_sig0 + (int)j);
+  add_query(vk, cid_h, 0, PolyRef{R_MISC, vk.misc_h()}, 1, b_h, -1);
+  add_query(vk, cid_rand, 0, PolyRef{R_RANDPOLY, 0}, 1, b_rand, e_rand);
+  build_multiopen(vk);
+  vk.nev = (uint32_t)e_lk0 + 5 * vk.L;
+  // proof size: points (32 B) + scalars (32 B)
+  const uint32_t npoints = cs.G + 2 * vk.L + vk.nsets + vk.L + 1 + vk.qdeg + 1 + 1 + 2 * cs.k;
+  const uint32_t nscalars = vk.nev + (uint32_t)vk.point_sets.size() + 2;
+  vk.proof_size = 32 * (npoints + nscalars);
+}
+
+// Everything of keygen_pk's image that needs no GPU: the verifying key's part (vk_host_setup), then the prover's own layouts of
+// the per-proof constants / randomness / polynomial slots, the evaluation list and the compiled programs.
+// (Also what bz_quotient_program runs at build time to emit the circuit-specialised kernels.)
+static void pk_host_setup(const bzh::Field& F, PkImpl& pk, const bz_circuit* cin) {
+  vk_host_setup(F, pk, cin);
+  const CircuitCopy& cs = pk.cs;
   pk.ext_k = cs.k;
   while ((1ull << pk.ext_k) < (uint64_t)pk.n * pk.qdeg) ++pk.ext_k;
   pk.ext_n = 1u << pk.ext_k;
-  pk.M = (uint32_t)cs.perm.size(); pk.L = (uint32_t)cs.lookups.size();
-  pk.chunk_len = cs.degree - 2;
-  pk.nsets = pk.M ? (pk.M + pk.chunk_len - 1) / pk.chunk_len : 0;
   pk.NS = cs.G + cs.I + 3 * pk.L + pk.nsets;
   pk.NC = (uint32_t)cs.consts.size();
-  pk.usable = pk.n - (cs.bf + 1);
-  BZ_CHECK(pk.chunk_len <= 8, "permutation chunk too wide");
-  // domain constants
   pk.ext_omega = F.root_of_unity();
   for (uint32_t i = pk.ext_k; i < 32; ++i) pk.ext_omega = F.sqr(pk.ext_omega);
-  pk.omega = pk.ext_omega;
-  for (uint32_t i = cs.k; i < pk.ext_k; ++i) pk.omega = F.sqr(pk.omega);
-  pk.omega_inv = F.inv(pk.omega);
   const uint32_t n = pk.n;
   derive_fixed_subexpressions(pk);
   // ---- const table layout
@@ -509,48 +556,19 @@ static void pk_host_setup(const bzh::Field& F, PkImpl& pk, const bz_circuit* cin
   pk.r_sblind = r; r += 1;
   pk.r_ipa = r; r += 2 * cs.k;
   pk.R = r;
+  // ---- per-proof blind slots of the queries: advice[G], lookup (A',S',Z)[3L], perm[nsets], h, random
+  pk.nblinds = cs.G + 3 * pk.L + pk.nsets + 2;
   // ---- MISC slots
   uint32_t m = 0;
   pk.m_cin0 = m; m += 2 * pk.L;
-  pk.m_hpoly = m++;
-  // ---- queries (SURVEY App. A step 19).  blind slots: advice[G], lookup (A',S',Z)[3L], perm[nsets], h, random
-  auto b_adv = [&](uint32_t g) { return (int)g; };
-  auto b_lk = [&](uint32_t l, uint32_t w) { return (int)(cs.G + 3 * l + w); };
-  auto b_pz = [&](uint32_t s) { return (int)(cs.G + 3 * pk.L + s); };
-  const int b_h = (int)(cs.G + 3 * pk.L + pk.nsets), b_rand = b_h + 1;
-  pk.nblinds = b_rand + 1;
-  const int last_rot = -((int)cs.bf + 1);
-  // positions in the proof's evaluation list (same order as the `ev(...)` pushes below; steps 14-18)
-  const int e_adv0 = (int)cs.iq.size(), e_fix0 = e_adv0 + (int)cs.aq.size(), e_rand = e_fix0 + (int)cs.fq.size(), e_sig0 = e_rand + 1;
-  const int e_perm0 = e_sig0 + (int)pk.M;
-  auto e_perm = [&](uint32_t s2) { return e_perm0 + 3 * (int)s2; };                     // z, z_next, (z_last: all but the last set)
-  const int e_lk0 = e_perm0 + (pk.nsets ? 3 * (int)pk.nsets - 1 : 0);
-  for (size_t i = 0; i < cs.iq.size(); ++i) add_query(pk, cid_inst + cs.iq[i].first, cs.iq[i].second, PolyRef{R_POLY, pk.slot_inst(cs.iq[i].first)}, 0, 0, (int)i);
-  for (size_t i = 0; i < cs.aq.size(); ++i) add_query(pk, cid_adv + cs.aq[i].first, cs.aq[i].second, PolyRef{R_POLY, (uint32_t)cs.aq[i].first}, 1, b_adv(cs.aq[i].first), e_adv0 + (int)i);
-  for (uint32_t s2 = 0; s2 < pk.nsets; ++s2) {
-    add_query(pk, cid_pz + s2, 0, PolyRef{R_POLY, pk.slot_pz(s2)}, 1, b_pz(s2), e_perm(s2));
-    add_query(pk, cid_pz + s2, 1, PolyRef{R_POLY, pk.slot_pz(s2)}, 1, b_pz(s2), e_perm(s2) + 1);
-  }
-  for (int s2 = (int)pk.nsets - 2; s2 >= 0; --s2) add_query(pk, cid_pz + s2, last_rot, PolyRef{R_POLY, pk.slot_pz(s2)}, 1, b_pz(s2), e_perm(s2) + 2);
-  for (uint32_t l = 0; l < pk.L; ++l) {
-    const int e = e_lk0 + 5 * (int)l;                                                   // z, z_next, a, a_inv, s
-    add_query(pk, cid_lk + 3 * l + 2, 0, PolyRef{R_POLY, pk.slot_lk(l, 2)}, 1, b_lk(l, 2), e);
-    add_query(pk, cid_lk + 3 * l + 0, 0, PolyRef{R_POLY, pk.slot_lk(l, 0)}, 1, b_lk(l, 0), e + 2);
-    add_query(pk, cid_lk + 3 * l + 1, 0, PolyRef{R_POLY, pk.slot_lk(l, 1)}, 1, b_lk(l, 1), e + 4);
-    add_query(pk, cid_lk + 3 * l + 0, -1, PolyRef{R_POLY, pk.slot_lk(l, 0)}, 1, b_lk(l, 0), e + 3);
-    add_query(pk, cid_lk + 3 * l + 2, 1, PolyRef{R_POLY, pk.slot_lk(l, 2)}, 1, b_lk(l, 2), e + 1);
-  }
-  for (size_t i = 0; i < cs.fq.size(); ++i) add_query(pk, cid_fix + cs.fq[i].first, cs.fq[i].second, PolyRef{R_SHPOLY, (uint32_t)cs.fq[i].first}, 0, 0, e_fix0 + (int)i);
-  for (uint32_t j = 0; j < pk.M; ++j) add_query(pk, cid_sig + j, 0, PolyRef{R_SHPOLY, cs.F + j}, 0, 0, e_sig0 + (int)j);
-  add_query(pk, cid_h, 0, PolyRef{R_MISC, pk.m_hpoly}, 1, b_h, -1);
-  add_query(pk, cid_rand, 0, PolyRef{R_RANDPOLY, 0}, 1, b_rand, e_rand);
-  build_multiopen(pk);
+  pk.m_hpoly = m++;                           // = misc_h(), the slot the h(X) query names
   const uint32_t nps = (uint32_t)pk.point_sets.size();
   pk.m_qset0 = m; m += nps;
   pk.m_qtmp0 = m; m += 2 * nps;
   pk.m_qprime = m++; pk.m_ppoly = m++; pk.m_pprime = m++; pk.m_b = m++; pk.m_coef = m++; pk.m_scl = m++; pk.m_scr = m++;
   pk.NM = m;
   // ---- evaluation list in transcript order (steps 14-18)
+  const int last_rot = -((int)cs.bf + 1);
   auto ev = [&](PolyRef p, int rot) { pk.evals.push_back(EvalQuery{p, pk.rot_const.at(rot)}); };
   for (auto& q : cs.iq) ev(PolyRef{R_POLY, pk.slot_inst(q.first)}, q.second);
   for (auto& q : cs.aq) ev(PolyRef{R_POLY, (uint32_t)q.first}, q.second);
@@ -566,12 +584,13 @@ static void pk_host_setup(const bzh::Field& F, PkImpl& pk, const bz_circuit* cin
     ev(PolyRef{R_POLY, pk.slot_lk(l, 0)}, 0); ev(PolyRef{R_POLY, pk.slot_lk(l, 0)}, -1);
     ev(PolyRef{R_POLY, pk.slot_lk(l, 1)}, 0);
   }
-  // proof size: points (32 B) + scalars (32 B)
-  uint32_t npoints = cs.G + 2 * pk.L + pk.nsets + pk.L + 1 + pk.qdeg + 1 + 1 + 2 * cs.k;
-  uint32_t nscalars = (uint32_t)pk.evals.size() + nps + 2;
-  pk.proof_size = 32 * (npoints + nscalars);
+  BZ_CHECK(pk.evals.size() == pk.nev, "internal: evaluation list mismatch");
   build_programs(pk);
 }
+
+}  // namespace bz
+
+extern "C" {
 
 static int pk_create_impl(bz_ctx* ctx, bz_params* params, const bz_circuit* cin, const void* fixed_values, const void* sigma_values,
                           const uint32_t* mapping, bz_pk** out) {

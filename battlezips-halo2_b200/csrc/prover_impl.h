@@ -1,5 +1,5 @@
 // Internal types shared by prover.cu (keygen + create_proof) and verifier.cu (verify_proof): the device images of
-// Params / ProvingKey, the flattened constraint system, the static multiopen structure, and the host transcript.
+// Params / VerifyingKey / ProvingKey, the flattened constraint system, the static multiopen structure, and the host transcript.
 // Not part of the C ABI (include/bzhalo2.h).
 #pragma once
 #include "../../include/bzhalo2.h"
@@ -84,18 +84,44 @@ enum { R_VAL = 0, R_POLY = 1, R_MISC = 2, R_RANDPOLY = 3, R_SPOLY = 4, R_SHPOLY 
 enum { cid_inst = 0, cid_adv = 100000, cid_pz = 200000, cid_lk = 300000, cid_fix = 400000, cid_sig = 500000, cid_h = 600000, cid_rand = 600001 };
 struct Query { int cid; int rot; PolyRef poly; int blind_kind; int blind_idx; int eval_idx; };   // eval_idx: position among the proof's evaluations (-1: h, computed by the verifier)   // blind_kind: 0 = one, 1 = per-proof blind slot
 
-struct PkImpl {
+// The verifying key: what halo2's VerifyingKey holds (domain, constraint system, fixed and permutation commitments, and in
+// cs.vk_repr the scalar vk.hash_into absorbs) plus the shape and multiopen layout derived from it.  Everything Verifier::run
+// reads, and nothing else: building one allocates no device memory.
+struct VkImpl {
   ParamsImpl* params = nullptr;
   CircuitCopy cs;
-  uint32_t n = 0, ext_k = 0, ext_n = 0, qdeg = 0;
-  uint32_t M = 0, L = 0, nsets = 0, chunk_len = 0, NS = 0, NC = 0, usable = 0;
-  HFe omega, omega_inv, ext_omega;
+  uint32_t n = 0, qdeg = 0;
+  uint32_t M = 0, L = 0, nsets = 0, chunk_len = 0, usable = 0;
+  HFe omega, omega_inv;
+  std::vector<uint64_t> vk_fixed_comm, vk_perm_comm;   // keygen_vk: commit_lagrange(column, Blind::default()) as affine (8 x u64 each)
+  // static multiopen structure
+  std::vector<Query> queries;
+  struct CommInfo { PolyRef poly; int blind_kind, blind_idx; int set; int cid; };
+  std::vector<CommInfo> cmap;                  // first-appearance order
+  std::vector<std::vector<int>> point_sets;    // rotations per set, ordered by point index
+  uint32_t nev = 0;                            // evaluations the proof carries (steps 14-18)
+  uint32_t proof_size = 0;
+  // slots
+  uint32_t slot_inst(uint32_t i) const { return cs.G + i; }
+  uint32_t slot_lk(uint32_t l, uint32_t which) const { return cs.G + cs.I + 3 * l + which; }   // 0 A', 1 S', 2 Z
+  uint32_t slot_pz(uint32_t s) const { return cs.G + cs.I + 3 * L + s; }
+  uint32_t misc_h() const { return 2 * L; }    // MISC slot of h(X), after the 2L compressed lookup expressions
+  DevBuf vwork[16];      // verifier staging, kept across verify calls (no cudaMalloc / cudaFree per call)
+};
+
+// The shape part of keygen: circuit copy, domain constants, queries, multiopen structure, evaluation count and proof size.
+// Host only; no GPU needed.
+void vk_host_setup(const bzh::Field& F, VkImpl& vk, const bz_circuit* cin);
+
+struct PkImpl : VkImpl {
+  uint32_t ext_k = 0, ext_n = 0;
+  uint32_t NS = 0, NC = 0;
+  HFe ext_omega;
   // device images
   DevBuf lval;        // [F + M][n]  fixed values then sigma values (Lagrange)
   DevBuf shpoly;      // [F + M][n]  coefficient form
   DevBuf shcoset;     // [F + M + 5][ext_n]: fixed, sigma, l0, l_blind, l_last, active, coset_x
   DevBuf omega_pows;  // [n]
-  std::vector<uint64_t> vk_fixed_comm, vk_perm_comm;   // keygen_vk: commit_lagrange(column, Blind::default()) as affine (8 x u64 each)
   DevBuf tev;         // [2^(ext_k-k)]
   // programs
   static constexpr uint32_t Q_TIERS = 3;     // h(X) tier t: terms whose quotient fits ext_n >> t points, evaluated on every 2^t-th extended point
@@ -121,21 +147,11 @@ struct PkImpl {
   uint32_t r_adv_rows, r_adv_blind, r_lk0, r_perm0, r_lkz0, r_randpoly, r_rand_blind, r_hblind, r_qprime, r_spoly, r_sblind, r_ipa;
   // per-proof blind slots (host)
   uint32_t nblinds = 0;
-  // static multiopen structure
-  std::vector<Query> queries;
-  struct CommInfo { PolyRef poly; int blind_kind, blind_idx; int set; int cid; };
-  std::vector<CommInfo> cmap;                  // first-appearance order
-  std::vector<std::vector<int>> point_sets;    // rotations per set, ordered by point index
-  // evaluation list (write order)
+  // evaluation list (write order; nev entries)
   std::vector<EvalQuery> evals;
   DevBuf d_evals;
   // MISC slots
   uint32_t NM = 0, m_cin0, m_hpoly, m_qset0, m_qtmp0, m_qprime, m_ppoly, m_pprime, m_b, m_coef, m_scl, m_scr;
-  uint32_t proof_size = 0;
-  // slots
-  uint32_t slot_inst(uint32_t i) const { return cs.G + i; }
-  uint32_t slot_lk(uint32_t l, uint32_t which) const { return cs.G + cs.I + 3 * l + which; }   // 0 A', 1 S', 2 Z
-  uint32_t slot_pz(uint32_t s) const { return cs.G + cs.I + 3 * L + s; }
   // workspace cache
   struct Work {
     uint32_t batch = 0;
@@ -143,7 +159,6 @@ struct PkImpl {
     void* h_pinned = nullptr; size_t h_pinned_bytes = 0;
     uint32_t* h_err = nullptr;      // pinned: error word of the device lookup permutation
   } work;
-  DevBuf vwork[16];      // verifier staging, kept across bz_verify_proofs calls (no cudaMalloc / cudaFree per call)
   ~PkImpl() { if (work.h_pinned) cudaFreeHost(work.h_pinned); if (work.h_err) cudaFreeHost(work.h_err); }
 };
 
@@ -204,6 +219,7 @@ static inline HFe rnd_host(const ProofState& ps, const bzh::Field& F, uint32_t i
 
 struct bz_params { bz::ParamsImpl p; };
 struct bz_pk { bz::PkImpl p; };
+struct bz_vk { bz::VkImpl v; };
 static inline bz::Ctx* ctx_of(bz_ctx* c) { return &c->c; }
 
 #define PV_TRY(ctx_, ...)                                     \

@@ -61,15 +61,15 @@ __global__ void __launch_bounds__(VFY_THREADS) verify_final_kernel(const Affine<
 }
 
 struct Verifier {
-  Ctx* C; PkImpl& pk; uint32_t B;
+  Ctx* C; VkImpl& vk; uint32_t B;
   const bzh::Field& F; const bzh::Field& Fq;
   cudaStream_t st;
-  Verifier(Ctx* c, PkImpl& p, uint32_t b) : C(c), pk(p), B(b), F(c->fp), Fq(c->fq), st(c->stream) {}
+  Verifier(Ctx* c, VkImpl& v, uint32_t b) : C(c), vk(v), B(b), F(c->fp), Fq(c->fq), st(c->stream) {}
 
   // host evaluation of one postfix expression at the claimed openings
   HFe eval_expr(uint32_t lo, uint32_t hi, const std::vector<HFe>& ev, const std::map<std::pair<int, int>, int>& aq,
                 const std::map<std::pair<int, int>, int>& fq, const std::map<std::pair<int, int>, int>& iq, int e_adv0, int e_fix0) const {
-    const CircuitCopy& cs = pk.cs;
+    const CircuitCopy& cs = vk.cs;
     std::vector<HFe> stck;
     for (uint32_t t = lo; t < hi; ++t) {
       const Token& k = cs.tokens[t];
@@ -92,17 +92,16 @@ struct Verifier {
 };
 
 void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_t instance_stride, const uint8_t* proofs, uint32_t proof_len, uint8_t* results) {
-  const CircuitCopy& cs = pk.cs;
-  const uint32_t G = cs.G, I = cs.I, L = pk.L, bf = cs.bf, n = pk.n, k = cs.k, nsets = pk.nsets, qdeg = pk.qdeg;
-  const uint32_t nps = (uint32_t)pk.point_sets.size();
+  const CircuitCopy& cs = vk.cs;
+  const uint32_t G = cs.G, I = cs.I, L = vk.L, bf = cs.bf, n = vk.n, k = cs.k, nsets = vk.nsets, qdeg = vk.qdeg;
+  const uint32_t nps = (uint32_t)vk.point_sets.size();
   for (uint32_t b = 0; b < B; ++b) results[b] = 0;
-  if (proof_len != pk.proof_size) return;                                  // short read / trailing bytes: Err
-  for (uint32_t i = 0; i < I; ++i) if (instance_lens[i] > pk.usable) return;   // Error::InstanceTooLarge
-  ParamsImpl& pr = *pk.params;
-  // vk commitments (computed once per pk)
-  if (pk.vk_fixed_comm.size() + pk.vk_perm_comm.size() != (size_t)(cs.F + pk.M) * 8) throw Error(BZ_ERR_INVALID, "internal: vk commitments missing");
+  if (proof_len != vk.proof_size) return;                                  // short read / trailing bytes: Err
+  for (uint32_t i = 0; i < I; ++i) if (instance_lens[i] > vk.usable) return;   // Error::InstanceTooLarge
+  ParamsImpl& pr = *vk.params;
+  if (vk.vk_fixed_comm.size() + vk.vk_perm_comm.size() != (size_t)(cs.F + vk.M) * 8) throw Error(BZ_ERR_INVALID, "internal: vk commitments missing");
   // ---- layout of the proof: which 32-byte items are points
-  const uint32_t nev = (uint32_t)pk.evals.size();
+  const uint32_t nev = vk.nev;
   std::vector<uint32_t> pt_off;        // byte offsets of the compressed points, in reading order
   uint32_t off = 0;
   auto take_pts = [&](uint32_t c) { for (uint32_t i = 0; i < c; ++i) { pt_off.push_back(off); off += 32; } };
@@ -113,13 +112,13 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
   take_pts(1);                                     // S
   take_pts(2 * k);                                 // L_j, R_j
   const uint32_t off_c = off; off += 64;
-  BZ_CHECK(off == pk.proof_size, "internal: proof layout mismatch");
+  BZ_CHECK(off == vk.proof_size, "internal: proof layout mismatch");
   const uint32_t NP = (uint32_t)pt_off.size();
   // ---- device: decompress every point of every proof; instance commitments
   std::vector<uint8_t> comp((size_t)B * NP * 32);
   for (uint32_t b = 0; b < B; ++b)
     for (uint32_t i = 0; i < NP; ++i) memcpy(&comp[((size_t)b * NP + i) * 32], proofs + (size_t)b * proof_len + pt_off[i], 32);
-  DevBuf &d_comp = pk.vwork[0], &d_pts = pk.vwork[1], &d_stat = pk.vwork[2], &d_inst = pk.vwork[3], &d_ptrs = pk.vwork[4], &d_extra = pk.vwork[5], &d_icomm = pk.vwork[6];
+  DevBuf &d_comp = vk.vwork[0], &d_pts = vk.vwork[1], &d_stat = vk.vwork[2], &d_inst = vk.vwork[3], &d_ptrs = vk.vwork[4], &d_extra = vk.vwork[5], &d_icomm = vk.vwork[6];
   d_comp.ensure(comp.size()); d_pts.ensure((size_t)B * NP * 64); d_stat.ensure((size_t)B * NP);
   BZ_CUDA(cudaMemcpyAsync(d_comp.p, comp.data(), comp.size(), cudaMemcpyHostToDevice, st));
   decompress_points_run(C, pr.curve, d_comp.p, d_pts.p, (uint8_t*)d_stat.p, B * NP);
@@ -152,10 +151,10 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
   for (size_t i = 0; i < cs.fq.size(); ++i) fqm[{cs.fq[i].first, cs.fq[i].second}] = (int)i;
   for (size_t i = 0; i < cs.iq.size(); ++i) iqm[{cs.iq[i].first, cs.iq[i].second}] = (int)i;
   const int e_adv0 = (int)cs.iq.size(), e_fix0 = e_adv0 + (int)cs.aq.size(), e_rand = e_fix0 + (int)cs.fq.size(), e_sig0 = e_rand + 1;
-  const int e_perm0 = e_sig0 + (int)pk.M, e_lk0 = e_perm0 + (nsets ? 3 * (int)nsets - 1 : 0);
+  const int e_perm0 = e_sig0 + (int)vk.M, e_lk0 = e_perm0 + (nsets ? 3 * (int)nsets - 1 : 0);
   // variable points of the final check, per proof: every cmap commitment (h expands into its qdeg pieces), q', S, L_j, R_j
   uint32_t NV = 0;
-  for (auto& ci : pk.cmap) NV += ci.cid == cid_h ? qdeg : 1;
+  for (auto& ci : vk.cmap) NV += ci.cid == cid_h ? qdeg : 1;
   NV += 2 + 2 * k;
   std::vector<uint64_t> v_pts((size_t)B * NV * 8, 0), v_scal((size_t)B * NV * 4, 0);
   const uint32_t cstride = 2 + k;
@@ -204,7 +203,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
     HFe xn = x; for (uint32_t i = 0; i < k; ++i) xn = F.sqr(xn);
     const HFe xn_m1 = F.sub(xn, one);
     std::vector<HFe> w_is, inv1;                     // rotations -(bf+1) .. 0; one inversion for (x - w_i)..., (x^n - 1)
-    for (int rot = -((int)bf + 1); rot <= 0; ++rot) { w_is.push_back(F.pow_u64(pk.omega_inv, (uint64_t)(-rot))); inv1.push_back(F.sub(x, w_is.back())); }
+    for (int rot = -((int)bf + 1); rot <= 0; ++rot) { w_is.push_back(F.pow_u64(vk.omega_inv, (uint64_t)(-rot))); inv1.push_back(F.sub(x, w_is.back())); }
     inv1.push_back(xn_m1);
     host_batch_invert(F, inv1);
     std::vector<HFe> l_evals;
@@ -230,7 +229,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
       for (uint32_t s2 = 1; s2 < nsets; ++s2) fold(F.mul(F.sub(pe(s2, 0), pe(s2 - 1, 2)), l_0));
       const HFe delta = F.delta();
       for (uint32_t s2 = 0; s2 < nsets; ++s2) {
-        const uint32_t c0 = s2 * pk.chunk_len, c1 = std::min<uint32_t>(pk.M, c0 + pk.chunk_len);
+        const uint32_t c0 = s2 * vk.chunk_len, c1 = std::min<uint32_t>(vk.M, c0 + vk.chunk_len);
         HFe left = pe(s2, 1), right = pe(s2, 0);
         HFe cur_delta = F.mul(F.mul(beta, x), F.pow_u64(delta, c0));
         for (uint32_t j = c0; j < c1; ++j) {
@@ -261,26 +260,26 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
     expected_h = F.mul(expected_h, xn_m1_inv);
     // ---- multiopen verifier
     const HFe x1 = t_squeeze(ps, F), x2 = t_squeeze(ps, F);
-    auto rot_point = [&](int r) { return r >= 0 ? F.mul(x, F.pow_u64(pk.omega, (uint64_t)r)) : F.mul(x, F.pow_u64(pk.omega_inv, (uint64_t)(-r))); };
+    auto rot_point = [&](int r) { return r >= 0 ? F.mul(x, F.pow_u64(vk.omega, (uint64_t)r)) : F.mul(x, F.pow_u64(vk.omega_inv, (uint64_t)(-r))); };
     // evaluation of every commitment at every point of its set
-    std::vector<std::vector<std::vector<HFe>>> c_evals(pk.cmap.size());
-    for (size_t ci = 0; ci < pk.cmap.size(); ++ci) c_evals[ci].assign(1, std::vector<HFe>(pk.point_sets[pk.cmap[ci].set].size(), F.zero()));
-    for (const Query& q : pk.queries) {
+    std::vector<std::vector<std::vector<HFe>>> c_evals(vk.cmap.size());
+    for (size_t ci = 0; ci < vk.cmap.size(); ++ci) c_evals[ci].assign(1, std::vector<HFe>(vk.point_sets[vk.cmap[ci].set].size(), F.zero()));
+    for (const Query& q : vk.queries) {
       size_t ci = 0;
-      while (pk.cmap[ci].cid != q.cid) ++ci;
-      const std::vector<int>& set = pk.point_sets[pk.cmap[ci].set];
+      while (vk.cmap[ci].cid != q.cid) ++ci;
+      const std::vector<int>& set = vk.point_sets[vk.cmap[ci].set];
       const size_t j = std::find(set.begin(), set.end(), q.rot) - set.begin();
       c_evals[ci][0][j] = q.eval_idx >= 0 ? ev[q.eval_idx] : expected_h;
     }
     std::vector<std::vector<HFe>> q_eval_sets(nps);
-    for (uint32_t s2 = 0; s2 < nps; ++s2) q_eval_sets[s2].assign(pk.point_sets[s2].size(), F.zero());
-    std::vector<HFe> comm_scalar(pk.cmap.size(), one);         // x1 power inside its set
+    for (uint32_t s2 = 0; s2 < nps; ++s2) q_eval_sets[s2].assign(vk.point_sets[s2].size(), F.zero());
+    std::vector<HFe> comm_scalar(vk.cmap.size(), one);         // x1 power inside its set
     {
       std::vector<HFe> set_pow(nps, one);
-      for (int ci = (int)pk.cmap.size() - 1; ci >= 0; --ci) { comm_scalar[ci] = set_pow[pk.cmap[ci].set]; set_pow[pk.cmap[ci].set] = F.mul(set_pow[pk.cmap[ci].set], x1); }
+      for (int ci = (int)vk.cmap.size() - 1; ci >= 0; --ci) { comm_scalar[ci] = set_pow[vk.cmap[ci].set]; set_pow[vk.cmap[ci].set] = F.mul(set_pow[vk.cmap[ci].set], x1); }
     }
-    for (size_t ci = 0; ci < pk.cmap.size(); ++ci) {
-      std::vector<HFe>& qs = q_eval_sets[pk.cmap[ci].set];
+    for (size_t ci = 0; ci < vk.cmap.size(); ++ci) {
+      std::vector<HFe>& qs = q_eval_sets[vk.cmap[ci].set];
       for (size_t j = 0; j < qs.size(); ++j) qs[j] = F.add(F.mul(qs[j], x1), c_evals[ci][0][j]);
     }
     const uint32_t qprime_pt = read_point();
@@ -294,7 +293,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
       std::vector<std::vector<HFe>> pts(nps), nums(nps);
       std::vector<HFe> inv2;
       for (uint32_t s2 = 0; s2 < nps; ++s2) {
-        for (int r : pk.point_sets[s2]) pts[s2].push_back(rot_point(r));
+        for (int r : vk.point_sets[s2]) pts[s2].push_back(rot_point(r));
         HFe den = one;
         for (size_t j = 0; j < pts[s2].size(); ++j) {
           HFe num = one, dj = one;
@@ -333,13 +332,13 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
     uint64_t* vs = &v_scal[(size_t)b * NV * 4];
     uint32_t nvi = 0;
     auto push = [&](const uint64_t* mont_pt, const HFe& sc) { memcpy(vp + (size_t)nvi * 8, mont_pt, 64); F.to_raw(sc, vs + (size_t)nvi * 4); ++nvi; };
-    for (size_t ci = 0; ci < pk.cmap.size(); ++ci) {
-      const int cid = pk.cmap[ci].cid;
-      const HFe sc = F.mul(comm_scalar[ci], x4pow[nps - 1 - pk.cmap[ci].set]);
+    for (size_t ci = 0; ci < vk.cmap.size(); ++ci) {
+      const int cid = vk.cmap[ci].cid;
+      const HFe sc = F.mul(comm_scalar[ci], x4pow[nps - 1 - vk.cmap[ci].set]);
       if (cid == cid_h) { HFe p2 = sc; for (uint32_t i = 0; i < qdeg; ++i) { push(point_mont(h_pt[i]), p2); p2 = F.mul(p2, xn); } }
       else if (cid == cid_rand) push(point_mont(rand_pt), sc);
-      else if (cid >= cid_sig) push(&pk.vk_perm_comm[(size_t)(cid - cid_sig) * 8], sc);
-      else if (cid >= cid_fix) push(&pk.vk_fixed_comm[(size_t)(cid - cid_fix) * 8], sc);
+      else if (cid >= cid_sig) push(&vk.vk_perm_comm[(size_t)(cid - cid_sig) * 8], sc);
+      else if (cid >= cid_fix) push(&vk.vk_fixed_comm[(size_t)(cid - cid_fix) * 8], sc);
       else if (cid >= cid_lk) { const uint32_t l = (cid - cid_lk) / 3, w = (cid - cid_lk) % 3; push(point_mont(w == 0 ? lkA[l] : w == 1 ? lkS[l] : lkz_pt[l]), sc); }
       else if (cid >= cid_pz) push(point_mont(pz_pt[cid - cid_pz]), sc);
       else if (cid >= cid_adv) push(point_mont(adv_pt[cid - cid_adv]), sc);
@@ -358,7 +357,7 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
     fx_extra[2 * b + 1] = F.neg(F.mul(F.mul(c_sc, bb), z));          // U
   }
   // ---- device: compute_s, the fixed-base part, the final check
-  DevBuf &d_sc = pk.vwork[7], &d_s = pk.vwork[8], &d_fx = pk.vwork[9], &d_fptrs = pk.vwork[10], &d_fpart = pk.vwork[11], &d_vp = pk.vwork[12], &d_vs = pk.vwork[13], &d_ok = pk.vwork[14];
+  DevBuf &d_sc = vk.vwork[7], &d_s = vk.vwork[8], &d_fx = vk.vwork[9], &d_fptrs = vk.vwork[10], &d_fpart = vk.vwork[11], &d_vp = vk.vwork[12], &d_vs = vk.vwork[13], &d_ok = vk.vwork[14];
   d_sc.ensure(s_consts.size() * 32); d_s.ensure((size_t)B * n * 32); d_fx.ensure((size_t)B * 64);
   d_fpart.ensure((size_t)B * 64); d_vp.ensure(v_pts.size() * 8); d_vs.ensure(v_scal.size() * 8); d_ok.ensure(B);
   BZ_CUDA(cudaMemcpyAsync(d_sc.p, s_consts.data(), s_consts.size() * 32, cudaMemcpyHostToDevice, st));
@@ -382,18 +381,75 @@ void Verifier::run(const void* instances, const uint32_t* instance_lens, uint32_
 
 }  // namespace bz
 
+namespace bz {
+
+static void check_verify_args(const VkImpl& vk, const void* instances, const uint32_t* instance_lens, uint32_t instance_stride) {
+  BZ_CHECK(vk.cs.I == 0 || (instances && instance_lens), "instances missing");
+  for (uint32_t i = 0; i < vk.cs.I; ++i) BZ_CHECK(instance_lens[i] <= instance_stride, "instance_lens[i] exceeds instance_stride");
+}
+
+// keygen_vk's commitments as the caller hands them over: `count` affine points (x || y, Montgomery).  A real vk never holds the
+// identity (keygen_vk commits with Blind::default(), which adds [1]W), and the final check takes its bases as affine points.
+static void take_commitments(const bzh::Field& Fq, const void* src, uint32_t count, const char* what, std::vector<uint64_t>& dst) {
+  dst.resize((size_t)count * 8);
+  if (count) memcpy(dst.data(), src, dst.size() * 8);
+  const HFe five = Fq.from_u64(5);
+  for (uint32_t i = 0; i < count; ++i) {
+    const uint64_t* p = &dst[(size_t)i * 8];
+    const std::string at = std::string(what) + " commitment " + std::to_string(i);
+    BZ_CHECK(!Fq.geq_mod(p) && !Fq.geq_mod(p + 4), at + ": coordinate not canonical (>= q)");
+    HFe x, y; memcpy(x.l, p, 32); memcpy(y.l, p + 4, 32);
+    BZ_CHECK(!(x.is_zero() && y.is_zero()), at + " is the identity");
+    BZ_CHECK(Fq.sqr(y) == Fq.add(Fq.mul(Fq.sqr(x), x), five), at + " is not on y^2 = x^3 + 5");
+  }
+}
+
+}  // namespace bz
+
 extern "C" API int bz_verify_proofs(bz_ctx* ctx, bz_pk* pkh, uint32_t batch, const void* instances, const uint32_t* instance_lens,
                                     uint32_t instance_stride, const void* proofs, uint32_t proof_len, uint8_t* results) {
   PV_TRY(ctx, {
     BZ_CHECK(pkh && proofs && results && batch >= 1, "null argument");
     PkImpl& pk = pkh->p;
-    BZ_CHECK(pk.cs.I == 0 || (instances && instance_lens), "instances missing");
-    for (uint32_t i = 0; i < pk.cs.I; ++i) BZ_CHECK(instance_lens[i] <= instance_stride, "instance_lens[i] exceeds instance_stride");
+    check_verify_args(pk, instances, instance_lens, instance_stride);
     if (pk.vk_fixed_comm.size() + pk.vk_perm_comm.size() != (size_t)(pk.cs.F + pk.M) * 8) {
       int rc = bz_pk_vk_commitments(ctx, pkh, nullptr, nullptr);
       if (rc != BZ_OK) return rc;
     }
     Verifier vf(C, pk, batch);
+    vf.run(instances, instance_lens, instance_stride, (const uint8_t*)proofs, proof_len, results);
+  });
+}
+
+extern "C" API int bz_vk_create(bz_ctx* ctx, bz_params* params, const bz_circuit* cin, const void* fixed_commitments,
+                                const void* perm_commitments, bz_vk** out) {
+  PV_TRY(ctx, {
+    BZ_CHECK(out && params && cin, "null argument");
+    *out = nullptr;
+    BZ_CHECK(params->p.curve == 0, "verifying key: only the Vesta commitment curve (circuits over pallas::Base) is wired up");
+    BZ_CHECK(cin->k == params->p.k, "circuit k != params k");
+    BZ_CHECK(fixed_commitments || !cin->num_fixed, "null fixed_commitments");
+    BZ_CHECK(perm_commitments || !cin->n_perm_columns, "null perm_commitments");
+    std::unique_ptr<bz_vk> h(new bz_vk());
+    VkImpl& vk = h->v;
+    vk.params = &params->p;
+    vk_host_setup(C->fp, vk, cin);
+    take_commitments(C->fq, fixed_commitments, vk.cs.F, "fixed", vk.vk_fixed_comm);
+    take_commitments(C->fq, perm_commitments, vk.M, "permutation", vk.vk_perm_comm);
+    *out = h.release();
+  });
+}
+
+extern "C" API void bz_vk_destroy(bz_vk* vk) { delete vk; }
+extern "C" API uint32_t bz_vk_proof_size(const bz_vk* vk) { return vk ? vk->v.proof_size : 0; }
+
+extern "C" API int bz_verify_proofs_vk(bz_ctx* ctx, bz_vk* vkh, uint32_t batch, const void* instances, const uint32_t* instance_lens,
+                                       uint32_t instance_stride, const void* proofs, uint32_t proof_len, uint8_t* results) {
+  PV_TRY(ctx, {
+    BZ_CHECK(vkh && proofs && results && batch >= 1, "null argument");
+    VkImpl& vk = vkh->v;
+    check_verify_args(vk, instances, instance_lens, instance_stride);
+    Verifier vf(C, vk, batch);
     vf.run(instances, instance_lens, instance_stride, (const uint8_t*)proofs, proof_len, results);
   });
 }

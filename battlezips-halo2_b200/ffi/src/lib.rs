@@ -24,6 +24,7 @@ pub use sys::*;
 #[repr(C)] pub struct bz_ctx { _p: [u8; 0] }
 #[repr(C)] pub struct bz_params { _p: [u8; 0] }
 #[repr(C)] pub struct bz_pk { _p: [u8; 0] }
+#[repr(C)] pub struct bz_vk { _p: [u8; 0] }
 #[repr(C)] pub struct bz_ipa { _p: [u8; 0] }
 /// all-gather callback of bz_ctx_set_sharding: gather `bytes_per_rank` bytes of every rank's send buffer into the receive buffer
 pub type bz_allgather_fn = Option<unsafe extern "C" fn(user: *mut c_void, bytes_per_rank: usize) -> c_int>;
@@ -270,6 +271,24 @@ impl DevicePk {
     pub fn proof_size(&self) -> usize { unsafe { bz_pk_proof_size(self.0) as usize } }
 }
 
+/// `VerifyingKey` on the device: the flattened `vk.cs`, `vk.fixed_commitments` and the permutation commitments.  No fixed values
+/// and no sigma columns; creating it allocates no device memory.  `params` must outlive it.
+pub struct DeviceVk(pub *mut bz_vk);
+unsafe impl Send for DeviceVk {}
+unsafe impl Sync for DeviceVk {}
+impl Drop for DeviceVk { fn drop(&mut self) { unsafe { bz_vk_destroy(self.0) } } }
+impl DeviceVk {
+    pub fn new(params: &DeviceParams, cs: &FlatCs, fixed_commitments: &[vesta::Affine], perm_commitments: &[vesta::Affine]) -> Result<Self, BzError> {
+        let (fc, pc) = (flatten_points(fixed_commitments), flatten_points(perm_commitments));
+        let mut h = std::ptr::null_mut();
+        let c = ctx();
+        let ffi = cs.as_ffi();
+        check(c, unsafe { bz_vk_create(c, params.0, &ffi, fc.as_ptr() as *const c_void, pc.as_ptr() as *const c_void, &mut h) })?;
+        Ok(DeviceVk(h))
+    }
+    pub fn proof_size(&self) -> usize { unsafe { bz_vk_proof_size(self.0) as usize } }
+}
+
 // ---- create_proof / verify_proof ------------------------------------------------------------------------------------------
 /// Pre-draw the RNG words `create_proof` consumes, in protocol order (`bz_pk_num_random` is shape-only).  `Fp::random(rng)` is
 /// `from_u512` of eight `next_u64()` little-endian limbs (ff 0.12 `Field::random` for pasta); the device performs the same
@@ -304,6 +323,15 @@ pub fn create_proofs<R: RngCore>(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], advi
 
 /// `verify_proof` with `SingleVerifier` semantics: one verdict per proof
 pub fn verify_proofs(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], proofs: &[Vec<u8>]) -> Result<Vec<bool>, BzError> {
+    verify_with(instances, proofs, |c, batch, inst, lens, stride, flat, len, res| unsafe { bz_verify_proofs(c, pk.0, batch, inst, lens, stride, flat, len, res) })
+}
+/// The same from a verifying key alone (what `plonk::verify_proof` is given)
+pub fn verify_proofs_vk(vk: &DeviceVk, instances: &[Vec<Vec<Fp>>], proofs: &[Vec<u8>]) -> Result<Vec<bool>, BzError> {
+    verify_with(instances, proofs, |c, batch, inst, lens, stride, flat, len, res| unsafe { bz_verify_proofs_vk(c, vk.0, batch, inst, lens, stride, flat, len, res) })
+}
+/// packs the batch and calls `call(ctx, batch, instances, instance_lens, instance_stride, proofs, proof_len, results)`
+fn verify_with(instances: &[Vec<Vec<Fp>>], proofs: &[Vec<u8>],
+               call: impl Fn(*mut bz_ctx, u32, *const c_void, *const u32, u32, *const c_void, u32, *mut u8) -> c_int) -> Result<Vec<bool>, BzError> {
     let batch = proofs.len();
     let ncol = instances.first().map(|i| i.len()).unwrap_or(0);
     let lens: Vec<u32> = (0..ncol).map(|c| instances[0][c].len() as u32).collect();
@@ -316,7 +344,7 @@ pub fn verify_proofs(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], proofs: &[Vec<u8
     let flat: Vec<u8> = proofs.iter().flat_map(|p| { assert_eq!(p.len(), len); p.iter().copied() }).collect();
     let mut res = vec![0u8; batch];
     let c = ctx();
-    check(c, unsafe { bz_verify_proofs(c, pk.0, batch as u32, inst.as_ptr() as *const c_void, lens.as_ptr(), stride, flat.as_ptr() as *const c_void, len as u32, res.as_mut_ptr()) })?;
+    check(c, call(c, batch as u32, inst.as_ptr() as *const c_void, lens.as_ptr(), stride, flat.as_ptr() as *const c_void, len as u32, res.as_mut_ptr()))?;
     Ok(res.into_iter().map(|r| r == 1).collect())
 }
 

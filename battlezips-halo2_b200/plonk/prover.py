@@ -62,6 +62,14 @@ def _bind(lib):
     lib.bz_pk_vk_commitments.argtypes = [vp, vp, vp, vp]
     lib.bz_verify_proofs.restype = i32
     lib.bz_verify_proofs.argtypes = [vp, vp, u32, vp, vp, u32, vp, u32, vp]
+    lib.bz_vk_create.restype = i32
+    lib.bz_vk_create.argtypes = [vp, vp, ctypes.POINTER(bz_circuit), vp, vp, ctypes.POINTER(vp)]
+    lib.bz_vk_destroy.restype = None
+    lib.bz_vk_destroy.argtypes = [vp]
+    lib.bz_vk_proof_size.restype = u32
+    lib.bz_vk_proof_size.argtypes = [vp]
+    lib.bz_verify_proofs_vk.restype = i32
+    lib.bz_verify_proofs_vk.argtypes = [vp, vp, u32, vp, vp, u32, vp, u32, vp]
     lib.bz_pk_destroy.restype = None
     lib.bz_pk_destroy.argtypes = [vp]
     lib.bz_pk_num_random.restype = u32
@@ -225,7 +233,7 @@ class ProvingKey:
 
     def __init__(self, ctx, params, ir, fixed_values, mapping, vk_repr, host_sigma=False):
         _bind(ctx.lib)
-        self.ctx, self.params, self.ir = ctx, params, ir
+        self.ctx, self.params, self.ir, self.vk_repr = ctx, params, ir, vk_repr
         self.k, self.n = params.k, params.n
         circ, keep = flatten_circuit(ir, params.k, vk_repr)
         fixed = mont([v for col in fixed_values for v in col]) if fixed_values else np.zeros((1, 4), np.uint64)
@@ -254,6 +262,11 @@ class ProvingKey:
         self.ctx._check(self.ctx.lib.bz_pk_vk_commitments(self.ctx.h, self.h, _np_ptr(fc), _np_ptr(pc)))
         return fc[:F], pc[:M]
 
+    def verifying_key(self):
+        """keygen_vk's result as an independent VerifyingKey: it keeps no reference to this proving key, which may be closed."""
+        fc, pc = self.vk_commitments()
+        return VerifyingKey(self.ctx, self.params, self.ir, fc, pc, self.vk_repr)
+
     def quotient(self, polys, theta, beta, gamma, y):
         """vanishing::Argument::construct up to h(X)'s coefficients (bz_pk_quotient): polys = (slots, n, 4) coefficient
         forms in the order advice, instance, per lookup (A', S', Z), permutation z; challenges as (4,) Montgomery limbs.
@@ -270,6 +283,34 @@ class ProvingKey:
     def close(self):
         if self.h:
             self.ctx.lib.bz_pk_destroy(self.h)
+            self.h = None
+
+
+class VerifyingKey:
+    """halo2's `VerifyingKey` on the device side: the constraint system, keygen_vk's commitments (fixed (F, 8) and permutation
+    (M, 8) Montgomery affine points) and the vk.hash_into scalar.  Holds no fixed values and no sigma columns, and creating it
+    allocates no device memory; `params` must stay open while it is used."""
+
+    def __init__(self, ctx, params, ir, fixed_commitments, perm_commitments, vk_repr):
+        _bind(ctx.lib)
+        self.ctx, self.params, self.ir, self.vk_repr = ctx, params, ir, vk_repr
+        self.k, self.n = params.k, params.n
+        circ, keep = flatten_circuit(ir, params.k, vk_repr)
+        F, M = ir["num_fixed"], len(ir["permutation"])
+        fc = np.ascontiguousarray(fixed_commitments, dtype=np.uint64).reshape(-1, 8)
+        pc = np.ascontiguousarray(perm_commitments, dtype=np.uint64).reshape(-1, 8)
+        if fc.shape[0] != F or pc.shape[0] != M:
+            raise ValueError(f"VerifyingKey: expected {F} fixed and {M} permutation commitments, got {fc.shape[0]} and {pc.shape[0]}")
+        fc = fc if F else np.zeros((1, 8), np.uint64)
+        pc = pc if M else np.zeros((1, 8), np.uint64)
+        h = ctypes.c_void_p()
+        ctx._check(ctx.lib.bz_vk_create(ctx.h, params.h, ctypes.byref(circ), _np_ptr(fc), _np_ptr(pc), ctypes.byref(h)))
+        self.h = h
+        self.proof_size = ctx.lib.bz_vk_proof_size(h)
+
+    def close(self):
+        if self.h:
+            self.ctx.lib.bz_vk_destroy(self.h)
             self.h = None
 
 
@@ -313,8 +354,8 @@ def _pack_instances(pk, instances, B):
 
 
 def verify_proofs(pk, instances, proofs):
-    """plonk::verify_proof for a batch: instances[b] = list (num_instance) of int lists, proofs[b] = bytes (equal lengths).
-    Returns a list of bools (Ok / Err of the reference's SingleVerifier)."""
+    """plonk::verify_proof for a batch: pk = a VerifyingKey or a ProvingKey, instances[b] = list (num_instance) of int lists,
+    proofs[b] = bytes (equal lengths).  Returns a list of bools (Ok / Err of the reference's SingleVerifier)."""
     ctx = pk.ctx
     B = len(proofs)
     plen = len(proofs[0])
@@ -323,5 +364,6 @@ def verify_proofs(pk, instances, proofs):
     inst, lens, stride = _pack_instances(pk, instances, B)
     buf = np.frombuffer(b"".join(proofs) or b"\0", dtype=np.uint8).copy()
     res = np.zeros(B, dtype=np.uint8)
-    ctx._check(ctx.lib.bz_verify_proofs(ctx.h, pk.h, B, _np_ptr(inst), _np_ptr(lens), stride, _np_ptr(buf), plen, _np_ptr(res)))
+    verify = ctx.lib.bz_verify_proofs_vk if isinstance(pk, VerifyingKey) else ctx.lib.bz_verify_proofs
+    ctx._check(verify(ctx.h, pk.h, B, _np_ptr(inst), _np_ptr(lens), stride, _np_ptr(buf), plen, _np_ptr(res)))
     return [bool(x) for x in res]

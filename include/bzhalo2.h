@@ -245,9 +245,27 @@ int bz_create_proofs(bz_ctx* ctx, bz_pk* pk, uint32_t batch, const void* instanc
  * /root/reference/benches/board.rs:84, src/circuits/shot.rs:933-940, src/circuits/board.rs:925-932).
  *   instances : as for bz_create_proofs      proofs : batch x proof_len bytes (host)
  *   results   : batch bytes, 1 = Ok(()), 0 = Err(_) (malformed point / scalar, wrong length, failed opening)
- * Point decompression, the instance commitments, compute_s and the final multi-scalar check run on the device. */
+ * Point decompression, the instance commitments, compute_s and the final multi-scalar check run on the device.
+ * Through a proving key, keygen_vk's commitments are computed on the first call and cached; bz_verify_proofs_vk below
+ * verifies from a verifying key alone. */
 int bz_verify_proofs(bz_ctx* ctx, bz_pk* pk, uint32_t batch, const void* instances, const uint32_t* instance_lens,
                      uint32_t instance_stride, const void* proofs, uint32_t proof_len, uint8_t* results);
+
+/* The verifying key (U: halo2_proofs 0.2.0 src/plonk.rs `VerifyingKey`): what a process that only verifies holds -- the
+ * constraint system (its k, domain and vk.hash_into scalar in `cs`), keygen_vk's fixed commitments (num_fixed x 64 B) and
+ * permutation commitments (n_perm_columns x 64 B), affine Montgomery as bz_pk_vk_commitments returns them (host memory; NULL
+ * only for an empty list).  No fixed values, no sigma columns: creating a vk allocates no device memory, and verifying needs
+ * no proving key.  `params` must outlive the vk.  BZ_ERR_INVALID for a null argument, cs.k != params' k, Pallas params, or a
+ * commitment that has a coordinate >= q, is not on y^2 = x^3 + 5, or is the identity (keygen_vk's Blind::default() adds
+ * [1]W, so a real vk never holds it). */
+typedef struct bz_vk bz_vk;
+int bz_vk_create(bz_ctx* ctx, bz_params* params, const bz_circuit* cs, const void* fixed_commitments,
+                 const void* perm_commitments, bz_vk** out);
+void bz_vk_destroy(bz_vk* vk);
+uint32_t bz_vk_proof_size(const bz_vk* vk); /* bytes of one proof of this circuit */
+/* bz_verify_proofs from a verifying key: same arguments, checks and verdicts */
+int bz_verify_proofs_vk(bz_ctx* ctx, bz_vk* vk, uint32_t batch, const void* instances, const uint32_t* instance_lens,
+                        uint32_t instance_stride, const void* proofs, uint32_t proof_len, uint8_t* results);
 
 /* ==================================================================================================
  * Fine-grained prover arithmetic (SURVEY 8b "minimum export set"): one call per inner loop of halo2_proofs 0.2.0, what a
