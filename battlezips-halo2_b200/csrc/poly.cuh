@@ -264,6 +264,10 @@ __global__ void __launch_bounds__(LKP_THREADS) lookup_permute_kernel(Regions reg
 }
 
 // ---- grand products ----------------------------------------------------------------------------------
+// halo2 multiplies every numerator by batch_invert(den), which leaves the inverse of a zero denominator at zero, so
+// z[i+1] = z[i] * num[i] * inv0(den[i]) drops to 0 after a zero denominator and is unaffected before it.  The fraction
+// kernels store such a row as (num, den) = (0, 1): the term is the same, and every suffix product of den stays non-zero,
+// which the finish kernels (z[i] = z0 * pnum[i] * sden[i] / sden[0]) need.
 // permutation fractions for one column set: num[i] = prod_j (v_j + (beta delta^j) w^i + gamma),
 //                                            den[i] = prod_j (v_j + beta sigma_j + gamma)
 struct PermSetDesc { uint32_t ncols; uint32_t val_kind[8]; uint32_t val_slot[8]; uint32_t sigma_slot[8]; uint32_t bd_const[8]; };
@@ -286,6 +290,7 @@ __global__ void perm_fraction_kernel(Regions reg, uint32_t n, PermSetDesc d, con
     de = fe_mul(de, fe_add(vg, fe_mul(beta, s)));
     nu = fe_mul(nu, fe_add(vg, fe_mul(fe_load(cb + d.bd_const[j]), w)));
   }
+  if (fe_is_zero(de)) { nu = fe_zero<P>(); de = fe_one<P>(); }
   fe_store(num + (uint64_t)b * nd_stride + i, nu);
   fe_store(den + (uint64_t)b * nd_stride + i, de);
 }
@@ -302,6 +307,7 @@ __global__ void lookup_fraction_kernel(Regions reg, uint32_t n, PolyRef cin, Pol
   Fe<P> beta = fe_load(cb + c_beta), gamma = fe_load(cb + c_gamma);
   Fe<P> nu = fe_mul(fe_add(fe_load(region_ptr<P>(reg, cin, b, n) + i), beta), fe_add(fe_load(region_ptr<P>(reg, ctab, b, n) + i), gamma));
   Fe<P> de = fe_mul(fe_add(fe_load(region_ptr<P>(reg, ap, b, n) + i), beta), fe_add(fe_load(region_ptr<P>(reg, sp, b, n) + i), gamma));
+  if (fe_is_zero(de)) { nu = fe_zero<P>(); de = fe_one<P>(); }
   fe_store(num + (uint64_t)b * nd_stride + i, nu);
   fe_store(den + (uint64_t)b * nd_stride + i, de);
 }
@@ -406,7 +412,7 @@ __global__ void grand_product_finish_kernel(const Fe<P>* __restrict__ pnum, cons
 // All grand products of a proof in one launch (blockIdx.z = product): the first `nsets` products are the permutation sets,
 // chained through z_s[0] = z_{s-1}[u] (u = first unusable row); the others (lookups) start at 1.
 //   z_g[i] = z0_g * pnum_g[i] * sden_g[i] / sden_g[0],   z0_s = prod_{s' < s} pnum_s'[u] * sden_s'[u] / sden_s'[0]
-// The <= 8 inversions a product needs share one Fermat chain (Montgomery's trick, zeros skipped), so a batch pays the
+// The <= 8 inversions a product needs share one Fermat chain (Montgomery's trick; no sden is zero), so a batch pays the
 // inversion latency once instead of once per product.  ONE CTA per (proof, product) walks all rows: B x G inversions per batch
 // (launch site in prover.cu).
 struct GpBatchDesc { uint32_t nprod, nsets; PolyRef zref[8]; };
@@ -422,13 +428,13 @@ __global__ void grand_product_finish_batch_kernel(const Fe<P>* __restrict__ pnum
     for (uint32_t gp = g0; gp <= g; ++gp) {
       s0[gp - g0] = fe_load(sden + (uint64_t)gp * prod_stride + (uint64_t)b * nd_stride);
       pre[gp - g0] = acc;
-      if (!fe_is_zero(s0[gp - g0])) acc = fe_mul(acc, s0[gp - g0]);
+      acc = fe_mul(acc, s0[gp - g0]);
     }
     Fe<P> inv = fe_inv_gcd(acc);
     Fe<P> z0 = fe_one<P>(), mine = fe_zero<P>();
     for (uint32_t gp = g + 1; gp-- > g0;) {                       // 1 / sden_gp[0], last product first
-      Fe<P> iv = fe_zero<P>();
-      if (!fe_is_zero(s0[gp - g0])) { iv = fe_mul(inv, pre[gp - g0]); inv = fe_mul(inv, s0[gp - g0]); }
+      const Fe<P> iv = fe_mul(inv, pre[gp - g0]);
+      inv = fe_mul(inv, s0[gp - g0]);
       if (gp == g) mine = iv;
       else {
         const uint64_t at = (uint64_t)gp * prod_stride + (uint64_t)b * nd_stride + u;

@@ -278,6 +278,7 @@ int bz_verify_proofs_vk(bz_ctx* ctx, bz_vk* vk, uint32_t batch, const void* inst
  * values[j] / sigmas[j] = the set's ncols (<= 8, i.e. cs degree <= 10) columns and their sigma columns (Lagrange values),
  * delta_omega0 = DELTA^(index of the set's first column), z0 = last_z of the previous set (ONE for the first).
  * out_z[0] = z0, out_z[i+1] = out_z[i] * prod_j (v_j[i] + delta_omega0 DELTA^j omega^i beta + gamma) / (v_j[i] + beta sigma_j[i] + gamma);
+ * the division is halo2's batch_invert, which takes 1/0 as 0: a zero denominator at row i makes out_z[i+1..] zero;
  * the caller overwrites the last `blinding_factors` rows and reads last_z = z[n - blinding_factors - 1] like upstream. */
 int bz_perm_product(bz_ctx* ctx, int field, uint32_t k, uint32_t ncols, const void* const* values, const void* const* sigmas,
                     const void* beta, const void* gamma, const void* delta_omega0, const void* z0, void* out_z);
@@ -287,7 +288,8 @@ int bz_perm_product(bz_ctx* ctx, int field, uint32_t k, uint32_t ncols, const vo
  * (Error::ConstraintSystemFailure). */
 int bz_lookup_permute(bz_ctx* ctx, int field, uint32_t k, uint32_t usable_rows, const void* compressed_input,
                       const void* compressed_table, void* out_permuted_input, void* out_permuted_table);
-/* lookup::Permuted::commit_product: z[0] = 1, z[i+1] = z[i] (A[i] + beta)(S[i] + gamma) / ((A'[i] + beta)(S'[i] + gamma)); n scalars out */
+/* lookup::Permuted::commit_product: z[0] = 1, z[i+1] = z[i] (A[i] + beta)(S[i] + gamma) / ((A'[i] + beta)(S'[i] + gamma)); n scalars out;
+ * 1/0 is taken as 0 as in bz_perm_product */
 int bz_lookup_product(bz_ctx* ctx, int field, uint32_t k, const void* compressed_input, const void* compressed_table,
                       const void* permuted_input, const void* permuted_table, const void* beta, const void* gamma, void* out_z);
 /* EvaluationDomain::divide_by_vanishing_poly (U: src/poly/domain.rs): a[i] *= t_evaluations[i mod 2^(extended_k - k)], in place,

@@ -301,6 +301,71 @@ def construct_intermediate_sets(queries):
 
 
 # ------------------------------------------------------------------------------------------------------
+# argument inner loops  [U: src/plonk/lookup/prover.rs, src/plonk/permutation/prover.rs]
+# ------------------------------------------------------------------------------------------------------
+def permute_expression_pair(V, usable, cin, ctab):
+    """lookup::prover::permute_expression_pair over the first `usable` rows of the compressed input / table ((n,4)
+    Montgomery arrays) -> (A', S'), `usable` rows each.  A' is the input sorted by canonical value; S' holds the table
+    value next to the first row of every run of equal inputs, and the left-over table values fill the repeated rows,
+    last row first, in BTreeMap (ascending) order.  An input value missing from the table's usable rows raises
+    ValueError("Error::ConstraintSystemFailure")."""
+    a_keys = V.sort_keys(cin[:usable])
+    s_keys = V.sort_keys(ctab[:usable])
+    a_list = [bytes(r) for r in a_keys]
+    order = sorted(range(usable), key=lambda i: a_list[i])
+    permuted_input = np.ascontiguousarray(cin[:usable][order]).reshape(-1, 4)
+    a_sorted = [a_list[i] for i in order]
+    leftover = {}
+    s_val = {}
+    for i in range(usable):
+        kb = bytes(s_keys[i])
+        leftover[kb] = leftover.get(kb, 0) + 1
+        s_val[kb] = ctab[i]
+    permuted_table = V.zeros(usable)
+    repeated = []
+    for row in range(usable):
+        if row == 0 or a_sorted[row] != a_sorted[row - 1]:
+            permuted_table[row] = permuted_input[row]
+            if a_sorted[row] not in leftover:
+                raise ValueError("Error::ConstraintSystemFailure")     # input value not in table
+            assert leftover[a_sorted[row]] > 0
+            leftover[a_sorted[row]] -= 1
+        else:
+            repeated.append(row)
+    for kb in sorted(leftover.keys()):            # BTreeMap iteration = ascending numeric order
+        for _ in range(leftover[kb]):
+            permuted_table[repeated.pop()] = s_val[kb]
+    assert not repeated
+    return permuted_input, permuted_table
+
+
+def permutation_product(V, omega, values, sigmas, beta, gamma, delta_omega0, z0):
+    """permutation::Argument::commit for one column set, before blinding: z[0] = z0,
+    z[i+1] = z[i] * prod_j (v_j[i] + beta delta_omega0 delta^j omega^i + gamma) * inv0(prod_j (v_j[i] + beta sigma_j[i] + gamma)),
+    where inv0 (ff::BatchInvert) leaves zero at zero.  values / sigmas: lists of (n,4) Montgomery arrays; scalars are ints."""
+    n, p = len(values[0]), V.p
+    modified = V.const(1, n)
+    for v, s in zip(values, sigmas):
+        modified = V.mul(modified, V.add(V.add_const(V.scale(s, beta), gamma), v))
+    modified = V.batch_invert(modified)
+    omega_pows = V.powers(1, omega, n)
+    deltaomega = delta_omega0
+    for v in values:
+        modified = V.mul(modified, V.add(V.add_const(V.scale(omega_pows, deltaomega * beta % p), gamma), v))
+        deltaomega = deltaomega * V.F.delta % p
+    return V.running_product(z0, modified)
+
+
+def lookup_product(V, cin, ctab, pin, ptab, beta, gamma):
+    """lookup::Permuted::commit_product before blinding: z[0] = 1,
+    z[i+1] = z[i] * (cin[i] + beta)(ctab[i] + gamma) * inv0((pin[i] + beta)(ptab[i] + gamma))."""
+    prod = V.batch_invert(V.mul(V.add_const(pin, beta), V.add_const(ptab, gamma)))
+    prod = V.mul(prod, V.add_const(cin, beta))
+    prod = V.mul(prod, V.add_const(ctab, gamma))
+    return V.running_product(1, prod)
+
+
+# ------------------------------------------------------------------------------------------------------
 # create_proof  [U: src/plonk/prover.rs and the argument provers; SURVEY App. A steps 0-21]
 # ------------------------------------------------------------------------------------------------------
 def create_proof(params, pk, instances, advice, draws, transcript, trace=None):
@@ -390,34 +455,7 @@ def create_proof(params, pk, instances, advice, draws, transcript, trace=None):
             return acc
         L = {"compressed_input": compress(lk["input"], lagrange_leaf, n),
              "compressed_table": compress(lk["table"], lagrange_leaf, n)}
-        # permute_expression_pair
-        a_keys = V.sort_keys(L["compressed_input"][:usable])
-        s_keys = V.sort_keys(L["compressed_table"][:usable])
-        a_list = [bytes(r) for r in a_keys]
-        order = sorted(range(usable), key=lambda i: a_list[i])
-        permuted_input = L["compressed_input"][:usable][order]
-        a_sorted = [a_list[i] for i in order]
-        leftover = {}
-        s_val = {}
-        for i in range(usable):
-            kb = bytes(s_keys[i])
-            leftover[kb] = leftover.get(kb, 0) + 1
-            s_val[kb] = L["compressed_table"][i]
-        permuted_table = V.zeros(usable)
-        repeated = []
-        for row in range(usable):
-            if row == 0 or a_sorted[row] != a_sorted[row - 1]:
-                permuted_table[row] = permuted_input[row]
-                if a_sorted[row] not in leftover:
-                    raise ValueError("Error::ConstraintSystemFailure")     # input value not in table
-                assert leftover[a_sorted[row]] > 0
-                leftover[a_sorted[row]] -= 1
-            else:
-                repeated.append(row)
-        for kb in sorted(leftover.keys()):            # BTreeMap iteration = ascending numeric order
-            for _ in range(leftover[kb]):
-                permuted_table[repeated.pop()] = s_val[kb]
-        assert not repeated
+        permuted_input, permuted_table = permute_expression_pair(V, usable, L["compressed_input"], L["compressed_table"])
         permuted_input = np.concatenate([permuted_input, rnd(bf + 1)])
         permuted_table = np.concatenate([permuted_table, rnd(bf + 1)])
         L["permuted_input"], L["permuted_table"] = permuted_input, permuted_table
@@ -450,25 +488,16 @@ def create_proof(params, pk, instances, advice, draws, transcript, trace=None):
     sets = []
     deltaomega = 1
     last_z = 1
-    omega_pows = V.powers(1, dom.omega, n)
 
     def col_values(kind, col):
         return {"advice": advice_values, "fixed": pk.fixed_values, "instance": instance_values}[kind][col]
 
     for s0 in range(0, len(perm_cols), chunk_len):
         cols = perm_cols[s0:s0 + chunk_len]
-        tr["perm_sets"].append({"values": [col_values(kind, col) for kind, col in cols], "sigmas": [pk.perm_values[s0 + j] for j in range(len(cols))],
-                                "delta_omega0": deltaomega, "z0": last_z})
-        modified = V.const(1, n)
-        for j, (kind, col) in enumerate(cols):
-            t = V.add(V.add_const(V.scale(pk.perm_values[s0 + j], beta), gamma), col_values(kind, col))
-            modified = V.mul(modified, t)
-        modified = V.batch_invert(modified)
-        for (kind, col) in cols:
-            t = V.add(V.add_const(V.scale(omega_pows, deltaomega * beta % p), gamma), col_values(kind, col))
-            modified = V.mul(modified, t)
-            deltaomega = deltaomega * V.F.delta % p
-        z = V.running_product(last_z, modified)
+        values, sigmas = [col_values(kind, col) for kind, col in cols], pk.perm_values[s0:s0 + len(cols)]
+        tr["perm_sets"].append({"values": values, "sigmas": sigmas, "delta_omega0": deltaomega, "z0": last_z})
+        z = permutation_product(V, dom.omega, values, sigmas, beta, gamma, deltaomega, last_z)
+        deltaomega = deltaomega * pow(V.F.delta, len(cols), p) % p
         tr["perm_sets"][-1]["z_unblinded"] = z.copy()
         z[n - bf:] = rnd(bf)
         last_z = V.int1(z[n - (bf + 1)])
@@ -482,13 +511,8 @@ def create_proof(params, pk, instances, advice, draws, transcript, trace=None):
 
     # step 8: lookup products
     for L in lookups:
-        den = V.mul(V.add_const(L["permuted_input"], beta), V.add_const(L["permuted_table"], gamma))
-        prod = V.batch_invert(den)
-        prod = V.mul(prod, V.add_const(L["compressed_input"], beta))
-        prod = V.mul(prod, V.add_const(L["compressed_table"], gamma))
-        z_full = V.running_product(1, np.concatenate([prod, V.zeros(1)]))      # z[0]=1, z[i]=prod of first i
-        L["z_unblinded"] = z_full[:n].copy()
-        z = np.concatenate([z_full[:n - bf], rnd(bf)])
+        L["z_unblinded"] = lookup_product(V, L["compressed_input"], L["compressed_table"], L["permuted_input"], L["permuted_table"], beta, gamma)
+        z = np.concatenate([L["z_unblinded"][:n - bf], rnd(bf)])
         assert len(z) == n
         L["product_blind"] = rnd1()
         comm = _affine_pts(cid, [params.commit_lagrange(z, L["product_blind"])])[0]

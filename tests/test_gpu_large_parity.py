@@ -81,19 +81,24 @@ def test_coset_extension_large_vs_oracle(k, ctx, oracle_c):
         assert np.array_equal(got, dom.extended_to_coeff(big))
 
 
-@pytest.mark.parametrize("k", [15, 16])
-def test_scaled_board_proof_bytes_match_oracle(k, ctx):
+@pytest.mark.parametrize("k,batch", [(15, 1), (16, 1), (16, 2)], ids=["15", "16", "16-batch2"])
+def test_scaled_board_proof_bytes_match_oracle(k, batch, ctx):
     """BASELINE config 5 on the way up: the Board circuit tiled down 2^15 / 2^16 rows, proof bytes against the oracle
-    prover and accepted by the restated verifier and by verify_proof on the device."""
+    prover and accepted by the restated verifier and by verify_proof on the device.  The batch of two (RNG indices 2 and 3
+    in one create_proofs call) runs every per-proof launch site of the large-domain paths with B = 2: the two-level
+    grand-product scan, the split Horner evaluation and Kate division, the lookup permutation per proof and the split
+    IPA inner products."""
     from battlezips_halo2_b200.circuits import board_circuit_scaled
     from battlezips_halo2_b200.plonk import prover as PR
     from tests.util_prover import Job, first_diff
     cs, cfg, asg = board_circuit_scaled(k)
     job = Job(cs, asg, params_from_device=ctx)
     params, pk = job.device_keys(ctx)
-    proof = PR.create_proofs(pk, [job.instances], job.advice[None], job.wide(2)[None])[0]
-    exp = job.oracle_proof(index=2)
-    assert first_diff(proof, exp) is None, first_diff(proof, exp)
-    assert job.verify(proof)
-    assert PR.verify_proofs(pk, [job.instances], [proof]) == [True]
+    indices = range(2, 2 + batch)
+    proofs = PR.create_proofs(pk, [job.instances] * batch, np.stack([job.advice] * batch), np.stack([job.wide(i) for i in indices]))
+    for i, proof in zip(indices, proofs):
+        exp = job.oracle_proof(index=i)
+        assert first_diff(proof, exp) is None, (i, first_diff(proof, exp))
+        assert job.verify(proof)
+    assert PR.verify_proofs(pk, [job.instances] * batch, proofs) == [True] * batch
     pk.close(); params.close()
