@@ -43,12 +43,17 @@ template <class BP> __device__ __noinline__ Xyzz<BP> xyzz_dbl(const Xyzz<BP>& p)
   return r;
 }
 
-// mixed addition acc += q (affine), complete: handles identity / doubling / inverse (madd-2008-s)
+// mixed addition acc += q (affine), complete: handles identity / doubling / inverse (madd-2008-s).
+// The loop body of both MSM accumulation kernels.  Six of its ten multiplications are inlined, four stay calls of the
+// shared out-of-line fe_mul: measured on B200 (1000 W), table-MSM accumulation per IPA-round launch at k = 11, c = 16
+// (scripts/fb_accumulate_time.py): 0 / 2 / 4 / 6 / 7 / 8 / 10 inlined 0.358 / 0.349 / 0.343 / 0.335 / 0.337 / 0.343 /
+// 0.346 ms -- every inlined product drops the call's operand and result moves, until the loop outgrows the instruction
+// cache.
 template <class BP> __device__ __forceinline__ void xyzz_add_mixed(Xyzz<BP>& acc, const Affine<BP>& q) {
   if (aff_is_identity(q)) return;
   if (xyzz_is_identity(acc)) { acc = xyzz_from_affine(q); return; }
-  Fe<BP> u2 = fe_mul(q.x, acc.zz);
-  Fe<BP> s2 = fe_mul(q.y, acc.zzz);
+  Fe<BP> u2 = fe_mul_inline(q.x, acc.zz);
+  Fe<BP> s2 = fe_mul_inline(q.y, acc.zzz);
   Fe<BP> p = fe_sub(u2, acc.x);
   Fe<BP> r = fe_sub(s2, acc.y);
   if (fe_is_zero(p)) {
@@ -57,13 +62,13 @@ template <class BP> __device__ __forceinline__ void xyzz_add_mixed(Xyzz<BP>& acc
     return;
   }
   Fe<BP> pp = fe_sqr(p);
-  Fe<BP> ppp = fe_mul(p, pp);
-  Fe<BP> qq = fe_mul(acc.x, pp);
+  Fe<BP> ppp = fe_mul_inline(p, pp);
+  Fe<BP> qq = fe_mul_inline(acc.x, pp);
   Fe<BP> x3 = fe_sub(fe_sub(fe_sqr(r), ppp), fe_dbl(qq));
   acc.y = fe_sub(fe_mul(r, fe_sub(qq, x3)), fe_mul(acc.y, ppp));
   acc.x = x3;
-  acc.zz = fe_mul(acc.zz, pp);
-  acc.zzz = fe_mul(acc.zzz, ppp);
+  acc.zz = fe_mul_inline(acc.zz, pp);
+  acc.zzz = fe_mul_inline(acc.zzz, ppp);
 }
 
 // acc += sign ? -q : q
@@ -153,6 +158,33 @@ template <class BP> __device__ Xyzz<BP> xyzz_mul_scalar(const Xyzz<BP>& p, const
 
 template <class BP> __device__ __forceinline__ Affine<BP> aff_load(const Affine<BP>* p) {
   Affine<BP> r; r.x = fe_load(&p->x); r.y = fe_load(&p->y); return r;
+}
+
+// Gather staging of the accumulation loops (fixedmsm.cu, msm.cu): the affine point a thread adds next is copied into the
+// thread's own shared-memory slot by cp.async (4 x 16 B, L1-allocating .ca, like the register loads it replaces) instead
+// of waiting in 16 registers while the current addition runs.  Chunk k of the slot of thread t is uint4 k * THREADS + t
+// of the slot array: a warp's copies and reads of one chunk are 512 contiguous bytes (no bank conflicts).
+__device__ __forceinline__ void cp_async16_ca(uint4* smem, const void* gmem) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;\n" :: "r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" :: "n"(N) : "memory"); }
+
+template <int THREADS, class BP> __device__ __forceinline__ void aff_stage(uint4* slot, const Affine<BP>* src) {
+  const uint4* g = reinterpret_cast<const uint4*>(src);
+#pragma unroll
+  for (int k = 0; k < 4; ++k) cp_async16_ca(slot + k * THREADS, g + k);
+}
+template <int THREADS, class BP> __device__ __forceinline__ Affine<BP> aff_staged(const uint4* slot) {
+  Affine<BP> r;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const uint4 v = slot[k * THREADS];
+    Fe<BP>& f = k < 2 ? r.x : r.y;
+    const int o = (k & 1) * 4;
+    f.l[o] = v.x; f.l[o + 1] = v.y; f.l[o + 2] = v.z; f.l[o + 3] = v.w;
+  }
+  return r;
 }
 
 }  // namespace bz

@@ -170,13 +170,16 @@ template <class P> __device__ __forceinline__ Fe<P> fe_mul_c(const Fe<P>& a, con
 #else
 #define BZ_MUL_ATTR __forceinline__
 #endif
+template <class P> __device__ __forceinline__ void fe_mul_body(uint32_t (&r)[8], const uint32_t (&a)[8], const uint32_t (&b)[8]) {
+  mm::mont_mul_wide<P::M1, P::M2, P::M3>(r, a, b);
+  fe_final_sub<P>(r);
+}
 struct MulRet { uint4 lo, hi; };      // returned in registers by the device ABI
 template <class P> __device__ BZ_MUL_ATTR MulRet fe_mul_raw(uint4 a0, uint4 a1, uint4 b0, uint4 b1) {
   uint32_t a[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
   uint32_t b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
   uint32_t r[8];
-  mm::mont_mul_wide<P::M1, P::M2, P::M3>(r, a, b);
-  fe_final_sub<P>(r);
+  fe_mul_body<P>(r, a, b);
   MulRet o;
   o.lo = make_uint4(r[0], r[1], r[2], r[3]); o.hi = make_uint4(r[4], r[5], r[6], r[7]);
   return o;
@@ -187,6 +190,14 @@ template <class P> __device__ __forceinline__ Fe<P> fe_mul(const Fe<P>& a, const
   Fe<P> r;
   r.l[0] = o.lo.x; r.l[1] = o.lo.y; r.l[2] = o.lo.z; r.l[3] = o.lo.w;
   r.l[4] = o.hi.x; r.l[5] = o.hi.y; r.l[6] = o.hi.z; r.l[7] = o.hi.w;
+  return r;
+}
+
+// The same product inlined at the call site, for the few hot call sites where the operand / result moves of the call (~22
+// fma-pipe instructions per multiplication) cost more than the instruction-cache space (see xyzz_add_mixed).
+template <class P> __device__ __forceinline__ Fe<P> fe_mul_inline(const Fe<P>& a, const Fe<P>& b) {
+  Fe<P> r;
+  fe_mul_body<P>(r.l, a.l, b.l);
   return r;
 }
 

@@ -212,16 +212,37 @@ __device__ __forceinline__ uint32_t fb_plan(const uint32_t* __restrict__ list_co
   return max(FB_MIN_SHARE, (total + total_threads - 1) / total_threads);
 }
 
+// The accumulate loop's gathers go through shared memory: every thread keeps the 64 B table points of its next FB_STAGES
+// entries in its own slots, copied by cp.async (4 x 16 B) with one commit group per entry.  No registers hold a
+// prefetched point (no spills; 128 registers and 76 B of spills when the next point was held in registers), and the
+// compiler cannot sink the gather next to its use.  The copies allocate in L1 (.ca), as the register loads did; L2-only
+// copies (.cg) were slower than the register prefetch.  Measured on B200 (1000 W power limit), IPA-round launch at k = 11,
+// c = 16 (scripts/fb_accumulate_time.py), ms per accumulate launch with every multiplication of the addition out of line
+// (the inlining in curve.cuh came after): register prefetch 0.3755; .ca with 1 / 2 / 3 stages
+// 0.357 / 0.363 / 0.366; .cg with 2 / 3 / 4 stages 0.378 / 0.388 / 0.396.  One stage already covers the round trip (an
+// addition is ~10 out-of-line multiplications at 4 warps per scheduler); each further stage takes 16 KB per SM of shared
+// memory out of the L1 carve-out and was slower.  Slot s of thread t starts at uint4 s * 4 * FB_THREADS + t (aff_stage).
+constexpr int FB_STAGES = 1;
+constexpr uint32_t FB_STAGE_BYTES = FB_STAGES * FB_THREADS * 64;
+// dynamic shared memory of the accumulate kernel: the n_msm + 1 offsets of fb_plan, then the stage buffer (16 B aligned)
+__host__ __device__ constexpr uint32_t fb_stage_off16(uint32_t n_msm) { return (n_msm + 4) / 4; }
+__host__ __device__ constexpr uint32_t fb_accumulate_smem(uint32_t n_msm) { return fb_stage_off16(n_msm) * 16 + FB_STAGE_BYTES; }
+
 // Warp W owns the flat entries [W*32q, (W+1)*32q); inside every MSM piece of that range lane l takes entries l, l+32, ...
-// (coalesced list reads) and keeps its own sum.  The table point of the NEXT entry is gathered before the current
-// addition starts, so the list -> table dependent DRAM round trips overlap the ~10 field multiplications of the addition.
+// (coalesced list reads) and keeps its own sum.  Entry j of a lane's piece is added once its copy -- issued FB_STAGES
+// additions earlier -- has landed; the list entry that addresses a copy is read one addition before the copy is issued,
+// so both dependent DRAM round trips (list, then table) overlap additions.  Every lane commits one group per prologue
+// stage and per entry of its own, so each wait counts that lane's copies only; copies past the end of a piece are not
+// issued (their groups are empty) and a piece ends with none in flight.
 // A warp emits 32 partials per MSM it touches, at index (W + m)*32 + lane (unique and increasing along the flat order).
 template <class BP>
 __global__ void __launch_bounds__(FB_THREADS, 4) fb_accumulate_kernel(const Affine<BP>* __restrict__ table, const uint32_t* __restrict__ lists,
                                  uint32_t list_stride, const uint32_t* __restrict__ list_count, uint32_t n_msm,
                                  Xyzz<BP>* __restrict__ partial, unsigned long long* __restrict__ add_counter) {
-  extern __shared__ uint32_t fb_off[];
+  extern __shared__ uint4 fb_acc_smem[];
   __shared__ uint32_t wsum[33];
+  uint32_t* const fb_off = reinterpret_cast<uint32_t*>(fb_acc_smem);
+  uint4* const stage = fb_acc_smem + fb_stage_off16(n_msm) + threadIdx.x;
   const uint32_t T = gridDim.x * FB_THREADS, t = blockIdx.x * FB_THREADS + threadIdx.x, lane = threadIdx.x & 31, W = t >> 5;
   const uint32_t q = fb_plan(list_count, n_msm, T, fb_off, wsum);
   const uint32_t total = fb_off[n_msm];
@@ -235,24 +256,34 @@ __global__ void __launch_bounds__(FB_THREADS, 4) fb_accumulate_kernel(const Affi
     while (pbeg < end) {
       while (fb_off[m + 1] <= pbeg) ++m;               // skip MSMs without entries
       const uint32_t pend = min(end, fb_off[m + 1]);
-      const uint32_t* list = lists + (size_t)m * list_stride - fb_off[m];
+      const uint32_t* list = lists + (size_t)m * list_stride - fb_off[m] + pbeg + lane;
+      const uint32_t n = pbeg + lane < pend ? (pend - pbeg - lane + 31) >> 5 : 0;    // this lane's entries: list[32 j], j < n
       Xyzz<BP> acc = xyzz_identity<BP>();
-      uint32_t p = pbeg + lane;
-      uint32_t ent = 0, ent_n = 0;
-      Affine<BP> pt;
-      if (p < pend) { ent = list[p]; pt = aff_load(table + (ent & 0x7fffffffu)); }
-      if (p + 32 < pend) ent_n = list[p + 32];
-      while (p < pend) {
-        const bool more = p + 32 < pend;
-        Affine<BP> pt_n;
-        uint32_t ent_nn = 0;
-        if (more) pt_n = aff_load(table + (ent_n & 0x7fffffffu));
-        if (p + 64 < pend) ent_nn = list[p + 64];
-        xyzz_add_mixed_signed(acc, pt, (ent >> 31) != 0);
+      uint32_t neg = 0;                                // bit s: sign of entry j + s (the staged ones)
+#pragma unroll
+      for (uint32_t s = 0; s < FB_STAGES; ++s) {
+        if (s < n) {
+          const uint32_t e = list[32 * s];
+          neg |= (e >> 31) << s;
+          aff_stage<FB_THREADS>(stage + s * 4 * FB_THREADS, table + (e & 0x7fffffffu));
+        }
+        cp_async_commit();
+      }
+      uint32_t ent_n = FB_STAGES < n ? list[32 * FB_STAGES] : 0u;     // entry j + FB_STAGES
+      uint32_t slot = 0;
+      for (uint32_t j = 0; j < n; ++j) {
+        const uint32_t ent_nn = j + FB_STAGES + 1 < n ? list[32 * (j + FB_STAGES + 1)] : 0u;
+        uint4* const sp = stage + slot * 4 * FB_THREADS;
+        cp_async_wait<FB_STAGES - 1>();             // entry j's group (the oldest of this lane's pending ones) has landed
+        const Affine<BP> pt = aff_staged<FB_THREADS, BP>(sp);  // read before the refill of the same slot is issued (same thread)
+        if (j + FB_STAGES < n) aff_stage<FB_THREADS>(sp, table + (ent_n & 0x7fffffffu));
+        cp_async_commit();
+        const bool negate = (neg & 1u) != 0;
+        neg = (neg >> 1) | ((ent_n >> 31) << (FB_STAGES - 1));
+        xyzz_add_mixed_signed(acc, pt, negate);
         ++my_adds;
-        if (more) pt = pt_n;
-        ent = ent_n; ent_n = ent_nn;
-        p += 32;
+        ent_n = ent_nn;
+        slot = slot + 1 == FB_STAGES ? 0 : slot + 1;
       }
       Xyzz<BP>* o = partial + ((size_t)W + m) * 32 + lane;
       fe_store(&o->x, acc.x); fe_store(&o->y, acc.y); fe_store(&o->zz, acc.zz); fe_store(&o->zzz, acc.zzz);
@@ -374,9 +405,9 @@ static void fixed_msm_run_t(Ctx* ctx, const FixedBase& fb, const void* const* d_
   const int dev = ctx->device >= 0 && ctx->device < BZ_MAX_DEVICES ? ctx->device : 0;
   once.run(ctx->device, [dev] {
     int ctas_per_sm = 0;
-    cudaFuncSetAttribute(fb_accumulate_kernel<BP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((FB_MAX_MSM + 1) * 4));
+    cudaFuncSetAttribute(fb_accumulate_kernel<BP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fb_accumulate_smem(FB_MAX_MSM));
     int v = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, fb_accumulate_kernel<BP>, FB_THREADS, (FB_MAX_MSM + 1) * 4);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, fb_accumulate_kernel<BP>, FB_THREADS, fb_accumulate_smem(FB_MAX_MSM));
     ctas_per_sm = v < 1 ? 1 : v;
     const int fold_smem = (int)((FB_MAX_MSM + 32) * 4 + FB_FOLD_THREADS_WIDE * sizeof(Xyzz<BP>));
     cudaFuncSetAttribute(fb_fold_kernel<BP, true, FB_FOLD_THREADS_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, fold_smem);
@@ -399,7 +430,7 @@ static void fixed_msm_run_t(Ctx* ctx, const FixedBase& fb, const void* const* d_
     Xyzz<BP>* partial = ctx->scratch[3].as<Xyzz<BP>>();
     BZ_CUDA(cudaMemsetAsync(counts, 0, (size_t)nm * 4, st));
     unsigned long long* cnt = ctx->profiling ? (unsigned long long*)ctx->counters.p : nullptr;
-    const size_t smem = ((size_t)nm + 1) * 4;
+    const size_t smem = fb_accumulate_smem(nm);
     {
       ProfScope p(ctx, PROF_FIXED_MSM);
       fb_decode_kernel<SP><<<dim3((fb.npts + FB_THREADS - 1) / FB_THREADS, nm), FB_THREADS, 0, st>>>(
