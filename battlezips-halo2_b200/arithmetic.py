@@ -5,7 +5,7 @@ Arrays are numpy uint64 of shape (n, 4) [field elements], (n, 8) [affine points]
 pasta's in-memory Montgomery limbs -- exactly the bytes the Rust side owns."""
 import ctypes
 import numpy as np
-from .binding import _np_ptr
+from .binding import _np_ptr, _seed_array
 
 
 def best_multiexp(ctx, curve, coeffs, bases):
@@ -96,6 +96,19 @@ def hash_to_curve(ctx, curve, domain_prefix, messages):
     out = np.zeros((len(msgs), 8), dtype=np.uint64)
     ctx._check(ctx.lib.bz_hash_to_curve(ctx.h, curve, domain_prefix.encode(), _np_ptr(buf), L, len(msgs), _np_ptr(out)))
     return out
+
+
+def chacha20_blocks(ctx, seeds, blocks, out=None):
+    """ChaCha20 keystream blocks 0 .. blocks-1 of every 32-byte seed (bz_chacha20_blocks): seeds = (B, 32) uint8 or a list of
+    32-byte strings.  Returns (B, blocks, 8) uint64 -- rand_wide's layout, the words create_proof's Scalar::random draws read.
+    out: optional device address (int) of B x blocks x 64 bytes to write instead; then nothing is returned."""
+    seeds = _seed_array(seeds)
+    if out is not None:
+        ctx._check(ctx.lib.bz_chacha20_blocks(ctx.h, _np_ptr(seeds), len(seeds), blocks, ctypes.c_void_p(int(out))))
+        return None
+    res = np.empty((len(seeds), blocks, 8), dtype=np.uint64)
+    ctx._check(ctx.lib.bz_chacha20_blocks(ctx.h, _np_ptr(seeds), len(seeds), blocks, _np_ptr(res)))
+    return res
 
 
 def params_new(ctx, k, curve=0):

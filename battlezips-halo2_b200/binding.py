@@ -109,9 +109,10 @@ def load_library():
         "bz_quotient_program": (i32, [vp, u32, vp, u32, ctypes.POINTER(u32), vp, u32, ctypes.POINTER(u32), ctypes.POINTER(u64)]),
         "bz_pk_quotient_generated": (i32, [vp, u32]),
         "bz_ctx_set_sharding": (i32, [vp, u32, u32, vp, vp, ctypes.c_size_t, ALLGATHER_FN, vp]),
+        "bz_chacha20_blocks": (i32, [vp, vp, u32, u64, vp]),
     }
     declared_elsewhere = {"bz_params_create", "bz_params_destroy", "bz_params_commit", "bz_pk_create", "bz_pk_destroy",
-                          "bz_pk_num_random", "bz_pk_proof_size", "bz_pk_quotient_muls", "bz_create_proofs", "bz_pk_create_from_assembly", "bz_pk_vk_commitments", "bz_verify_proofs", "bz_params_commit_batch_dev",
+                          "bz_pk_num_random", "bz_pk_proof_size", "bz_pk_quotient_muls", "bz_create_proofs", "bz_create_proofs_seeded", "bz_pk_create_from_assembly", "bz_pk_vk_commitments", "bz_verify_proofs", "bz_params_commit_batch_dev",
                           "bz_vk_create", "bz_vk_destroy", "bz_vk_proof_size", "bz_verify_proofs_vk"}     # bound in plonk/prover.py
     missing = [n for n in EXPORTS if n not in sigs and n not in declared_elsewhere]
     assert not missing, f"unbound C-ABI symbols: {missing}"
@@ -124,6 +125,20 @@ def load_library():
 
 def _np_ptr(a):
     return a.ctypes.data_as(ctypes.c_void_p)
+
+
+def _seed_array(seeds):
+    """(B, 32) uint8 array or a list of 32-byte strings -> contiguous (B, 32) uint8."""
+    if isinstance(seeds, np.ndarray):
+        arr = np.ascontiguousarray(seeds, dtype=np.uint8)
+    else:
+        seeds = [bytes(s) for s in seeds]
+        if any(len(s) != 32 for s in seeds):
+            raise ValueError("every seed must be 32 bytes")
+        arr = np.frombuffer(b"".join(seeds), dtype=np.uint8).reshape(len(seeds), 32).copy()
+    if arr.ndim != 2 or arr.shape[1] != 32:
+        raise ValueError(f"seeds must have shape (B, 32), got {arr.shape}")
+    return arr
 
 
 class DeviceBuffer:

@@ -319,6 +319,31 @@ __attribute__((visibility("default"))) int bz_curve_op(bz_ctx* ctx, int curve, i
   });
 }
 
+// ---- ChaCha20 keystream (the stream bz_create_proofs_seeded expands) --------------------------------
+__attribute__((visibility("default"))) int bz_chacha20_blocks(bz_ctx* ctx, const void* seeds, uint32_t batch, uint64_t blocks_per_seed, void* out) {
+  BZ_TRY(ctx, {
+    BZ_CHECK(seeds && out, "null argument");
+    if (!batch || !blocks_per_seed) return BZ_OK;
+    BZ_CHECK(blocks_per_seed <= (SIZE_MAX / 64) / batch, "chacha20: output size overflows");
+    const size_t bytes = (size_t)batch * blocks_per_seed * 64;
+    cudaStream_t st = ctx->c.stream;
+    bz::DevBuf &ds = ctx->c.stage[0], &dout = ctx->c.stage[1];
+    ds.ensure((size_t)batch * 32);
+    BZ_CUDA(cudaMemcpyAsync(ds.p, seeds, (size_t)batch * 32, cudaMemcpyHostToDevice, st));
+    cudaPointerAttributes at{};
+    const bool on_device = cudaPointerGetAttributes(&at, out) == cudaSuccess && at.type == cudaMemoryTypeDevice;
+    cudaGetLastError();
+    if (on_device && ((uintptr_t)out & 15) == 0) {
+      bz::chacha20_fill_run(&ctx->c, ds.p, batch, blocks_per_seed, out);
+    } else {
+      dout.ensure(bytes);
+      bz::chacha20_fill_run(&ctx->c, ds.p, batch, blocks_per_seed, dout.p);
+      BZ_CUDA(cudaMemcpyAsync(out, dout.p, bytes, cudaMemcpyDefault, st));
+    }
+    BZ_CUDA(cudaStreamSynchronize(st));
+  });
+}
+
 // ---- MSM ----------------------------------------------------------------------------------------
 __attribute__((visibility("default"))) int bz_msm_dev(bz_ctx* ctx, int curve, const void* d_coeffs, const void* d_bases, uint64_t n, void* d_out_jac, int window_bits) {
   BZ_TRY(ctx, {

@@ -173,6 +173,11 @@ struct NttFusion {
 void ntt_run(Ctx* ctx, int field, const void* in, void* out, int logN, bool inverse, int batch, const NttFusion& fu,
              int batch2 = 1, uint64_t in_stride2 = 0, uint64_t out_stride2 = 0);
 
+// ---- rng.cu ----
+// ChaCha20 keystream blocks 0 .. blocks-1 of each of B 32-byte keys (d_seeds) into d_out (B x blocks x 64 B, the layout of
+// rand_wide); device buffers, 16-byte aligned; asynchronous on the context's stream.
+void chacha20_fill_run(Ctx* ctx, const void* d_seeds, uint32_t B, uint64_t blocks, void* d_out);
+
 }  // namespace bz
 
 // the opaque handle of the C ABI

@@ -1070,7 +1070,8 @@ void Prover::run(const void* instances, const uint32_t* instance_lens, uint32_t 
       for (uint32_t b = 0; b < B; ++b) ps[b].wide = wide_host.get() + (size_t)b * pk.R * 64;
     } else cudaGetLastError();
   }
-  BZ_CUDA(cudaMemcpyAsync(w.wide.p, rand_wide, (size_t)B * pk.R * 64, cudaMemcpyDefault, st));
+  if (rand_wide != w.wide.p)        // bz_create_proofs_seeded expands the stream in place
+    BZ_CUDA(cudaMemcpyAsync(w.wide.p, rand_wide, (size_t)B * pk.R * 64, cudaMemcpyDefault, st));
   {
     uint64_t tot = (uint64_t)B * pk.R;
     from_u512_kernel<FpP><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>((const uint32_t*)w.wide.p, (DFe*)w.rnd.p, tot);
@@ -1565,6 +1566,32 @@ extern "C" API int bz_create_proofs(bz_ctx* ctx, bz_pk* pkh, uint32_t batch, con
     ensure_work(C, pk, batch);
     Prover pr(C, pk, batch);
     pr.run(instances, instance_lens, instance_stride, advice, rand_wide, (uint8_t*)proofs);
+  });
+}
+
+// The same proofs with the blinding randomness expanded on the device: proof b is bz_create_proofs' proof with rand_wide[b] =
+// the ChaCha20 keystream of seeds[b].  The stream is written into the staging buffer bz_create_proofs copies rand_wide to, and
+// Prover::run takes it from there through its device-pointer path (the short ranges the host reads are mirrored back).
+extern "C" API int bz_create_proofs_seeded(bz_ctx* ctx, bz_pk* pkh, uint32_t batch, const void* instances, const uint32_t* instance_lens,
+                                           uint32_t instance_stride, const void* advice, const void* seeds, void* proofs) {
+  PV_TRY(ctx, {
+    BZ_CHECK(pkh && advice && seeds && proofs && batch >= 1, "null argument");
+    PkImpl& pk = pkh->p;
+    BZ_CHECK(pk.cs.I == 0 || (instances && instance_lens), "instances missing");
+    // the same seed for two witnesses would give both proofs the same blinds, which breaks zero knowledge
+    std::set<std::array<uint8_t, 32>> distinct;
+    for (uint32_t b = 0; b < batch; ++b) {
+      std::array<uint8_t, 32> s;
+      memcpy(s.data(), (const uint8_t*)seeds + (size_t)b * 32, 32);
+      BZ_CHECK(distinct.insert(s).second, "bz_create_proofs_seeded: seed " + std::to_string(b) + " repeats an earlier seed of the batch");
+    }
+    ensure_work(C, pk, batch);
+    PkImpl::Work& w = pk.work;
+    w.seeds.ensure((size_t)batch * 32);
+    BZ_CUDA(cudaMemcpyAsync(w.seeds.p, seeds, (size_t)batch * 32, cudaMemcpyHostToDevice, C->stream));
+    chacha20_fill_run(C, w.seeds.p, batch, pk.R, w.wide.p);
+    Prover pr(C, pk, batch);
+    pr.run(instances, instance_lens, instance_stride, advice, w.wide.p, (uint8_t*)proofs);
   });
 }
 

@@ -155,7 +155,7 @@ struct PkImpl : VkImpl {
   // workspace cache
   struct Work {
     uint32_t batch = 0;
-    DevBuf val, poly, coset, misc, rnd, wide, hext, hcoef, hext_low, hcoef_low, nd, consts, extras, evalout, commits, ptrs, descs, msm_jac, ipa_coefq, ipa_gm, ipa_tmp, lk_sorted, lk_err, scan_tmp, eval_tmp;
+    DevBuf val, poly, coset, misc, rnd, wide, seeds, hext, hcoef, hext_low, hcoef_low, nd, consts, extras, evalout, commits, ptrs, descs, msm_jac, ipa_coefq, ipa_gm, ipa_tmp, lk_sorted, lk_err, scan_tmp, eval_tmp;
     void* h_pinned = nullptr; size_t h_pinned_bytes = 0;
     uint32_t* h_err = nullptr;      // pinned: error word of the device lookup permutation
   } work;

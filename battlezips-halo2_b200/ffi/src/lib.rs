@@ -299,9 +299,8 @@ pub fn predraw<R: RngCore>(rng: &mut R, n: usize) -> Vec<u8> {
     out
 }
 
-/// One call for `batch` proofs of one circuit: instances[b][col] values, advice[b] = num_advice x n scalars.  Returns the
-/// proof byte strings exactly as `Blake2bWrite::finalize()` yields them in halo2_proofs 0.2.0.
-pub fn create_proofs<R: RngCore>(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], advice: &[Fp], rng: &mut R) -> Result<Vec<Vec<u8>>, BzError> {
+/// instances[b][col] values -> (batch x ncol x stride scalars, lens, stride), the layout bz_create_proofs reads
+fn pack_instances(instances: &[Vec<Vec<Fp>>]) -> (Vec<Fp>, Vec<u32>, u32) {
     let batch = instances.len();
     let ncol = instances.first().map(|i| i.len()).unwrap_or(0);
     let lens: Vec<u32> = (0..ncol).map(|c| instances[0][c].len() as u32).collect();
@@ -313,11 +312,33 @@ pub fn create_proofs<R: RngCore>(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], advi
             inst[(b * ncol + c) * stride as usize..][..col.len()].copy_from_slice(col);
         }
     }
+    (inst, lens, stride)
+}
+
+/// One call for `batch` proofs of one circuit: instances[b][col] values, advice[b] = num_advice x n scalars.  Returns the
+/// proof byte strings exactly as `Blake2bWrite::finalize()` yields them in halo2_proofs 0.2.0.
+pub fn create_proofs<R: RngCore>(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], advice: &[Fp], rng: &mut R) -> Result<Vec<Vec<u8>>, BzError> {
+    let batch = instances.len();
+    let (inst, lens, stride) = pack_instances(instances);
     let words = predraw(rng, pk.num_random() * batch);
     let size = pk.proof_size();
     let mut proofs = vec![0u8; size * batch];
     let c = ctx();
     check(c, unsafe { bz_create_proofs(c, pk.0, batch as u32, inst.as_ptr() as *const c_void, lens.as_ptr(), stride, advice.as_ptr() as *const c_void, words.as_ptr() as *const c_void, proofs.as_mut_ptr() as *mut c_void) })?;
+    Ok(proofs.chunks_exact(size).map(|p| p.to_vec()).collect())
+}
+
+/// `create_proofs` with the blinding randomness expanded on the device from one 32-byte seed per proof: proof b is the proof
+/// stock halo2 writes when its `rng` is `rand_chacha::ChaCha20Rng::from_seed(seeds[b])`.  The host uploads 32 bytes per proof
+/// instead of `num_random() x 64`.  A seed must come from a CSPRNG and never be reused (equal seeds in one call are an error).
+pub fn create_proofs_seeded(pk: &DevicePk, instances: &[Vec<Vec<Fp>>], advice: &[Fp], seeds: &[[u8; 32]]) -> Result<Vec<Vec<u8>>, BzError> {
+    let batch = instances.len();
+    assert_eq!(seeds.len(), batch, "one seed per proof");
+    let (inst, lens, stride) = pack_instances(instances);
+    let size = pk.proof_size();
+    let mut proofs = vec![0u8; size * batch];
+    let c = ctx();
+    check(c, unsafe { bz_create_proofs_seeded(c, pk.0, batch as u32, inst.as_ptr() as *const c_void, lens.as_ptr(), stride, advice.as_ptr() as *const c_void, seeds.as_ptr() as *const c_void, proofs.as_mut_ptr() as *mut c_void) })?;
     Ok(proofs.chunks_exact(size).map(|p| p.to_vec()).collect())
 }
 

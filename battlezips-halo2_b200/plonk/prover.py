@@ -5,7 +5,7 @@ Params / ProvingKey hold opaque device handles; create_proof returns exactly the
 yields in halo2_proofs 0.2.0."""
 import ctypes
 import numpy as np
-from ..binding import _np_ptr, BzError
+from ..binding import _np_ptr, _seed_array, BzError
 
 FP = 0x40000000000000000000000000000000224698fc094cf91b992d30ed00000001
 _FP_ROOT = 0x2bce74deac30ebda362120830561f81aea322bf2b7bb7584bdad6fabd87ea32f
@@ -80,6 +80,8 @@ def _bind(lib):
     lib.bz_pk_quotient_muls.argtypes = [vp, u32, vp]
     lib.bz_create_proofs.restype = i32
     lib.bz_create_proofs.argtypes = [vp, vp, u32, vp, vp, u32, vp, vp, vp]
+    lib.bz_create_proofs_seeded.restype = i32
+    lib.bz_create_proofs_seeded.argtypes = [vp, vp, u32, vp, vp, u32, vp, vp, vp]
     lib._prover_bound = True
 
 
@@ -336,6 +338,24 @@ def create_proofs(pk, instances, advice, rand_wide):
                 inst[b, i, :lens[i]] = mont(instances[b][i])
     out = np.zeros((B, pk.proof_size), dtype=np.uint8)
     ctx._check(ctx.lib.bz_create_proofs(ctx.h, pk.h, B, _np_ptr(inst), _np_ptr(lens), stride, _np_ptr(advice), _np_ptr(rand_wide), _np_ptr(out)))
+    return [bytes(out[b]) for b in range(B)]
+
+
+def create_proofs_seeded(pk, instances, advice, seeds):
+    """create_proof for a batch with the blinding randomness expanded on the device (bz_create_proofs_seeded): proof b equals
+    create_proofs(..., rand_wide[b] = ChaCha20 keystream of seeds[b]), i.e. stock halo2 run with ChaCha20Rng::from_seed(seeds[b]).
+    seeds: (B, 32) uint8 or a list of B 32-byte strings, drawn from a CSPRNG and never reused (equal seeds in one call are
+    rejected).  instances, advice as for create_proofs.  Returns list of B proof byte strings."""
+    ctx = pk.ctx
+    advice = np.ascontiguousarray(advice, dtype=np.uint64)
+    B = advice.shape[0]
+    assert advice.shape == (B, pk.ir["num_advice"], pk.n, 4)
+    seeds = _seed_array(seeds)
+    if len(seeds) != B:
+        raise ValueError(f"{len(seeds)} seeds for {B} witnesses")
+    inst, lens, stride = _pack_instances(pk, instances, B)
+    out = np.zeros((B, pk.proof_size), dtype=np.uint8)
+    ctx._check(ctx.lib.bz_create_proofs_seeded(ctx.h, pk.h, B, _np_ptr(inst), _np_ptr(lens), stride, _np_ptr(advice), _np_ptr(seeds), _np_ptr(out)))
     return [bytes(out[b]) for b in range(B)]
 
 

@@ -103,6 +103,15 @@ int bz_batch_invert_assigned_dev(bz_ctx* ctx, int field, const void* d_numerator
 /* affine in, affine out (64 B each): op 0 a+b, 1 2a, 2 a-b, 3 2a+b (full projective add), 4 [k]a, k = first u32 of b */
 int bz_curve_op(bz_ctx* ctx, int curve, int op, const void* a, const void* b, void* out, uint64_t n);
 
+/* ---- ChaCha20 keystream: the blinding randomness of bz_create_proofs_seeded ---------------------------------------------------
+ * out[b][j] = ChaCha20 block j (64 B) of key seeds[b], for b < batch and j < blocks_per_seed: 20 rounds, key = the 32-byte seed,
+ * a 64-bit block counter j in state words 12-13 and stream id 0 in words 14-15 (the original layout that rand_chacha's
+ * ChaCha20Rng uses; for j < 2^32 it equals RFC 8439 with an all-zero nonce).  Block j is the 64-byte Scalar::random draw j
+ * (8 x next_u64, low word first), so out has rand_wide's layout: batch x blocks_per_seed x 64 B.
+ *   seeds : batch x 32 B (host).  A seed must come from a CSPRNG and never be reused.
+ *   out   : host or device memory; 16-byte aligned device memory is written in place, without a copy.  Synchronous. */
+int bz_chacha20_blocks(bz_ctx* ctx, const void* seeds, uint32_t batch, uint64_t blocks_per_seed, void* out);
+
 /* ---- arithmetic::best_multiexp(coeffs, bases) -> C::Curve  (U: halo2_proofs/src/arithmetic.rs) -- */
 /* host buffers; copies are part of the call.  out_jac: 96 B. */
 int bz_best_multiexp(bz_ctx* ctx, int curve, const void* coeffs, const void* bases, uint64_t n, void* out_jac);
@@ -239,6 +248,17 @@ int bz_pk_quotient_generated(const bz_pk* pk, uint32_t tier);
  * Errors: BZ_ERR_SYNTHESIS when a lookup input is missing from its table (Error::ConstraintSystemFailure). */
 int bz_create_proofs(bz_ctx* ctx, bz_pk* pk, uint32_t batch, const void* instances, const uint32_t* instance_lens,
                      uint32_t instance_stride, const void* advice, const void* rand_wide, void* proofs);
+
+/* bz_create_proofs with the blinding randomness drawn on the device: proof b has exactly the bytes bz_create_proofs gives for
+ * rand_wide[b] = the ChaCha20 keystream of seeds[b] (bz_chacha20_blocks with blocks_per_seed = bz_pk_num_random), which is the
+ * stream stock halo2 consumes from `rand_chacha::ChaCha20Rng::from_seed(seeds[b])`.  The caller uploads 32 bytes per proof
+ * instead of bz_pk_num_random x 64.
+ *   seeds     : batch x 32 B (host).  A seed must come from a CSPRNG and never be reused: the seed fixes every blind of the
+ *               proof, so one seed for two witnesses breaks zero knowledge.
+ *   instances, instance_lens, instance_stride, advice, proofs : as for bz_create_proofs
+ * Errors: BZ_ERR_INVALID for a null argument, batch = 0 or two equal seeds in one call; otherwise as bz_create_proofs. */
+int bz_create_proofs_seeded(bz_ctx* ctx, bz_pk* pk, uint32_t batch, const void* instances, const uint32_t* instance_lens,
+                            uint32_t instance_stride, const void* advice, const void* seeds, void* proofs);
 
 /* plonk::verify_proof (SingleVerifier semantics: one verdict per proof) for `batch` proofs of the same circuit
  * (U: halo2_proofs 0.2.0 src/plonk/verifier.rs and the argument verifiers; reference call sites
